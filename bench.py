@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload train|render|rollout|et_rollout|bert|train_bert|train_rollout|mapprep]
     python bench.py --impl reference ...        # the reference's CPU path, same metric
+    python bench.py --dump-outputs DIR ...      # also write the last timed step's outputs as DIR/<name>.npy
 
 One JSON line on stdout (rank 0).  Under torchrun (N>1) every rank runs its shard
 of the workload; the timed region is bracketed by a barrier + synchronize and the
@@ -327,7 +328,7 @@ def use_all_host_threads():
 
 def run_reference(args, W):
     """``--impl reference``: the reference's CPU implementation of the path (cv2 for the renderer; the oracle port
-    pinned to the reference modules for the training step -- /root/reference does not exist on the GPU box) on the
+    pinned to the reference modules for the training step -- the reference tree is not part of this project) on the
     box's host cores, on a bounded sample of the workload.  The line states ITS OWN configuration."""
     rank, world, _ = dist_env()
     if rank != 0:
@@ -359,11 +360,37 @@ def run_reference(args, W):
     emit(line)
 
 
-def measure(wl, dev, rank, world, local, steps, warmup, with_cpu, dist):
+DUMP_SAMPLE = 1 << 20          # elements kept of a larger output (fixed seeded indices)
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(wl, out_dir):
+    """``--dump-outputs``: write the arrays of ``wl.outputs()`` (what the last timed step computed) as
+    ``<name>.npy``, float64 where the output is float64 and float32 otherwise.  An output of more than
+    ``DUMP_SAMPLE`` elements is reduced to a sample at indices drawn from a generator seeded by its name, so that
+    two builds of the project can be compared array for array."""
+    import zlib
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in sorted(wl.outputs().items()):
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            g = torch.Generator().manual_seed(zlib.crc32(name.encode()))
+            idx = torch.randint(0, t.numel(), (DUMP_SAMPLE,), generator=g).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        a = t.cpu().numpy().astype(np.float64 if t.dtype == torch.float64 else np.float32)
+        total += a.nbytes
+        if total > DUMP_MAX_BYTES:
+            raise RuntimeError(f"--dump-outputs: the outputs exceed {DUMP_MAX_BYTES >> 20} MB at {name}")
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def measure(wl, dev, rank, world, local, steps, warmup, with_cpu, dist, dump_dir=None):
     """One workload, the bench contract: W untimed warm-up steps, exactly K timed steps bracketed by barrier +
     synchronize, CUDA events on the launching stream, L2 flushed between timed steps, max over ranks; then the same
     metric end to end through the public API with host buffers; then the roofline of the dominant kernel and (rank 0)
-    the CPU leg.  Returns the result dict on every rank (the CPU leg and the formatting only matter on rank 0)."""
+    the CPU leg.  With ``dump_dir`` rank 0 writes the outputs of the last timed step there first (``dump_outputs``).
+    Returns the result dict on every rank (the CPU leg and the formatting only matter on rank 0)."""
     use_dist = dist is not None
     peaks = load_peaks()
 
@@ -374,7 +401,9 @@ def measure(wl, dev, rank, world, local, steps, warmup, with_cpu, dist):
 
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)      # > L2 (126 MB)
     launches = 0
+    before_step = getattr(wl, "before_step", lambda: None)
     for _ in range(warmup):
+        before_step()
         wl.step()
         wl.after_step(False)
     barrier()
@@ -383,6 +412,7 @@ def measure(wl, dev, rank, world, local, steps, warmup, with_cpu, dist):
         barrier()
         t_wall0 = time.perf_counter()
         for i in range(steps):
+            before_step()                                   # untimed
             flush.zero_()                                   # L2 flush between timed iterations (untimed)
             evs[i][0].record()
             launches += wl.step()
@@ -390,6 +420,8 @@ def measure(wl, dev, rank, world, local, steps, warmup, with_cpu, dist):
             wl.after_step(True)
         barrier()
         t_wall = time.perf_counter() - t_wall0
+    if dump_dir is not None and rank == 0:
+        dump_outputs(wl, dump_dir)
     ms = sum(a.elapsed_time(b) for a, b in evs)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if use_dist:
@@ -440,7 +472,9 @@ def measure(wl, dev, rank, world, local, steps, warmup, with_cpu, dist):
             "scaling": "weak", "vs_baseline": None, "dtype": wl.dtype, "data": "synthetic",
             "config": wl.config(), "roofline": wl.roofline(peaks) if rank == 0 else None, "cpu_baseline": cpu,
             "e2e": {"value": e2e_val, "unit": wl.unit, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h},
-            "gpu_launches": launches, "clocks": clk.summary(), "wall_s_timed_region": t_wall}
+            "gpu_launches": launches, "clocks": clk.summary(),
+            # host time of the whole timed loop: it also counts the untimed L2 flushes and before_step restores
+            "wall_s_timed_region": t_wall}
     if multi:
         line.update(multi)
     extra = getattr(wl, "extra", None)
@@ -461,6 +495,11 @@ def main():
                     help="train workload only: skip the render (configs[2]) and rollout (configs[4]) entries")
     ap.add_argument("--no-library-bar", action="store_true",
                     help="train workload only: skip the stock torch / cuDNN / cuBLAS timing of the same step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="training workloads (train, train_bert, train_rollout) only: after the timed steps, write "
+                         "what the last one computed as DIR/<name>.npy (float32 / float64, a fixed seeded sample of "
+                         "large outputs, 64 MB at most); the inputs are the same from run to run, so two builds can "
+                         "be compared output for output.  The secondary entries of the default line are not dumped")
     args = ap.parse_args()
     # stdout carries exactly ONE line (the JSON result): anything libraries print on file descriptor 1
     # (e.g. NCCL's version banner) is sent to stderr instead
@@ -470,10 +509,11 @@ def main():
     os.dup2(2, 1)
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     W = WORKLOADS[args.workload]
+    if args.dump_outputs is not None and (args.impl != "ours" or not hasattr(W, "outputs")):
+        raise SystemExit(f"--dump-outputs is available for the GPU arm of the workloads "
+                         f"{sorted(k for k, w in WORKLOADS.items() if hasattr(w, 'outputs'))}")
 
     if args.impl == "reference":
-        if args.steps > 5:
-            args.steps = 5
         args.warmup = min(args.warmup, 1)
         run_reference(args, W)
         return
@@ -489,7 +529,8 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
     wl = W(rank, world)
     wl.setup_gpu(dev)
-    line = measure(wl, dev, rank, world, local, args.steps, args.warmup, not args.no_cpu_baseline, dist)
+    line = measure(wl, dev, rank, world, local, args.steps, args.warmup, not args.no_cpu_baseline, dist,
+                   dump_dir=args.dump_outputs)
 
     if args.workload == "train":
         # BASELINE.json's metric names two more numbers -- "rendered views/s" (configs[2]) and the greedy rollout

@@ -118,6 +118,42 @@ class TrainWorkload:
         self.loss_host = torch.zeros(1, dtype=torch.float64).pin_memory()
         self.profile = None
         self.last_loss = None
+        self._start_state = None
+
+    def _state_tensors(self):
+        ag = self.agent
+        return [t for o in ag.optimizers for t in (o.p, o.m, o.v)] + list(ag.vision_model.buffers())
+
+    def _dropout_modules(self):
+        ag = self.agent
+        return [m for model in (ag.vision_model, ag.vln_model, ag.lang_model) if model is not None
+                for m in model.modules() if hasattr(type(m), "dropout_config")]
+
+    def snapshot(self):
+        """Everything a training step reads and updates besides the batch: weights, AdamW moments and step counts,
+        the trunk's BatchNorm running statistics and the dropout step counters (the masks derive from them)."""
+        return ([t.clone() for t in self._state_tensors()], [o.step_count for o in self.agent.optimizers],
+                [getattr(m, "_drop_step", 0) for m in self._dropout_modules()])
+
+    def restore(self, snap):
+        tensors, counts, drop = snap
+        for t, t0 in zip(self._state_tensors(), tensors):
+            t.copy_(t0)
+        for o, n in zip(self.agent.optimizers, counts):
+            o.step_count = n
+        for m, n in zip(self._dropout_modules(), drop):
+            m._drop_step = n
+
+    def before_step(self):
+        """Untimed, before every warm-up and timed step: put back the state the first step started from
+        (``snapshot``), so that every step computes the same training step from the same state on the same batch.
+        Without it each step trains on from the previous one, and the order of atomic reductions -- which is not
+        fixed -- makes two runs of one command drift apart step by step (AdamW's first updates are nearly
+        sign(grad), and the random-init train-mode trunk amplifies small differences)."""
+        if self._start_state is None:
+            self._start_state = self.snapshot()
+        else:
+            self.restore(self._start_state)
 
     def step(self):
         l0 = self.agent.launches
@@ -126,6 +162,21 @@ class TrainWorkload:
 
     def after_step(self, timed):
         pass
+
+    def outputs(self):
+        """What the last ``step()`` produced (``bench.py --dump-outputs``): the step loss ``train_step`` returns and
+        the state the step leaves -- the trunk's BatchNorm running statistics and, per model, the gradients and the
+        updated parameters, concatenated in sorted parameter-name order so that they do not depend on the layout of
+        the optimiser arenas.  ``before_step`` makes the last step start from the same state in every run."""
+        ag = self.agent
+        out = {"loss": ag.loss_total,
+               "trunk_bn_running": torch.cat([b.flatten().float() for n, b in sorted(ag.vision_model.named_buffers())
+                                              if "running" in n])}
+        for model, opt in zip(("et", "trunk", "lang"), ag.optimizers):
+            names = sorted(opt.params)
+            out[f"{model}_grad"] = torch.cat([opt.grads[n].flatten() for n in names])
+            out[f"{model}_param"] = torch.cat([opt.params[n].detach().flatten() for n in names])
+        return out
 
     def step_e2e(self):
         h2d = 0
@@ -237,17 +288,13 @@ class TrainWorkload:
             return e0.elapsed_time(e1) / k
 
         synced = back_to_back()                       # same loop with the all-reduce on, for a like-for-like pair
-        snap = [(o, o.p.clone(), o.m.clone(), o.v.clone(), o.step_count) for o in ag.optimizers]
-        bn = [b.clone() for b in ag.vision_model.buffers()]
+        snap = self.snapshot()
         world, ag.world = ag.world, 1
         try:
             solo = back_to_back()
         finally:
             ag.world = world
-        for o, p_, m_, v_, sc in snap:
-            o.p.copy_(p_); o.m.copy_(m_); o.v.copy_(v_); o.step_count = sc
-        for b, b0 in zip(ag.vision_model.buffers(), bn):
-            b.copy_(b0)
+        self.restore(snap)
         per = [torch.zeros(2, dtype=torch.float64, device=self.dev) for _ in range(world)]
         dist.all_gather(per, torch.tensor([solo, synced], dtype=torch.float64, device=self.dev))
         synced = max(float(x[1].item()) for x in per)

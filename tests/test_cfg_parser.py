@@ -1,13 +1,10 @@
 """CPU: D1 -- the product's cfg parser (models/dark_net.py) against the reference's own ``parse_model_config``
-(src/models/dark_net.py:243-261), imported from /root/reference in the build container (skipped where the reference
-tree is absent), on the synthetic 79-block trunk cfg and on a cfg with comments, blank lines and fringe whitespace."""
-import importlib.util
+(src/models/dark_net.py:243-261), on the synthetic 79-block trunk cfg and on a cfg with comments, blank lines and
+fringe whitespace.  tests/golden/cfg_parser_golden.json stores both cfg texts with the module-definition lists the
+reference parser returns for them (values stay strings, ``batch_normalize`` defaults to the int 0)."""
+import json
 import os
 import tempfile
-
-import pytest
-
-REF = "/root/reference/src/models/dark_net.py"
 
 TRICKY = """# leading comment
 [net]
@@ -38,32 +35,24 @@ anchors = 10,13,  16,30
 """
 
 
-def _reference_parser():
-    spec = importlib.util.spec_from_file_location("ref_dark_net", REF)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod.parse_model_config
-
-
-@pytest.mark.skipif(not os.path.exists(REF), reason="the reference tree is not present on this box")
-def test_parse_model_config_matches_reference(built_lib):
+def _parse(text):
     from avdn_b200.models.dark_net import parse_model_config
-    from avdn_b200.utils import synthetic
-    ref = _reference_parser()
-    for text in (synthetic.yolov3_trunk_cfg(), TRICKY):
-        with tempfile.NamedTemporaryFile("w", suffix=".cfg", delete=False) as f:
-            f.write(text)
-        try:
-            ours, theirs = parse_model_config(f.name), ref(f.name)
-        finally:
-            os.unlink(f.name)
-        assert ours == theirs
-    # the synthetic cfg is the truncated-79 trunk: [net] + 80 blocks (57 convolutions, 23 shortcuts)
     with tempfile.NamedTemporaryFile("w", suffix=".cfg", delete=False) as f:
-        f.write(synthetic.yolov3_trunk_cfg())
+        f.write(text)
     try:
-        defs = parse_model_config(f.name)
+        return parse_model_config(f.name)
     finally:
         os.unlink(f.name)
+
+
+def test_parse_model_config_matches_reference(built_lib, golden_dir):
+    from avdn_b200.utils import synthetic
+    with open(os.path.join(golden_dir, "cfg_parser_golden.json")) as f:
+        golden = json.load(f)
+    assert golden["tricky"]["text"] == TRICKY
+    for case in ("trunk", "tricky"):
+        assert _parse(golden[case]["text"]) == golden[case]["module_defs"], case
+    # the synthetic cfg is the truncated-79 trunk: [net] + 80 blocks (57 convolutions, 23 shortcuts)
+    defs = _parse(synthetic.yolov3_trunk_cfg())
     kinds = [d["type"] for d in defs]
     assert kinds[0] == "net" and kinds.count("convolutional") == 57 and kinds.count("shortcut") == 23
