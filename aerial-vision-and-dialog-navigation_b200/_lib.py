@@ -116,6 +116,11 @@ _SIGNATURES = {
     "avdn_lstm_cell": [c_void_p, c_void_p, c_void_p, c_i64, c_void_p, c_int, c_int, c_void_p],
     "avdn_direction_embed": [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p],
     "avdn_lang_attn_fwd": [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_i64, c_void_p],
+    "avdn_lstm_cell_bwd": [c_void_p, c_void_p, c_void_p, c_void_p, c_i64, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                           c_void_p],
+    "avdn_direction_embed_bwd": [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p],
+    "avdn_lang_attn_bwd": [c_void_p, c_void_p, c_void_p, c_void_p, c_i64, c_int, c_int, c_int, c_void_p, c_void_p,
+                           c_void_p],
     "avdn_waypoint_step": [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_f32, c_int, c_void_p, c_void_p,
                            c_void_p, c_void_p],
     # ---- agent slice

@@ -134,7 +134,9 @@ __global__ void __launch_bounds__(256) frame_attn_bwd_kernel(
     s_wc[tid] = wc[(size_t)bt * NSP + tid];
     s_e[tid] = e49[(size_t)bt * NSP + tid];
   }
-  for (int o = tid; o < E; o += 256) s_demb[o] = d_emb[(size_t)bt * E + o];
+  if (fc2_w) {
+    for (int o = tid; o < E; o += 256) s_demb[o] = d_emb[(size_t)bt * E + o];
+  }
   for (int c = tid; c < NCH; c += 256) s_attn[c] = attn[(size_t)bt * NCH + c];
   __syncthreads();
   if (tid < NSP) {
@@ -142,8 +144,8 @@ __global__ void __launch_bounds__(256) frame_attn_bwd_kernel(
     for (int j = 0; j < NSP; ++j) a = fmaf(w_in[tid * NSP + j], s_h[j], a);
     s_t[tid] = a;
   }
-  // fc2: d_e[j] = sum_o fc2_w[o][j] d_emb[o]   (d_fc2_w / d_fc2_b: frame_attn_fc2_grad_kernel)
-  {
+  if (fc2_w) {
+    // fc2: d_e[j] = sum_o fc2_w[o][j] d_emb[o]   (d_fc2_w / d_fc2_b: frame_attn_fc2_grad_kernel)
     float a0 = 0.f, a1 = 0.f;       // warp w: rows o = w, w+8, ... ; lanes over j
     for (int o = warp; o < E; o += 8) {
       const float g = s_demb[o];
@@ -156,7 +158,11 @@ __global__ void __launch_bounds__(256) frame_attn_bwd_kernel(
   __syncthreads();
   if (tid < NSP) {
     float a = 0.f;
-    for (int w = 0; w < 8; ++w) a += s_red[w][tid];
+    if (fc2_w) {
+      for (int w = 0; w < 8; ++w) a += s_red[w][tid];
+    } else {
+      a = d_emb[(size_t)bt * NSP + tid];                   // no fc2 (ViT_LSTM): d_emb is d_e49 [B*T,49]
+    }
     s_de[tid] = a;
     s_dpre[tid] = a * (1.f - s_e[tid] * s_e[tid]);       // tanh'
   }
@@ -841,13 +847,14 @@ extern "C" int avdn_frame_attn_bwd_cls(const float* frames, const float* lang_cl
                                        const float* wc, const float* e49, const float* d_emb, float* d_frames,
                                        float* d_w_in, float* d_w_out, float* d_fc2_w, float* d_fc2_b,
                                        float* d_lang_cls, avdn_stream_t stream) {
-  AVDN_REQUIRE(frames && lang_cls && w_in && w_out && fc2_w && attn && wc && e49 && d_emb && d_frames && d_w_in &&
-                   d_w_out && d_fc2_w && d_fc2_b,
+  AVDN_REQUIRE(frames && lang_cls && w_in && w_out && attn && wc && e49 && d_emb && d_frames && d_w_in && d_w_out &&
+                   (!fc2_w || (d_fc2_w && d_fc2_b)),
                "avdn_frame_attn_bwd: null pointer");
   if (B * T == 0) return AVDN_OK;
   static_assert(E % FC2_ROWS == 0, "fc2 gradient blocks tile the 768 rows");
-  frame_attn_fc2_grad_kernel<<<dim3(E / FC2_ROWS, FC2_SLICES), FC2_ROWS * (NSP + 1), 0, avdn::to_cuda(stream)>>>(
-      d_emb, e49, B * T, d_fc2_w, d_fc2_b);
+  if (fc2_w)
+    frame_attn_fc2_grad_kernel<<<dim3(E / FC2_ROWS, FC2_SLICES), FC2_ROWS * (NSP + 1), 0, avdn::to_cuda(stream)>>>(
+        d_emb, e49, B * T, d_fc2_w, d_fc2_b);
   frame_attn_bwd_kernel<<<B * T, 256, 0, avdn::to_cuda(stream)>>>(frames, lang_cls, w_in, w_out, fc2_w, T, attn, wc,
                                                                 e49, d_emb, d_frames, d_w_in, d_w_out, d_fc2_w,
                                                                 d_fc2_b, d_lang_cls);

@@ -10,6 +10,8 @@
 //   lstm_cell      nn.LSTMCell pointwise part (gate order i,f,g,o)
 //   lang_attn      SoftDotAttention(768) over the dialog tokens: scores, softmax over L, weighted sum
 //   waypoint_step  agent.py:637-653,700-730 + move_view_corners, one thread per sample, float64
+// and the backward of the training rollout (ViT_LSTM.train_engine): lstm_cell_bwd, lang_attn_bwd and
+// direction_embed_bwd.  The weight gradients of the linear layers go through avdn_linear_f32_bwd (bert.cu).
 #include "common.cuh"
 
 namespace {
@@ -172,14 +174,61 @@ __global__ void lstm_cell_kernel(const float* __restrict__ gates, const float* _
   h_out[(size_t)b * ldh + j] = og * tanhf(c);
 }
 
+// Backward of lstm_cell_kernel from the saved pre-activations and cell state (autograd of nn.LSTMCell's pointwise
+// part): dc = dh * o * (1 - tanh(c)^2) + dc_next; dgates = (dc g i(1-i), dc c_prev f(1-f), dc i (1-g^2),
+// dh tanh(c) o(1-o)); dc_prev = dc f.  The gate activations are recomputed exactly as the forward computes them.
+// dc_next and dc_prev are not __restrict__: a caller may pass one buffer for both (same element read, then written).
+__global__ void lstm_cell_bwd_kernel(const float* __restrict__ gates, const float* __restrict__ c_prev,
+                                     const float* __restrict__ c, const float* __restrict__ dh, long long lddh,
+                                     const float* dc_next, float* __restrict__ dgates, float* dc_prev, int B, int H) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= B * H) return;
+  const int b = i / H, j = i - b * H;
+  const float* g = gates + (size_t)b * 4 * H;
+  const float ig = 1.f / (1.f + expf(-g[j]));
+  const float fg = 1.f / (1.f + expf(-g[H + j]));
+  const float gg = tanhf(g[2 * H + j]);
+  const float og = 1.f / (1.f + expf(-g[3 * H + j]));
+  const float tc = tanhf(c[i]);
+  const float cp = c_prev ? c_prev[i] : 0.f;
+  const float d_h = dh[(size_t)b * lddh + j];
+  const float dc = d_h * og * (1.f - tc * tc) + (dc_next ? dc_next[i] : 0.f);
+  float* dg = dgates + (size_t)b * 4 * H;
+  dg[j] = dc * gg * ig * (1.f - ig);
+  dg[H + j] = dc * cp * fg * (1.f - fg);
+  dg[2 * H + j] = dc * ig * (1.f - gg * gg);
+  dg[3 * H + j] = d_h * tc * og * (1.f - og);
+  if (c_prev) dc_prev[i] = dc * fg;
+}
+
 // direction_embedding([sin, cos](d / 180 * 3.14159)) (vln_model.py:228-229), float32 as torch evaluates it
+__device__ __forceinline__ float direction_angle(float deg) { return __fmul_rn(__fdiv_rn(deg, 180.f), 3.14159f); }
+
 __global__ void direction_embed_kernel(const float* __restrict__ deg, const float* __restrict__ w,
                                        const float* __restrict__ b, float* __restrict__ out, int B, int N) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= B * N) return;
   const int s = i / N, n = i - s * N;
-  const float a = __fmul_rn(__fdiv_rn(deg[s], 180.f), 3.14159f);
+  const float a = direction_angle(deg[s]);
   out[i] = __fadd_rn(__fadd_rn(__fmul_rn(w[n * 2], sinf(a)), __fmul_rn(w[n * 2 + 1], cosf(a))), b[n]);
+}
+
+// Its parameter gradient: one thread per (n, k), k = 0 (weight of sin), 1 (weight of cos), 2 (bias), summing over the
+// B rows.  The sin / cos are the forward's (same expression, same translation unit, same flags), so the gradient
+// sees exactly the inputs the forward used.
+__global__ void direction_embed_bwd_kernel(const float* __restrict__ deg, const float* __restrict__ d_out, int B, int N,
+                                           float* __restrict__ d_w, float* __restrict__ d_b) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= 3 * N) return;
+  const int n = i / 3, k = i - n * 3;
+  float acc = 0.f;
+  for (int s = 0; s < B; ++s) {
+    const float a = direction_angle(deg[s]);
+    const float v = k == 0 ? sinf(a) : (k == 1 ? cosf(a) : 1.f);
+    acc = fmaf(d_out[(size_t)s * N + n], v, acc);
+  }
+  if (k < 2) d_w[n * 2 + k] += acc;
+  else d_b[n] += acc;
 }
 
 // ------------------------------------------------------------------ lang_attn
@@ -313,6 +362,60 @@ __global__ void __launch_bounds__(256) lang_attn_v2_kernel(const float* __restri
     }
     float* o = weighted + (size_t)b * ldw + 4 * tid;      // ldw need not be a multiple of 4: scalar stores
     o[0] = acc.x; o[1] = acc.y; o[2] = acc.z; o[3] = acc.w;
+  }
+}
+
+// Backward of lang_attn (autograd of vln_model.py:33-42 between the two Linear layers), one CTA per sample:
+//   d_attn_l = ctx_l . d_weighted ; d_score_l = attn_l (d_attn_l - sum_l' attn_l' d_attn_l')
+//   d_target = sum_l d_score_l ctx_l ; d_ctx_l += attn_l d_weighted + d_score_l target
+// Two passes over the sample's context: the row dots (a warp per row), then one thread per column walks the rows
+// for d_target and the d_ctx update together.
+__global__ void __launch_bounds__(256) lang_attn_bwd_kernel(const float* __restrict__ ctx,
+                                                            const float* __restrict__ target,
+                                                            const float* __restrict__ attn,
+                                                            const float* __restrict__ d_weighted, long long lddw,
+                                                            int L, int D, float* __restrict__ d_target,
+                                                            float* __restrict__ d_ctx) {
+  extern __shared__ float sm[];            // [D] d_weighted, [D] target, [L] attn, [L] d_attn -> d_score
+  float* s_dw = sm;
+  float* s_t = sm + D;
+  float* s_a = s_t + D;
+  float* s_ds = s_a + L;
+  __shared__ float s_dot;
+  const int b = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const float* c = ctx + (size_t)b * L * D;
+  for (int d = tid; d < D; d += 256) {
+    s_dw[d] = d_weighted[(size_t)b * lddw + d];
+    s_t[d] = target[(size_t)b * D + d];
+  }
+  for (int l = tid; l < L; l += 256) s_a[l] = attn[(size_t)b * L + l];
+  __syncthreads();
+  for (int l = warp; l < L; l += 8) {
+    float a = 0.f;
+    for (int d = lane; d < D; d += 32) a = fmaf(c[(size_t)l * D + d], s_dw[d], a);
+    a = warp_sum(a);
+    if (lane == 0) s_ds[l] = a;
+  }
+  __syncthreads();
+  if (warp == 0) {
+    float a = 0.f;
+    for (int l = lane; l < L; l += 32) a = fmaf(s_a[l], s_ds[l], a);
+    a = warp_sum(a);
+    if (lane == 0) s_dot = a;
+  }
+  __syncthreads();
+  for (int l = tid; l < L; l += 256) s_ds[l] = s_a[l] * (s_ds[l] - s_dot);
+  __syncthreads();
+  float* dc = d_ctx ? d_ctx + (size_t)b * L * D : nullptr;
+  for (int d = tid; d < D; d += 256) {
+    const float wd = s_dw[d], td = s_t[d];
+    float acc = 0.f;
+    for (int l = 0; l < L; ++l) {
+      const float ds = s_ds[l];
+      acc = fmaf(ds, c[(size_t)l * D + d], acc);
+      if (dc) dc[(size_t)l * D + d] += fmaf(s_a[l], wd, ds * td);
+    }
+    d_target[(size_t)b * D + d] = acc;
   }
 }
 
@@ -496,6 +599,35 @@ extern "C" int avdn_lang_attn_fwd(const float* ctx, const float* target, int B, 
   }
   lang_attn_kernel<<<B, 256, smem, s>>>(ctx, target, L, D, attn, weighted, ldw);
   return avdn::check_launch("avdn_lang_attn_fwd");
+}
+
+extern "C" int avdn_lstm_cell_bwd(const float* gates, const float* c_prev, const float* c, const float* dh,
+                                  long long lddh, const float* dc_next, float* dgates, float* dc_prev, int B, int H,
+                                  avdn_stream_t stream) {
+  AVDN_REQUIRE(gates && c && dh && dgates && B > 0 && H > 0 && lddh >= H, "avdn_lstm_cell_bwd: bad argument");
+  AVDN_REQUIRE(!c_prev || dc_prev, "avdn_lstm_cell_bwd: dc_prev is required when c_prev is given");
+  lstm_cell_bwd_kernel<<<(B * H + 255) / 256, 256, 0, avdn::to_cuda(stream)>>>(gates, c_prev, c, dh, lddh, dc_next,
+                                                                              dgates, dc_prev, B, H);
+  return avdn::check_launch("avdn_lstm_cell_bwd");
+}
+
+extern "C" int avdn_direction_embed_bwd(const float* deg, const float* d_out, int B, int N, float* d_w, float* d_b,
+                                        avdn_stream_t stream) {
+  AVDN_REQUIRE(deg && d_out && d_w && d_b && B > 0 && N > 0, "avdn_direction_embed_bwd: bad argument");
+  direction_embed_bwd_kernel<<<(3 * N + 127) / 128, 128, 0, avdn::to_cuda(stream)>>>(deg, d_out, B, N, d_w, d_b);
+  return avdn::check_launch("avdn_direction_embed_bwd");
+}
+
+extern "C" int avdn_lang_attn_bwd(const float* ctx, const float* target, const float* attn, const float* d_weighted,
+                                  long long lddw, int B, int L, int D, float* d_target, float* d_ctx,
+                                  avdn_stream_t stream) {
+  AVDN_REQUIRE(ctx && target && attn && d_weighted && d_target && B > 0 && L > 0 && D > 0 && lddw >= D,
+               "avdn_lang_attn_bwd: bad argument");
+  const size_t smem = (size_t)(2 * D + 2 * L) * sizeof(float);
+  AVDN_REQUIRE(smem <= 48 * 1024, "avdn_lang_attn_bwd: D + L = %d too large", D + L);
+  lang_attn_bwd_kernel<<<B, 256, smem, avdn::to_cuda(stream)>>>(ctx, target, attn, d_weighted, lddw, L, D, d_target,
+                                                               d_ctx);
+  return avdn::check_launch("avdn_lang_attn_bwd");
 }
 
 extern "C" int avdn_waypoint_step(const float* output, double* corners, const double* bounds, double* cur_dir,

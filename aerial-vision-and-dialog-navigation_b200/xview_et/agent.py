@@ -41,6 +41,8 @@ from ..models import dark_net as DN
 from ..models.dark_net import Darknet
 from ..optim import FusedAdamW
 from .. import parallel
+from ..agent_common import (RolloutTrainer, render_rollout_views, rollout_trunk_backward,
+                            rollout_trunk_forward, student_rollout_targets)
 
 PI_REF = 3.14159
 
@@ -57,7 +59,7 @@ def get_direction(start, end):
     return (360 - ang + 90) % 360
 
 
-class NavCMTAgent:
+class NavCMTAgent(RolloutTrainer):
     def __init__(self, args, rank=0, world_size=1, device=None, process_group=None):
         if not torch.cuda.is_available():
             raise RuntimeError("NavCMTAgent needs a CUDA device (sm_100); there is no CPU fallback")
@@ -262,33 +264,6 @@ class NavCMTAgent:
         self.launches += n
         return output, h_sali
 
-    @property
-    def nss_w(self):
-        ov = getattr(self, "_nss_w_override", None)
-        return float(ov if ov is not None else getattr(self.args, "nss_w", 1.0))        # parser.py:38 default 1
-
-    @property
-    def train_ml(self):
-        ov = getattr(self, "_train_ml_override", None)
-        return float(ov if ov is not None else getattr(self.args, "ml_weight", 0.2))     # parser.py:54
-
-    class _Weights:
-        """``with agent._weights(nss_w, train_ml):`` -- the per-rollout loss weights the reference passes to
-        ``rollout(train_ml=..., nss_w=...)`` (agent.py:229-235); ``None`` keeps the value from ``args``."""
-
-        def __init__(self, agent, nss_w, train_ml):
-            self.a, self.v = agent, (nss_w, train_ml)
-
-        def __enter__(self):
-            self.old = (getattr(self.a, "_nss_w_override", None), getattr(self.a, "_train_ml_override", None))
-            self.a._nss_w_override, self.a._train_ml_override = self.v
-
-        def __exit__(self, *exc):
-            self.a._nss_w_override, self.a._train_ml_override = self.old
-
-    def _weights(self, nss_w=None, train_ml=None):
-        return NavCMTAgent._Weights(self, nss_w, train_ml)
-
     def forward_loss(self, batch):
         """Validation: forward + loss (trunk in eval mode).  Returns (loss, output, h_sali)."""
         self.vision_model.eval()
@@ -356,45 +331,6 @@ class NavCMTAgent:
             self.exposed_events.append((e0, e1))
         else:
             cur.wait_stream(self._comm_stream)
-
-    LOG_KEEP = 4096
-
-    def _log_loss(self):
-        """``self.logs['IL_loss']`` (agent.py:885): one entry per rollout.  Device scalars (a copy: ``loss_total`` is
-        rewritten every step), converted lazily by ``il_losses()``; bounded."""
-        log = self.logs["IL_loss"]
-        log.append(self.loss_total.clone())
-        if len(log) > self.LOG_KEEP:
-            del log[: len(log) - self.LOG_KEEP]
-
-    def il_losses(self):
-        """The logged losses as host floats (one synchronisation)."""
-        log = self.logs["IL_loss"]
-        return torch.stack([x.reshape(()) for x in log]).cpu().tolist() if log else []
-
-    def train_iteration(self, teacher_batch, student_batch=None, sync_loss=False, feedback="student",
-                        nss_w_weighting=1):
-        """One iteration of ``train`` (agent.py:225-251).  ``feedback='student'`` (the reference's recipe): the
-        teacher-feedback rollout with ``train_ml = args.ml_weight`` and **nss_w = 0** (agent.py:232), then the
-        student-feedback rollout with ``nss_w = args.nss_w * nss_w_weighting`` (agent.py:235); the two add their
-        losses, ONE backward's worth of gradients (accumulated over both), clip, one step of every optimiser.
-        ``feedback='teacher'``: the teacher rollout alone with ``train_ml = args.teacher_weight`` and the NSS term
-        (agent.py:229).  ``student_batch`` comes from ``student_batch()``.  Returns the summed loss."""
-        nss = float(getattr(self.args, "nss_w", 1.0)) * nss_w_weighting
-        if feedback == "teacher":
-            tot = self.train_rollout_step(teacher_batch, nss_w=nss,
-                                          train_ml=float(getattr(self.args, "teacher_weight", 1.0))).clone()
-        elif feedback == "student":
-            l1 = self.train_rollout_step(teacher_batch, step=False, nss_w=0.0).clone()
-            tot = l1 + self.train_rollout_step(student_batch, zero=False, nss_w=nss)
-        else:
-            raise ValueError("Invalid feedback option")
-        return float(tot.item()) if sync_loss else tot
-
-    def train_rollout_step(self, batch, sync_loss=False, zero=True, step=True, nss_w=None, train_ml=None,
-                           collect=None, bn_per_step=None):
-        with self._weights(nss_w, train_ml):
-            return self._train_rollout_step(batch, sync_loss, zero, step, collect, bn_per_step)
 
     def _train_rollout_step(self, batch, sync_loss=False, zero=True, step=True, collect=None, bn_per_step=None):
         """One teacher-forced training ROLLOUT (agent.py:580-760, 883-885, 245-251) as one batched pass: the loss is
@@ -464,48 +400,11 @@ class NavCMTAgent:
             xb = dict(att=torch.empty((BT, 224, 224), dtype=torch.uint8, device=dev),
                       d_frames=torch.empty((BT, 512, 49), dtype=torch.float32, device=dev))
             self._bufs[key] = xb
-        att = batch.get("att")
-        if "images" in batch:
-            x = batch["images"]
-        else:
-            r = self.renderer
-            ti = batch.get("tile_idx")
-            ti = None if ti is None else ti.reshape(-1)
-            minv = r.homography(batch["corners_px"].view(BT, 4, 2))
-            r.render(None, ti, views=False, norm_nhwc=True, minv=minv, out={"norm_nhwc": bufs["x"]})
-            n += 2
-            x = bufs["x"]
-            if att is None and self.nss_w != 0:
-                r.render(None, ti, views=False, att=True, minv=minv, out={"att": xb["att"]})
-                att = xb["att"]
-                n += 1
+        x, att, k = render_rollout_views(self, batch, BT, bufs["x"], xb["att"])
+        n += k
         vm, et = self.vision_model, self.vln_model
-        if bn_per_step is None:
-            bn_per_step = bool(getattr(self.args, "bn_per_step", False))
-        if bn_per_step:
-            # the reference's loop: Darknet sees the B views of one time step per call (agent.py:593)
-            key = ("rollout_steps", B, T)
-            sb = self._bufs.get(key)
-            if sb is None:
-                sb = dict(x=[torch.empty((B, 224, 224, 4), dtype=torch.bfloat16, device=dev) for _ in range(T)],
-                          f=torch.empty((B, 512, 7, 7), dtype=torch.float32, device=dev),
-                          df=torch.empty((B, 512, 7, 7), dtype=torch.float32, device=dev))
-                self._bufs[key] = sb
-            tengs = [vm.engine(B, 224, 224, dev, slot=1 + t) for t in range(T)]
-            l0 = sum(e.launches for e in tengs)
-            x5 = x.view(B, T, 224, 224, 4)
-            f5 = bufs["frames"].view(B, T, 512, 49)
-            for t in range(T):
-                sb["x"][t].copy_(x5[:, t])
-                DN._trunk_forward(vm, tengs[t], sb["x"][t], True, out=sb["f"])
-                f5[:, t].copy_(sb["f"].view(B, 512, 49))
-            n += 2 * T
-            teng = tengs[0]
-        else:
-            tengs = None
-            teng = vm.engine(BT, 224, 224, dev)
-            l0 = teng.launches
-            DN._trunk_forward(vm, teng, x, True, out=bufs["frames"])
+        teng, tengs, l0, k = rollout_trunk_forward(self, x, B, T, bufs["frames"], bn_per_step)
+        n += k
         # ---- step t: the encoder over the history [:t+1], its loss, and straight back (the loss is a sum over steps,
         #      so only one step's activations are alive at a time; every step adds into the one gradient arena) ----
         frames = bufs["frames"].view(B, T, 512, 49)
@@ -573,22 +472,8 @@ class NavCMTAgent:
                                if li in buckets else None)
         else:
             hook = None
-        if tengs is None:
-            DN._trunk_backward(vm, teng, bufs["d_frames"].view(-1, 512, 7, 7), after_layer=hook,
-                               flush_layers=set(buckets) if dp else None)
-            trunk_launches = teng.launches - l0
-        else:
-            # one backward pass per time step, each through the activations of its own forward pass; the parameter
-            # gradients accumulate, the last pass releases the data-parallel buckets
-            sb = self._bufs[("rollout_steps", B, T)]
-            d5 = bufs["d_frames"].view(B, T, 512, 49)
-            for t in reversed(range(T)):
-                sb["df"].view(B, 512, 49).copy_(d5[:, t])
-                last = (t == 0)
-                DN._trunk_backward(vm, tengs[t], sb["df"], after_layer=hook if last else None,
-                                   flush_layers=set(buckets) if (dp and last) else None)
-            n += T
-            trunk_launches = sum(e.launches for e in tengs) - l0
+        trunk_launches = rollout_trunk_backward(self, teng, tengs, l0, bufs["d_frames"], B, T, after_layer=hook,
+                                                flush_layers=set(buckets) if dp else None)
         if dp:
             self._wait_comm()
         if step:
@@ -606,28 +491,14 @@ class NavCMTAgent:
         result is a ``train_rollout_step`` batch.  ``batch`` as for ``rollout_greedy``; returns the training batch
         (device tensors; ``lenths`` from the steps each sample was alive)."""
         res = self.rollout_greedy(batch, max_action_len=max_action_len)
-        T = int(res["steps"])
-        corners = res["corners"][:T]                                   # [T,B,4,2] gps
-        B = corners.shape[1]
-        ended_before = torch.zeros((T, B), dtype=torch.uint8, device=self.device)
-        ended_before[1:] = res["ended"][:T - 1]
-        tgt_xy, tgt_alt, prog = self.teacher_action(corners.reshape(T * B, 4, 2),
-                                                    [gt_path_corners[k % B] for k in range(T * B)],
-                                                    ended_before.reshape(-1), feedback="student")
-        geo = batch["geo"].contiguous()
-        px = torch.empty((T * B, 4, 2), dtype=torch.int32, device=self.device)
-        _lib.call("avdn_gps_to_pixels", _lib.ptr(corners.reshape(T * B, 4, 2).contiguous()),
-                  _lib.ptr(geo.repeat(T, 1).contiguous()), T * B, _lib.ptr(px))
+        out, ended_before, T = student_rollout_targets(self, batch, res, gt_path_corners)
         rad = res["directions"][:T].float() / 180 * PI_REF
         alive = (ended_before == 0).cpu().numpy()
         lens = np.cumsum(alive, axis=0).T                              # [B,T]: history length seen at step t
-        tb = lambda a: a.view(T, B, *a.shape[1:]).transpose(0, 1).contiguous()
-        ti = batch.get("tile_idx")
-        return dict(corners_px=tb(px), tile_idx=None if ti is None else ti.view(B, 1).expand(B, T).contiguous(),
-                    lang=batch["lang"], lang_cls=batch["lang_cls"],
-                    directions=torch.stack([torch.sin(rad), torch.cos(rad)], -1).transpose(0, 1).contiguous(),
-                    gt_xy=tb(tgt_xy.float()), gt_alt=tb(tgt_alt.float()), gt_prog=tb(prog.float()),
-                    lenths=np.maximum(lens, 1).tolist())
+        out.update(lang=batch["lang"], lang_cls=batch["lang_cls"],
+                   directions=torch.stack([torch.sin(rad), torch.cos(rad)], -1).transpose(0, 1).contiguous(),
+                   lenths=np.maximum(lens, 1).tolist())
+        return out
 
     # ----------------------------------------------------------------- inference
     STOP_THRESHOLD = 0.5               # agent.py:738-745 (the LSTM agent uses 0.25)
@@ -831,42 +702,6 @@ class NavCMTAgent:
                         traj["path_corners"].append((c_host[t + 1, i], d_host[t + 1, i]))
                 self.results[traj["instr_id"]] = traj
         return self.results
-
-    def teacher_action(self, corners, gt_path_corners, ended, feedback=None):
-        """``teacher_action`` (agent.py:386-507) for the whole batch on the device; ``feedback`` 'student' /
-        'teacher' (default ``self.feedback`` or 'student').
-        ``corners`` [B,4,2] f64 (lat,lng); ``gt_path_corners``: list (len B) of ``[n_i,4,2]`` arrays or a padded
-        ``[B,Pmax,4,2]`` tensor with ``gt_len``; ``ended`` [B].  Returns device tensors
-        ``(next_pos_ratio [B,2] f32, altitude [B] f32, progress [B] f32)`` -- the targets of ``output[:,0:2]``,
-        ``output[:,2]`` and ``output[:,3]`` (agent.py:655-671)."""
-        dev = self.device
-        c = torch.as_tensor(np.asarray(corners) if not torch.is_tensor(corners) else corners).to(dev, torch.float64).contiguous()
-        B = c.shape[0]
-        packed = isinstance(gt_path_corners, tuple) and len(gt_path_corners) == 2 and torch.is_tensor(gt_path_corners[0])
-        if isinstance(gt_path_corners, (list, tuple)) and not packed:
-            lens = [len(g) for g in gt_path_corners]
-            pmax = max(lens)
-            gt = np.zeros((B, pmax, 4, 2), dtype=np.float64)
-            for i, g in enumerate(gt_path_corners):
-                gt[i, :lens[i]] = np.asarray(g, dtype=np.float64)
-            gt_t = torch.from_numpy(gt).to(dev)
-            len_t = torch.tensor(lens, dtype=torch.int32, device=dev)
-        else:
-            gt_t, len_t = gt_path_corners
-            gt_t = gt_t.to(dev, torch.float64).contiguous()
-            len_t = len_t.to(dev, torch.int32).contiguous()
-            pmax = gt_t.shape[1]
-        e = torch.as_tensor(np.asarray(ended, dtype=np.uint8) if not torch.is_tensor(ended) else ended).to(dev, torch.uint8).contiguous()
-        ratio = torch.empty((B, 2), dtype=torch.float32, device=dev)
-        alt = torch.empty(B, dtype=torch.float32, device=dev)
-        prog = torch.empty(B, dtype=torch.float32, device=dev)
-        fb = feedback if feedback is not None else getattr(self, "feedback", "student")
-        if fb not in ("student", "teacher"):
-            raise ValueError("Invalid feedback option")
-        _lib.call("avdn_teacher_action", _lib.ptr(c), _lib.ptr(gt_t), int(pmax), _lib.ptr(len_t), _lib.ptr(e), B,
-                  int(fb == "teacher"), _lib.ptr(ratio), _lib.ptr(alt), _lib.ptr(prog))
-        self.launches += 1
-        return ratio, alt, prog
 
     # ------------------------------------------------------------ API helpers
     def NSS(self, sal, fix):

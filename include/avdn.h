@@ -401,7 +401,9 @@ int avdn_frame_attn_bwd(const float* frames, const float* lang_cls, const float*
                         const float* d_emb, float* d_frames, float* d_w_in, float* d_w_out, float* d_fc2_w,
                         float* d_fc2_b, avdn_stream_t stream);
 /* The same, also accumulating (+=) the gradient of the query into d_lang_cls [B,49] (NULL to skip): in the
- * reference lang_cls = linear_cls comes from the trained BERT head (src/xview_et/agent.py:527-543).          */
+ * reference lang_cls = linear_cls comes from the trained BERT head (src/xview_et/agent.py:527-543).
+ * fc2_w == NULL (ViT_LSTM's attention_layer_vision, vln_model.py:219, as in avdn_frame_attn_fwd): d_emb is read
+ * as d_e49 [B*T,49], the gradient of the attention output, and d_fc2_w / d_fc2_b may be NULL.                */
 int avdn_frame_attn_bwd_cls(const float* frames, const float* lang_cls, const float* w_in, const float* w_out,
                         const float* fc2_w, int B, int T, const float* attn, const float* wc, const float* e49,
                         const float* d_emb, float* d_frames, float* d_w_in, float* d_w_out, float* d_fc2_w,
@@ -616,6 +618,25 @@ int avdn_direction_embed(const float* deg, const float* w, const float* b, float
  * ctx [B,L,D], target [B,D] -> attn [B,L] (may be NULL), weighted [B,D] (row pitch ldw). */
 int avdn_lang_attn_fwd(const float* ctx, const float* target, int B, int L, int D, float* attn, float* weighted,
                        long long ldw, avdn_stream_t stream);
+/* Backward of avdn_lstm_cell (autograd of nn.LSTMCell's pointwise part, vln_model.py:224-236), from the saved
+ * pre-activations gates [B,4H] (order i,f,g,o), c_prev [B,H] or NULL (zero state of the first step), and the saved
+ * cell state c [B,H]; dh [B,H] has row pitch lddh (h lives inside a wider buffer); dc_next [B,H] or NULL (no
+ * gradient from a later step).  dgates [B,4H] is overwritten (it is the gradient of both bias vectors and the
+ * operand of the W_ih / W_hh gradients); dc_prev [B,H] is overwritten when c_prev is given, not written otherwise.
+ * dc_next and dc_prev may be the same buffer.                                                                  */
+int avdn_lstm_cell_bwd(const float* gates, const float* c_prev, const float* c, const float* dh, long long lddh,
+                       const float* dc_next, float* dgates, float* dc_prev, int B, int H, avdn_stream_t stream);
+/* Gradient of avdn_direction_embed's parameters (vln_model.py:228-229): d_w [N,2] += sum_s d_out[s] [sin, cos](a_s),
+ * d_b [N] += sum_s d_out[s], with a_s = deg[s] / 180 * 3.14159 in float32 and the same sin / cos as the forward.
+ * deg [B], d_out [B,N].                                                                                        */
+int avdn_direction_embed_bwd(const float* deg, const float* d_out, int B, int N, float* d_w, float* d_b,
+                             avdn_stream_t stream);
+/* Backward of avdn_lang_attn_fwd (SoftDotAttention(768) over the dialog tokens, vln_model.py:33-42): from ctx
+ * [B,L,D], target [B,D], the saved attn [B,L] and d_weighted [B,D] (row pitch lddw):
+ * d_target [B,D] is overwritten; d_ctx [B,L,D] (the gradient of lang_feature) is accumulated (+=), NULL to skip.
+ * Any L (2D + 2L floats of shared memory, at most 48 KB).                                                    */
+int avdn_lang_attn_bwd(const float* ctx, const float* target, const float* attn, const float* d_weighted,
+                       long long lddw, int B, int L, int D, float* d_target, float* d_ctx, avdn_stream_t stream);
 /* One rollout step of the simulator for B samples (xview_lstm/agent.py:607-626,700-730 and
  * move_view_corners, xview_et/agent.py:285-384), float64, one thread per sample:
  *   output [B,4] f32 -> normalise / clamp / discretise (as avdn_postprocess_waypoints);
