@@ -129,6 +129,7 @@ _SIGNATURES = {
     "avdn_loss": [c_void_p] * 7 + [c_int, c_f32, c_int, c_f64] + [c_void_p] * 4 + [c_void_p],
     "avdn_upsample_saliency": [c_void_p, c_int, c_void_p, c_void_p],
     "avdn_upsample_saliency_bwd": [c_void_p, c_int, c_void_p, c_void_p],
+    "avdn_saliency_metrics": [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p],
     "avdn_postprocess_waypoints": [c_void_p, c_void_p, c_int, c_f32] + [c_void_p] * 5 + [c_void_p],
     "avdn_sumsq": [c_void_p, c_i64, c_void_p, c_void_p],
     "avdn_adamw": [c_void_p] * 4 + [c_i64] + [c_f32] * 5 + [c_int, c_void_p, c_f32, c_f32, c_void_p],

@@ -361,17 +361,83 @@ __global__ void teacher_action_kernel(const double* __restrict__ corners, const 
   ratio[2 * i + 1] = (float)(r1 / m);
 }
 
+// Pixel (y, x) of the 8x8 -> 224x224 bilinear upsample of h [64].  Not inlined: upsample_kernel and
+// saliency_metrics_kernel run the same machine code, so their pixel values are bit-identical.
+__device__ __noinline__ float upsample_px(const float* h, int y, int x) {
+  int y0, y1, x0, x1; float ly, lx;
+  bilin_tap(y, &y0, &y1, &ly);
+  bilin_tap(x, &x0, &x1, &lx);
+  return (1.f - ly) * ((1.f - lx) * h[y0 * 8 + x0] + lx * h[y0 * 8 + x1]) +
+         ly * ((1.f - lx) * h[y1 * 8 + x0] + lx * h[y1 * 8 + x1]);
+}
+
 // 8x8 -> 224x224 bilinear upsample (pred_saliency of the reference API)
 __global__ void upsample_kernel(const float* __restrict__ h_sali, int B, float* __restrict__ pred) {
   const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   if (i >= (long long)B * NPX) return;
   const int b = (int)(i / NPX), r = (int)(i % NPX), y = r / VIEW, x = r - y * VIEW;
-  int y0, y1, x0, x1; float ly, lx;
-  bilin_tap(y, &y0, &y1, &ly);
-  bilin_tap(x, &x0, &x1, &lx);
-  const float* h = h_sali + b * 64;
-  pred[i] = (1.f - ly) * ((1.f - lx) * h[y0 * 8 + x0] + lx * h[y0 * 8 + x1]) +
-            ly * ((1.f - lx) * h[y1 * 8 + x0] + lx * h[y1 * 8 + x1]);
+  pred[i] = upsample_px(h_sali + b * 64, y, x);
+}
+
+// Sum of one double over the 256 threads of a CTA in a fixed order (xor tree per warp, then the 8 warps in order);
+// every thread gets the result.  `red` holds 8 doubles.
+__device__ __forceinline__ double block_sum_256(double v, double* red) {
+  v = warp_sum_d(v);
+  __syncthreads();                               // red may still be read from the previous call
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+  __syncthreads();
+  double t = 0.0;
+#pragma unroll
+  for (int w = 0; w < 8; ++w) t += red[w];
+  return t;
+}
+
+// Human-attention validation scores of one row per CTA (xview_et/agent.py:683-693 per sample): sal = the upsample of
+// h_sali[row], gt = att[row] / 255, p = clip(sal, 0, 1).  Two passes over the 224x224 pixels in float64: sums of sal,
+// gt, p, p*gt, then the centred sums of (sal - mean)^2 and (sal - mean)*gt (torch.std's unbiased variance and the
+// NSS numerator without the cancellation of a one-pass formula).
+__global__ void __launch_bounds__(256) saliency_metrics_kernel(const float* __restrict__ h_sali,
+                                                               const uint8_t* __restrict__ att, int nss_r,
+                                                               double* __restrict__ out) {
+  __shared__ float s_h[64];
+  __shared__ double s_red[8];
+  const int row = blockIdx.x, tid = threadIdx.x;
+  if (tid < 64) s_h[tid] = h_sali[(size_t)row * 64 + tid];
+  __syncthreads();
+  const uint8_t* f = att + (size_t)row * NPX;
+  double ss = 0.0, sg = 0.0, sp = 0.0, spg = 0.0;
+  for (int i = tid; i < NPX; i += 256) {
+    const int y = i / VIEW, x = i - y * VIEW;
+    const float s = upsample_px(s_h, y, x);
+    const double g = (double)f[i] / 255.0;
+    const double p = (double)fminf(fmaxf(s, 0.f), 1.f);
+    ss += (double)s; sg += g; sp += p; spg += p * g;
+  }
+  ss = block_sum_256(ss, s_red);
+  sg = block_sum_256(sg, s_red);
+  sp = block_sum_256(sp, s_red);
+  spg = block_sum_256(spg, s_red);
+  const double m = ss / NPX;
+  double dd = 0.0, dg = 0.0;
+  for (int i = tid; i < NPX; i += 256) {
+    const int y = i / VIEW, x = i - y * VIEW;
+    const double d = (double)upsample_px(s_h, y, x) - m;
+    dd += d * d; dg += d * ((double)f[i] / 255.0);
+  }
+  dd = block_sum_256(dd, s_red);
+  dg = block_sum_256(dg, s_red);
+  if (tid == 0) {
+    const double sd = sqrt(dd / (NPX - 1));
+    // sum_px n_sal * gt with n_sal = (sal - m) / sd, then nss_r's affine map (n/2 + 1 or n/2 - 1)
+    double sns = dg / sd;
+    if (nss_r == 1) sns = sns / 2 + sg;
+    else if (nss_r == -1) sns = sns / 2 - sg;
+    double* o = out + (size_t)row * 4;
+    o[0] = sp != 0.0 ? spg / sp : 0.0;
+    o[1] = sg > 0.0 ? spg / sg : 0.0;
+    o[2] = -(sns / (sg + 0.001));
+    o[3] = sg;
+  }
 }
 
 // adjoint of the upsample: d_h_sali[b][64] = sum_pixels w * d_pred.  One CTA per sample.
@@ -501,6 +567,16 @@ extern "C" int avdn_upsample_saliency(const float* h_sali, int B, float* pred, a
   const long long n = (long long)B * NPX;
   upsample_kernel<<<(unsigned)((n + 255) / 256), 256, 0, avdn::to_cuda(stream)>>>(h_sali, B, pred);
   return avdn::check_launch("avdn_upsample_saliency");
+}
+
+extern "C" int avdn_saliency_metrics(const float* h_sali, const uint8_t* att, int N, int nss_r, double* out,
+                                     avdn_stream_t stream) {
+  AVDN_REQUIRE(h_sali && att && out, "avdn_saliency_metrics: null pointer");
+  AVDN_REQUIRE(N >= 0, "avdn_saliency_metrics: N must be >= 0");
+  AVDN_REQUIRE(nss_r >= -1 && nss_r <= 1, "avdn_saliency_metrics: nss_r must be -1, 0 or 1");
+  if (N == 0) return AVDN_OK;
+  saliency_metrics_kernel<<<N, 256, 0, avdn::to_cuda(stream)>>>(h_sali, att, nss_r, out);
+  return avdn::check_launch("avdn_saliency_metrics");
 }
 
 extern "C" int avdn_upsample_saliency_bwd(const float* d_pred, int B, float* d_h_sali, avdn_stream_t stream) {

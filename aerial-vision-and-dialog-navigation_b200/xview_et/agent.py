@@ -119,19 +119,12 @@ class NavCMTAgent(RolloutTrainer):
         instead of ``lang`` / ``lang_cls``, and the gradients of both
         flow back into BERT and its head (one encoder pass per step = the reference's ``train_val_on_full`` mode,
         agent.py:530-538)."""
-        from ..models.bert import CustomBERTModel
-        self.lang_model = (lang_model if lang_model is not None else CustomBERTModel()).to(self.device)
-        self.lang_optimizer = FusedAdamW(self.lang_model.used_parameters(),
-                                         lr=lr if lr is not None else getattr(self.args, "lr", 1e-5))
-        self.lang_model._grad_arena = self.lang_optimizer.grads
-        self.lang_model._engines.clear()
-        self.lang_model.drop_rank = self.rank
-        self.optimizers = (self.et_optimizer, self.vision_model_optimizer, self.lang_optimizer)
+        lm = super().attach_lang_model(lang_model, lr)
         if self.world > 1:
             # every rank built (and randomly initialised) its own encoder: replicas start from rank 0's, like the
             # other two models in __init__
             parallel.broadcast_([self.lang_optimizer.p], 0, self.pg)
-        return self.lang_model
+        return lm
 
     def broadcast_parameters(self):
         """Replicas start identical (DDP semantics): rank 0's arenas and BN buffers."""
@@ -369,23 +362,7 @@ class NavCMTAgent(RolloutTrainer):
         leng = leng2 = None
         if "input_ids" in batch:
             # the language encoder runs once per rollout (agent.py:519-538) and collects the gradients of all steps
-            if self.lang_model is None:
-                raise RuntimeError("batch carries input_ids but no language model is attached (attach_lang_model)")
-            lm = self.lang_model
-            lm.train(not getattr(self.args, "no_dropout", False))
-            ids, am = batch["input_ids"], batch["attention_mask"]
-            leng = lm.engine(ids.shape[0], ids.shape[1], self.device)
-            leng.set_dropout(*lm.dropout_config())
-            l0l = leng.launches
-            seq, lin, _ = leng.forward(ids.long(), am)
-            n += leng.launches - l0l
-            if "cls_input_ids" in batch:
-                ids2, am2 = batch["cls_input_ids"], batch["cls_attention_mask"]
-                leng2 = lm.engine(ids2.shape[0], ids2.shape[1], self.device, slot=1)
-                leng2.set_dropout(*lm.dropout_config())
-                l0l = leng2.launches
-                _, lin, _ = leng2.forward(ids2.long(), am2)
-                n += leng2.launches - l0l
+            seq, lin, leng, leng2 = self._lang_train_forward(batch)
             batch = dict(batch, lang=seq, lang_cls=lin)
         dirs = batch["directions"].contiguous().float()
         B, T = dirs.shape[0], dirs.shape[1]
@@ -452,15 +429,7 @@ class NavCMTAgent(RolloutTrainer):
             et_launches += eng.launches - e0
         e0 = eng.launches - et_launches
         if leng is not None:
-            l0l = leng.launches
-            if leng2 is None:
-                leng.backward(d_lang_sum, d_cls_sum, None)
-            else:
-                leng.backward(d_lang_sum, None, None)
-                l1 = leng2.launches
-                leng2.backward(None, d_cls_sum, None)
-                n += leng2.launches - l1
-            n += leng.launches - l0l
+            self._lang_train_backward(leng, leng2, d_lang_sum, d_cls_sum)
         self._ctx = (teng, eng, bufs, l0, e0)
         dp = self.world > 1 and step               # gradients are reduced once, after the iteration's last rollout
         if dp:
@@ -641,68 +610,6 @@ class NavCMTAgent(RolloutTrainer):
             out.append(path)
         return out
 
-    def test(self, batches, env_name="no_name_provided", feedback="student", not_in_train=False, **kwargs):
-        """``agent.test`` (agent.py:191-206): greedy rollouts in eval mode, one trajectory dict per
-        episode in ``self.results[instr_id]`` -- the structure ``ANDHNavBatch.eval_metrics`` scores.
-
-        With ``self.env`` set to an ``ANDHNavBatch`` this is the reference's loop: ``batches`` is the data loader (it
-        fills ``self.env`` as it is iterated) and every item triggers ``self.rollout(not_in_train=True)``.  Otherwise:
-
-        Every batch is the ``rollout_greedy`` input dict plus host metadata: ``instr_id`` list[str],
-        ``gt_path_corners`` list of ``[n_i,4,2]`` arrays (optional: without it ``gt_progress`` is omitted, as for
-        the unseen test split, agent.py:655) and ``num_dia`` list[int] (optional).  ``gt_progress`` is the
-        reference's per-step IoU of the current view with the goal (``teacher_action``'s progress, agent.py:660,
-        721), evaluated for all steps of the batch in one ``avdn_teacher_action`` launch."""
-        self.feedback, self.env_name = feedback, env_name
-        self.results, self.losses = {}, []
-        if hasattr(self.env, "_get_obs"):
-            self.vln_model.eval(); self.vision_model.eval()
-            if self.lang_model is not None:
-                self.lang_model.eval()
-            self.loss = 0
-            for _ in batches:
-                for traj in self.rollout(not_in_train=True, **kwargs):
-                    self.loss = 0
-                    self.results[traj["instr_id"]] = traj
-            return self.results
-        for batch in batches:
-            meta = {k: batch[k] for k in ("instr_id", "gt_path_corners", "num_dia") if k in batch}
-            res = self.rollout_greedy({k: v for k, v in batch.items() if k not in meta}, **kwargs)
-            steps = int(res["steps"])
-            corners = res["corners"]                                       # [T+1,B,4,2]
-            B = corners.shape[1]
-            ended = res["ended"].cpu().numpy().astype(bool)
-            prog = None
-            gts = meta.get("gt_path_corners")
-            if gts is not None:
-                flat = corners[:steps].reshape(steps * B, 4, 2)
-                _, _, pr = self.teacher_action(flat, [gts[i % B] for i in range(steps * B)],
-                                               np.zeros(steps * B, dtype=np.uint8), feedback="student")
-                prog = pr.view(steps, B).cpu().numpy()
-            c_host = corners.cpu().numpy()
-            d_host = res["directions"].cpu().numpy()
-            out_host = res["output"].cpu().numpy()
-            for i in range(B):
-                traj = {"instr_id": meta["instr_id"][i] if "instr_id" in meta else f"{env_name}_{len(self.results)}",
-                        "path_corners": [(c_host[0, i], d_host[0, i])], "actions": [], "progress": []}
-                if "num_dia" in meta:
-                    traj["num_dia"] = int(meta["num_dia"][i])
-                if gts is not None:
-                    traj["gt_path_corners"] = gts[i]
-                    traj["gt_progress"] = []
-                alive = True
-                for t in range(steps):
-                    if alive:                                              # logged while the episode has not ended
-                        traj["actions"].append(out_host[t, i, :3].copy())
-                        traj["progress"].append(float(out_host[t, i, 3]))
-                        if prog is not None:
-                            traj["gt_progress"].append(float(prog[t, i]))
-                    alive = not ended[t, i]
-                    if alive:
-                        traj["path_corners"].append((c_host[t + 1, i], d_host[t + 1, i]))
-                self.results[traj["instr_id"]] = traj
-        return self.results
-
     # ------------------------------------------------------------ API helpers
     def NSS(self, sal, fix):
         """src/xview_et/agent.py:256-270 on device tensors (torch elementwise; off the hot
@@ -795,70 +702,6 @@ class NavCMTAgent(RolloutTrainer):
         return np.array(moved), (cur + angle) % 360
 
     # ------------------------------------------------- the reference's agent loop (drop-in signatures)
-    def _language_batch(self, items):
-        """agent.py:519-538: the dialog of every episode through the tokenizer -- ``instructions`` for the
-        transformer's language rows, ``pre_dialogs + instructions`` for ``linear_cls`` unless
-        ``args.train_val_on_full``.  Needs ``self.tokenizer`` (the reference's ``BertTokenizerFast``: any callable
-        ``tok(list[str], padding=True, return_tensors='pt')`` -> ``input_ids`` / ``attention_mask``) and an attached
-        language model."""
-        if self.lang_model is None or self.tokenizer is None:
-            raise RuntimeError("rollout() tokenises the dialogs and runs CustomBERTModel (agent.py:124-126,519-538): "
-                               "set agent.tokenizer and call attach_lang_model() first")
-        vis_only = bool(getattr(self.args, "vision_only", False))
-        texts = ["" if vis_only else it["instructions"] for it in items]
-        enc = self.tokenizer(texts, padding=True, return_tensors="pt")
-        out = {"input_ids": enc["input_ids"].to(self.device), "attention_mask": enc["attention_mask"].to(self.device)}
-        lang_inputs = texts
-        if not bool(getattr(self.args, "train_val_on_full", False)):
-            lang_inputs = [it["pre_dialogs"] + it["instructions"] for it in items]
-            enc2 = self.tokenizer(lang_inputs, padding=True, return_tensors="pt")
-            out["cls_input_ids"] = enc2["input_ids"].to(self.device)
-            out["cls_attention_mask"] = enc2["attention_mask"].to(self.device)
-        return out, lang_inputs
-
-    @torch.no_grad()
-    def _teacher_rollout_poses(self, corners0, dirs0, geo, gt_paths, T):
-        """The pose sequence of a teacher-feedback rollout (agent.py:580-770 with ``feedback == 'teacher'``): the
-        action of every step is the ground-truth action, so the sequence does not depend on the model.  Per step:
-        ``teacher_action`` (target waypoint / altitude / progress at the current view) and the simulator update with
-        that target -- stop once the ground-truth progress exceeds 0.5 or at the last step.  All on the device; the
-        host reads the stop flags once at the end.  Returns a dict of ``[T, B, ...]`` tensors and the step count."""
-        ptr, call = _lib.ptr, _lib.call
-        dev = self.device
-        B = corners0.shape[0]
-        f64, i32 = torch.float64, torch.int32
-        corners = corners0.to(dev, f64).contiguous().clone()
-        cur = dirs0.to(dev, f64).contiguous().clone()
-        ended = torch.zeros(B, dtype=torch.uint8, device=dev)
-        bounds = geo[:, :4].contiguous()
-        H = dict(corners=torch.empty((T + 1, B, 4, 2), dtype=f64, device=dev), dirs=torch.empty((T + 1, B), dtype=f64, device=dev),
-                 ended=torch.empty((T, B), dtype=torch.uint8, device=dev), xy=torch.empty((T, B, 2), device=dev),
-                 alt=torch.empty((T, B), device=dev), prog=torch.empty((T, B), device=dev))
-        ang = torch.empty(B, dtype=i32, device=dev); dist = torch.empty(B, dtype=f64, device=dev); alt_i = torch.empty(B, dtype=i32, device=dev)
-        gts = [gt_paths[i] for i in range(B)]
-        lens = [len(g) for g in gts]
-        gt = np.zeros((B, max(lens), 4, 2), dtype=np.float64)
-        for i, g in enumerate(gts):
-            gt[i, :lens[i]] = np.asarray(g, dtype=np.float64)
-        gt_pack = (torch.from_numpy(gt).to(dev), torch.tensor(lens, dtype=i32, device=dev))
-        for t in range(T):
-            H["corners"][t].copy_(corners); H["dirs"][t].copy_(cur)
-            xy, alt, prog = self.teacher_action(corners, gt_pack, ended, feedback="teacher")
-            H["xy"][t].copy_(xy); H["alt"][t].copy_(alt); H["prog"][t].copy_(prog)
-            out = torch.cat((xy, alt[:, None], prog[:, None]), 1).contiguous()
-            call("avdn_waypoint_step", ptr(out), ptr(corners), ptr(bounds), ptr(cur), ptr(ended), B,
-                 float(self.STOP_THRESHOLD), int(t == T - 1), ptr(ang), ptr(dist), ptr(alt_i))
-            H["ended"][t].copy_(ended)
-            self.launches += 8
-        H["corners"][T].copy_(corners); H["dirs"][T].copy_(cur)
-        e = H["ended"].cpu().numpy().astype(bool)
-        steps = T
-        for t in range(T):
-            if e[t].all():                                   # agent.py:773-774: early exit once every sample has ended
-                steps = t + 1
-                break
-        return H, steps
-
     def rollout(self, train_ml=None, not_in_train=False, nss_w=0, **kwargs):
         """Drop-in for ``NavCMTAgent.rollout`` (src/xview_et/agent.py:512-894) over ``self.env`` (an
         ``ANDHNavBatch`` whose ``batch`` / maps the data loader has filled): one rollout of the current batch under
@@ -873,40 +716,15 @@ class NavCMTAgent(RolloutTrainer):
         * ``not_in_train``: no gradients; student feedback is ``rollout_greedy``; teacher feedback additionally logs
           ``human_att_performance`` / ``nss`` per step (agent.py:683-693)."""
         env = self.env
-        items = list(env.batch)
-        B = len(items)
         dev = self.device
-        env._sync_maps()
         T = int(getattr(self.args, "max_action_len", 15))
-        lb, lang_inputs = self._language_batch(items)
-        gps0 = np.stack([np.asarray(it["gt_path_corners"][0], dtype=np.float64) for it in items])
-        _, geo_h, tidx_h = env._gather_poses(None, 0)
-        geo = torch.from_numpy(geo_h).to(dev)
-        tidx = torch.from_numpy(tidx_h).to(dev)
-        dirs0 = torch.tensor([float(it["angle"]) for it in items], dtype=torch.float64, device=dev)
-        gt_paths = [np.asarray(it["gt_path_corners"], dtype=np.float64) for it in items]
+        items, lb, gps0, geo, tidx, dirs0, gt_paths, traj = self._rollout_setup()
+        B = len(items)
         has_gt = "test" not in self.env_name
-        traj = []
-        for i, it in enumerate(items):
-            rounds = lang_inputs[i].split("[QUE]")
-            remove = sum(1 for r in rounds if "Yes" in r[0:5])
-            traj.append({"instr_id": it["map_name"] + "__" + it["route_index"], "num_dia": len(rounds) - remove,
-                         "path_corners": [(np.array(it["gt_path_corners"][0]), it["angle"])],
-                         "gt_path_corners": it["gt_path_corners"], "actions": [], "gt_actions": [], "gt_progress": [],
-                         "progress": []})
         prev_r, self.renderer = self.renderer, env.renderer
         try:
             if not_in_train and self.feedback == "student":
-                lm = self.lang_model
-                lm.eval()
-                with torch.no_grad():
-                    leng = lm.engine(lb["input_ids"].shape[0], lb["input_ids"].shape[1], dev)
-                    leng.set_dropout(*lm.dropout_config())
-                    seq, lin, _ = leng.forward(lb["input_ids"].long(), lb["attention_mask"])
-                    if "cls_input_ids" in lb:
-                        leng2 = lm.engine(lb["cls_input_ids"].shape[0], lb["cls_input_ids"].shape[1], dev, slot=1)
-                        leng2.set_dropout(*lm.dropout_config())
-                        _, lin, _ = leng2.forward(lb["cls_input_ids"].long(), lb["cls_attention_mask"])
+                seq, lin = self._lang_eval_forward(lb)
                 res = self.rollout_greedy(dict(corners_gps=torch.from_numpy(gps0).to(dev), directions=dirs0, geo=geo,
                                                tile_idx=tidx, lang=seq.float(), lang_cls=lin.float()), max_action_len=T)
                 steps = int(res["steps"])
@@ -936,15 +754,7 @@ class NavCMTAgent(RolloutTrainer):
                 # the student's own (no-grad, eval-mode) greedy rollout fixes the poses; the teacher supplies the
                 # target of every visited pose (agent.py:655-661)
                 with torch.no_grad():
-                    lm = self.lang_model
-                    lm.eval()
-                    leng = lm.engine(lb["input_ids"].shape[0], lb["input_ids"].shape[1], dev)
-                    leng.set_dropout(*lm.dropout_config())
-                    seq, lin, _ = leng.forward(lb["input_ids"].long(), lb["attention_mask"])
-                    if "cls_input_ids" in lb:
-                        leng2 = lm.engine(lb["cls_input_ids"].shape[0], lb["cls_input_ids"].shape[1], dev, slot=1)
-                        leng2.set_dropout(*lm.dropout_config())
-                        _, lin, _ = leng2.forward(lb["cls_input_ids"].long(), lb["cls_attention_mask"])
+                    seq, lin = self._lang_eval_forward(lb)
                     res = self.rollout_greedy(dict(corners_gps=torch.from_numpy(gps0).to(dev), directions=dirs0, geo=geo,
                                                    tile_idx=tidx, lang=seq.float().clone(), lang_cls=lin.float().clone()),
                                               max_action_len=T)
@@ -986,36 +796,10 @@ class NavCMTAgent(RolloutTrainer):
             self._last_rollout = dict(corners=corners, ended=ended, steps=steps, tgt_xy=tgt_xy, tgt_alt=tgt_alt,
                                       tgt_prog=tgt_prog, batch=batch, lenths=lens)
             self._log_traj(traj, torch.stack(outs).cpu().numpy(), tgt, ended_h, c_all.cpu().numpy(), d_all.cpu().numpy(), steps)
-            if train_ml is not None:
-                l = loss.clone()
-                self.loss = l if isinstance(self.loss, (int, float)) else self.loss + l
-                self.losses.append(l)
-            else:
-                self.losses.append(0.0)
+            self._add_rollout_loss(loss, train_ml)
         finally:
             self.renderer = prev_r
         return traj
-
-    @staticmethod
-    def _log_traj(traj, outs, tgt, ended, corners, dirs, steps):
-        """agent.py:637-653,725-770: per alive step the clipped prediction, the ground-truth action / progress and the
-        pose the simulator moved to."""
-        B = len(traj)
-        for i in range(B):
-            alive = True
-            for t in range(steps):
-                if alive:
-                    o = outs[t, i]
-                    m = max(abs(float(o[0])), abs(float(o[1])), 1.0)
-                    traj[i]["actions"].append([np.array([o[0] / m, o[1] / m], dtype=np.float32),
-                                               np.float32(min(1.0, max(0.0, float(o[2]))))])
-                    traj[i]["progress"].append(float(o[3]))
-                    if tgt is not None:
-                        traj[i]["gt_actions"].append([tgt[0][t, i].copy(), float(tgt[1][t, i])])
-                        traj[i]["gt_progress"].append(float(tgt[2][t, i]))
-                alive = not ended[t, i]
-                if alive:
-                    traj[i]["path_corners"].append((corners[t + 1, i].copy(), float(dirs[t + 1, i])))
 
     @torch.no_grad()
     def _eval_rollout(self, batch, traj, outs):
@@ -1027,16 +811,7 @@ class NavCMTAgent(RolloutTrainer):
         self.vision_model.eval()
         et = self.vln_model
         et.eval()
-        lm = self.lang_model
-        lm.eval()
-        ids, am = batch["input_ids"], batch["attention_mask"]
-        leng = lm.engine(ids.shape[0], ids.shape[1], dev)
-        leng.set_dropout(*lm.dropout_config())
-        seq, lin, _ = leng.forward(ids.long(), am)
-        if "cls_input_ids" in batch:
-            leng2 = lm.engine(batch["cls_input_ids"].shape[0], batch["cls_input_ids"].shape[1], dev, slot=1)
-            leng2.set_dropout(*lm.dropout_config())
-            _, lin, _ = leng2.forward(batch["cls_input_ids"].long(), batch["cls_attention_mask"])
+        seq, lin = self._lang_eval_forward(batch)
         lang, lang_cls = seq.float().contiguous(), lin.float().contiguous()
         dirs = batch["directions"].contiguous().float()
         B, T = dirs.shape[:2]
@@ -1088,36 +863,6 @@ class NavCMTAgent(RolloutTrainer):
                         traj[i].setdefault("nss", []).append(float(nss))
         return total
 
-    def train(self, loader, n_epochs, feedback="student", nss_w_weighting=1, **kwargs):
-        """Drop-in for ``NavCMTAgent.train`` (src/xview_et/agent.py:208-254): for every batch the loader yields (the
-        loader fills ``self.env`` as a side effect, as the reference's ``num_workers=0`` DataLoader does): zero the
-        gradients, one teacher rollout (``feedback='teacher'``) or a teacher rollout without the NSS term followed by
-        a student rollout (``'student'``), clip the ET gradients to 40, one step of every optimiser."""
-        self.vision_model.train(); self.vln_model.train()
-        if self.lang_model is not None:
-            self.lang_model.train()
-        self.losses = []
-        for epoch in range(1, n_epochs + 1):
-            for _ in loader:
-                for opt in self.optimizers:
-                    opt.zero_grad()
-                self.loss = 0
-                if feedback == "teacher":
-                    self.feedback = "teacher"
-                    self.rollout(train_ml=float(getattr(self.args, "teacher_weight", 1.0)), train_rl=False,
-                                 nss_w=float(getattr(self.args, "nss_w", 1.0)) * nss_w_weighting, **kwargs)
-                elif feedback == "student":
-                    self.feedback = "teacher"
-                    self.rollout(train_ml=float(getattr(self.args, "ml_weight", 0.2)), train_rl=False, nss_w=0, **kwargs)
-                    self.feedback = "student"
-                    self.rollout(train_ml=float(getattr(self.args, "ml_weight", 0.2)), train_rl=False,
-                                 nss_w=float(getattr(self.args, "nss_w", 1.0)) * nss_w_weighting, **kwargs)
-                else:
-                    assert False
-                # (the reference calls self.loss.backward() here; the rollouts above already left their gradients in
-                #  the arenas)  gradient all-reduce, clip (ET only, agent.py:247), step
-                self._reduce_and_step()
-
     def _reduce_and_step(self):
         if self.world > 1:
             for opt in self.optimizers:
@@ -1129,39 +874,10 @@ class NavCMTAgent(RolloutTrainer):
 
     # ------------------------------------------------------------- checkpoints
     def _checkpoint_items(self):
-        items = [("vision_model", self.vision_model, self.vision_model_optimizer),
-                 ("vln_model", self.vln_model, self.et_optimizer)]
+        """agent.py:899-916: vision_model, vln_model and (when attached) lang_model; optimiser moments in the
+        flat-arena format (``RolloutTrainer.save`` / ``load``)."""
+        items = [("vision_model", self.vision_model, self.vision_model_optimizer, None),
+                 ("vln_model", self.vln_model, self.et_optimizer, None)]
         if self.lang_model is not None:
-            items.insert(0, ("lang_model", self.lang_model, self.lang_optimizer))
+            items.insert(0, ("lang_model", self.lang_model, self.lang_optimizer, None))
         return items
-
-    def save(self, epoch, path):
-        """agent.py:899-916: vision_model, vln_model and (when attached) lang_model."""
-        d = os.path.dirname(path)
-        if d:
-            os.makedirs(d, exist_ok=True)
-        states = {}
-        for name, model, opt in self._checkpoint_items():
-            states[name] = {"epoch": epoch + 1, "state_dict": model.state_dict(),
-                            "optimizer": {"m": opt.m.clone(), "v": opt.v.clone(), "step": opt.step_count}}
-        torch.save(states, path)
-
-    def load(self, path):
-        """agent.py:918-940: parameters (and optimiser moments when ``args.resume_optimizer``)."""
-        states = torch.load(path, map_location=self.device)
-        for name, model, opt in self._checkpoint_items():
-            if name not in states:
-                continue
-            state = model.state_dict()                       # tensors alias the arena: copy IN PLACE
-            with torch.no_grad():
-                for k, v in states[name]["state_dict"].items():
-                    if k in state:
-                        state[k].copy_(v)
-            if getattr(self.args, "resume_optimizer", False):
-                o = states[name].get("optimizer", {})
-                if "m" not in o:
-                    raise ValueError(f"checkpoint '{name}': optimiser state is not in the flat-arena format this agent "
-                                     "writes ({'m', 'v', 'step'}); torch per-parameter optimiser states (the reference's "
-                                     "format) cannot be resumed -- load with resume_optimizer=False")
-                opt.m.copy_(o["m"]); opt.v.copy_(o["v"]); opt.step_count = int(o["step"])
-        return states.get("vln_model", {}).get("epoch", 0) - 1

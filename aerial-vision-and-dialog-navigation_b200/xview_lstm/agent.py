@@ -1,6 +1,8 @@
 """``NavCMTAgent`` of the LSTM baseline (mirror of src/xview_lstm/agent.py, hot-path subset): greedy
-waypoint-rollout inference (BASELINE config 5) and teacher-forced training (``train_rollout_step``,
-``student_batch``, ``train_iteration``: the ET agent's batch-level training API, ``agent_common.RolloutTrainer``).
+waypoint-rollout inference (BASELINE config 5), teacher-forced training (``train_rollout_step``,
+``student_batch``, ``train_iteration``: the ET agent's batch-level training API, ``agent_common.RolloutTrainer``),
+and the reference's agent loop with its signatures: ``attach_lang_model``, ``rollout(train_ml, not_in_train, nss_w)``,
+``train(loader, n_epochs, feedback, nss_w_weighting)``, ``test(loader, ...)``, ``save`` / ``load``.
 
 ``rollout_greedy`` is the student-feedback loop of ``rollout`` (src/xview_lstm/agent.py:518-750)
 with every per-step stage on the device and no host round trip inside the loop:
@@ -16,17 +18,26 @@ agent.py:527-543) is an input of the path (SURVEY.md §8f N1).
 Training: one ``FusedAdamW`` over ``vln_model.used_parameters()`` (gradients clipped to a global norm of 40) and one
 over the trunk (unclipped), built here before any rollout captures a CUDA graph of the trunk (the arenas re-home
 the parameter storage).  AdamW is elementwise, so two optimisers update as one would; the clipping mirrors the ET
-agent, which the in-tree record of the reference supports for ET only (DESIGN.md §8).
+agent, which the in-tree record of the reference supports for ET only (DESIGN.md §8).  With ``attach_lang_model``
+``CustomBERTModel`` is trained in the loop by a third, unclipped ``FusedAdamW``.
+
+Checkpoints (``save`` / ``load``, ``agent_common.RolloutTrainer``): a ``torch.save`` dict with the entries
+``vision_model`` (the trunk), ``vln_model`` (the ``ViT_LSTM`` state without the ``vision_model.*`` keys: the trunk is
+written once) and, when attached, ``lang_model``; each ``{'epoch', 'state_dict', 'optimizer': {'m', 'v', 'step'}}``
+with the flat AdamW arena of that model.  ``load`` also takes a ``vln_model`` entry holding a full
+``ViT_LSTM.state_dict()`` (the reference's layout: the trunk is a sub-module, agent.py:140-142); its
+``vision_model.*`` keys then load into the trunk.
 """
 from __future__ import annotations
 
 import os
 
+import numpy as np
 import torch
 
 from .. import _lib
 from ..agent_common import (RolloutTrainer, render_rollout_views, rollout_trunk_backward, rollout_trunk_forward,
-                            student_rollout_targets)
+                            steps_until_all_ended, student_rollout_targets)
 from ..env import ViewRenderer
 from ..models import dark_net as DN
 from ..models.dark_net import Darknet
@@ -37,6 +48,10 @@ STOP_THRESHOLD_STUDENT = 0.25          # src/xview_lstm/agent.py:705 (the ET age
 
 
 class NavCMTAgent(RolloutTrainer):
+    # stop threshold of the simulator on the progress output (agent.py:701,705): the student path's value, also used
+    # for the teacher path's ground-truth progress, whose value in the reference is unverified (DESIGN.md §8)
+    STOP_THRESHOLD = STOP_THRESHOLD_STUDENT
+
     def __init__(self, args, rank=0, device=None):
         if not torch.cuda.is_available():
             raise RuntimeError("NavCMTAgent needs a CUDA device (sm_100); there is no CPU fallback")
@@ -61,7 +76,11 @@ class NavCMTAgent(RolloutTrainer):
         self.vln_model._grad_arena = self.policy_optimizer.grads
         self.vision_model._grad_arena = self.vision_model_optimizer.grads
         self.optimizers = (self.policy_optimizer, self.vision_model_optimizer)
+        self.lang_model, self.lang_optimizer = None, None     # attach_lang_model
+        self.tokenizer = getattr(args, "tokenizer", None)     # BertTokenizerFast in the reference (agent.py:124)
         self.feedback = "student"
+        self.env_name = ""
+        self.loss = 0
         self.logs = {"IL_loss": []}
         self.loss_total = torch.zeros(1, dtype=torch.float64, device=self.device)
         self.renderer = ViewRenderer(self.device)
@@ -148,6 +167,18 @@ class NavCMTAgent(RolloutTrainer):
                     output=bf["output_hist"], angle=bf["angle"], altitude=bf["altitude"], dist=bf["dist"])
 
     # ------------------------------------------------------------------ training
+    def _rollout_bufs(self, B, T):
+        """Views, attention maps and trunk features of the B*T poses of a rollout."""
+        key = ("rollout_train", B, T)
+        tb = self._bufs.get(key)
+        if tb is None:
+            dev, BT = self.device, B * T
+            tb = dict(x=torch.empty((BT, 224, 224, 4), dtype=torch.bfloat16, device=dev),
+                      att=torch.empty((BT, 224, 224), dtype=torch.uint8, device=dev),
+                      frames=torch.empty((BT, NCH, 7, 7), dtype=torch.float32, device=dev))
+            self._bufs[key] = tb
+        return tb
+
     def _train_rollout_step(self, batch, sync_loss=False, zero=True, step=True, collect=None, bn_per_step=None):
         """One teacher-forced training rollout (src/xview_lstm/agent.py:546-550,592-602,636; ``train_rollout_step``):
         the B*T views of the given poses are rendered and pushed through the train-mode trunk (one pass over all of
@@ -160,25 +191,28 @@ class NavCMTAgent(RolloutTrainer):
         ``batch``: ``corners_px`` i32 [B,T,4,2] (or ``images`` bf16 [B*T,224,224,4]), ``tile_idx`` i32 [B,T] | None,
         ``lang_feature`` [B,L,768], ``cls_hidden`` [B,49], ``directions`` [B,T] (headings in DEGREES),
         ``gt_xy`` [B,T,2], ``gt_alt`` / ``gt_prog`` [B,T], optional ``att`` u8 [B,T,224,224] (default: rendered
-        from the poses when ``nss_w != 0``).  ``zero`` / ``step`` / ``collect`` as in the ET agent."""
+        from the poses when ``nss_w != 0``).  ``zero`` / ``step`` / ``collect`` as in the ET agent.
+        With an attached language model the batch may carry ``input_ids`` / ``attention_mask`` (and optionally
+        ``cls_input_ids`` / ``cls_attention_mask``) instead of ``lang_feature`` / ``cls_hidden``: BERT runs once per
+        rollout in train mode, its sequence output is ``lang_feature`` and its ``linear_cls`` is ``cls_hidden``
+        (agent.py:527-543), and the gradients of both, summed over the T steps, go through one BERT backward (two
+        with the cls pass) into the language arena."""
         deg = batch["directions"].contiguous().float()
         B, T = deg.shape
         BT = B * T
-        lang, cls = batch["lang_feature"].contiguous().float(), batch["cls_hidden"].contiguous().float()
-        L = lang.shape[1]
         dev = self.device
         n = 0
         if zero:
             for opt in self.optimizers:
                 opt.zero_grad()
             n += 2
-        key = ("rollout_train", B, T)
-        tb = self._bufs.get(key)
-        if tb is None:
-            tb = dict(x=torch.empty((BT, 224, 224, 4), dtype=torch.bfloat16, device=dev),
-                      att=torch.empty((BT, 224, 224), dtype=torch.uint8, device=dev),
-                      frames=torch.empty((BT, NCH, 7, 7), dtype=torch.float32, device=dev))
-            self._bufs[key] = tb
+        leng = leng2 = None
+        if "input_ids" in batch:
+            seq, lin, leng, leng2 = self._lang_train_forward(batch)
+            batch = dict(batch, lang_feature=seq, cls_hidden=lin)
+        lang, cls = batch["lang_feature"].contiguous().float(), batch["cls_hidden"].contiguous().float()
+        L = lang.shape[1]
+        tb = self._rollout_bufs(B, T)
         x, att, k = render_rollout_views(self, batch, BT, tb["x"], tb["att"])
         n += k
         vln, vm = self.vln_model, self.vision_model
@@ -197,7 +231,13 @@ class NavCMTAgent(RolloutTrainer):
         n += 5
         if collect is not None:
             collect.extend(eng.output[t].clone() for t in range(T))
-        eng.backward()
+        if leng is None:
+            eng.backward()
+        else:
+            d_lang = torch.zeros((B, L, 768), dtype=torch.float32, device=dev)
+            d_cls = torch.zeros((B, 49), dtype=torch.float32, device=dev)
+            eng.backward(d_lang, d_cls)
+            self._lang_train_backward(leng, leng2, d_lang, d_cls)
         trunk_launches = rollout_trunk_backward(self, teng, tengs, l0, eng.d_frames, B, T)
         self._ctx = (teng, tengs, eng, tb)
         if step:
@@ -235,3 +275,136 @@ class NavCMTAgent(RolloutTrainer):
                     path.append((corners[t + 1, i], dirs[t + 1, i]))
             out.append(path)
         return out
+
+    # ------------------------------------------------- the reference's agent loop (drop-in signatures)
+    def rollout(self, train_ml=None, not_in_train=False, nss_w=0, **kwargs):
+        """Drop-in for ``NavCMTAgent.rollout`` (src/xview_lstm/agent.py:518-894) over ``self.env`` (an
+        ``ANDHNavBatch`` whose ``batch`` / maps the data loader has filled): one rollout of the current batch under
+        ``self.feedback``; returns the list of trajectory dicts the reference returns.
+
+        * Poses: teacher feedback from the ground-truth actions (``_teacher_rollout_poses``), student feedback from a
+          no-grad greedy rollout on BERT's eval-mode features, with the ``teacher_action`` target of every pose.  The
+          loop stops after the step at which every sample has ended (agent.py:773-774).
+        * Training (``not_in_train`` false): ``train_rollout_step`` over the poses with BERT in train mode -- the loss
+          ``ml_loss * train_ml / B`` is added to ``self.loss`` and the gradients to the arenas (the reference's
+          ``self.loss.backward()`` in ``train``; ``train`` then only clips and steps).  The LSTM has no ``lenths``: a
+          sample that has stopped keeps stepping on its final pose, as in the reference.
+        * ``not_in_train``: no gradients; student feedback logs the greedy rollout; teacher feedback also logs
+          ``human_att_performance`` / ``nss`` per step (``_eval_rollout``)."""
+        env = self.env
+        dev = self.device
+        T = int(getattr(self.args, "max_action_len", 20))
+        items, lb, gps0, geo, tidx, dirs0, gt_paths, traj = self._rollout_setup()
+        B = len(items)
+        has_gt = "test" not in self.env_name
+        prev_r, self.renderer = self.renderer, env.renderer
+        try:
+            if self.feedback == "teacher":
+                H, steps = self._teacher_rollout_poses(torch.from_numpy(gps0), dirs0, geo, gt_paths, T)
+                corners, ended, heads = H["corners"][:steps], H["ended"][:steps], H["dirs"][:steps]
+                tgt_xy, tgt_alt, tgt_prog = H["xy"][:steps], H["alt"][:steps], H["prog"][:steps]
+                c_all, d_all = H["corners"], H["dirs"]
+            elif self.feedback == "student":
+                seq, lin = self._lang_eval_forward(lb)
+                res = self.rollout_greedy(dict(corners_gps=torch.from_numpy(gps0).to(dev), directions=dirs0, geo=geo,
+                                               tile_idx=tidx, lang_feature=seq.float().clone(),
+                                               cls_hidden=lin.float().clone()), max_action_len=T)
+                steps = steps_until_all_ended(res["ended"])
+                corners, ended, heads = res["corners"][:steps], res["ended"][:steps], res["directions"][:steps]
+                c_all, d_all = res["corners"], res["directions"]
+                tgt_xy = tgt_alt = tgt_prog = None
+                if has_gt or not not_in_train:
+                    # the teacher's target at every visited pose (agent.py:655-661)
+                    eb = torch.zeros((steps, B), dtype=torch.uint8, device=dev)
+                    eb[1:] = ended[:steps - 1]
+                    xy, alt, pr = self.teacher_action(corners.reshape(steps * B, 4, 2),
+                                                      [gt_paths[k % B] for k in range(steps * B)], eb.reshape(-1),
+                                                      feedback="student")
+                    tgt_xy, tgt_alt, tgt_prog = xy.view(steps, B, 2), alt.view(steps, B), pr.view(steps, B)
+            else:
+                raise SystemExit("Invalid feedback option")
+            ended_h = ended.cpu().numpy().astype(bool)
+            tgt = (tgt_xy.cpu().numpy(), tgt_alt.cpu().numpy(), tgt_prog.cpu().numpy()) if has_gt else None
+            if not_in_train and self.feedback == "student":
+                self._log_traj(traj, res["output"][:steps].cpu().numpy(), tgt, ended_h, c_all.cpu().numpy(),
+                               d_all.cpu().numpy(), steps)
+                return traj
+            px = torch.empty((steps * B, 4, 2), dtype=torch.int32, device=dev)
+            _lib.call("avdn_gps_to_pixels", _lib.ptr(corners.reshape(steps * B, 4, 2).contiguous()),
+                      _lib.ptr(geo.repeat(steps, 1).contiguous()), steps * B, _lib.ptr(px))
+            tb = lambda a: a.reshape(steps, B, *a.shape[2:]).transpose(0, 1).contiguous()
+            batch = dict(lb, corners_px=tb(px.view(steps, B, 4, 2)), tile_idx=tidx.view(B, 1).expand(B, steps).contiguous(),
+                         directions=tb(heads.float()), gt_xy=tb(tgt_xy.float()), gt_alt=tb(tgt_alt.float()),
+                         gt_prog=tb(tgt_prog.float()))
+            outs = []
+            if not_in_train:
+                loss = self._eval_rollout(batch, traj, outs)
+            else:
+                loss = self.train_rollout_step(batch, zero=False, step=False, nss_w=float(nss_w),
+                                               train_ml=train_ml if train_ml is not None else 0.0, collect=outs,
+                                               bn_per_step=bool(getattr(self.args, "bn_per_step", True)))
+            # what the rollout was made of (inspection / tests): poses, stop flags, targets, the training batch
+            self._last_rollout = dict(corners=corners, ended=ended, steps=steps, tgt_xy=tgt_xy, tgt_alt=tgt_alt,
+                                      tgt_prog=tgt_prog, batch=batch)
+            self._log_traj(traj, torch.stack(outs).cpu().numpy(), tgt, ended_h, c_all.cpu().numpy(), d_all.cpu().numpy(),
+                           steps)
+            self._add_rollout_loss(loss, train_ml)
+        finally:
+            self.renderer = prev_r
+        return traj
+
+    @torch.no_grad()
+    def _eval_rollout(self, batch, traj, outs):
+        """``not_in_train`` with teacher feedback (validation of the human-attention head, agent.py:673-693): trunk
+        and policy in eval mode over the given poses (the T policy steps in one ``train_engine`` forward with p = 0),
+        the loss of every step, and for every step and every sample with a non-empty fixation map precision / recall
+        of the clipped saliency map and its NSS -- all T*B rows scored by one ``avdn_saliency_metrics`` launch and
+        read back in one copy.  Appends the per-step outputs to ``outs``; returns the loss."""
+        ptr = _lib.ptr
+        dev = self.device
+        vm, vln = self.vision_model, self.vln_model
+        vm.eval()
+        vln.eval()
+        seq, lin = self._lang_eval_forward(batch)
+        lang, cls = seq.float().contiguous(), lin.float().contiguous()
+        deg = batch["directions"].contiguous().float()
+        B, T = deg.shape
+        BT, L = B * T, lang.shape[1]
+        tb = self._rollout_bufs(B, T)
+        r = self.renderer
+        ti = batch["tile_idx"].reshape(-1)
+        minv = r.homography(batch["corners_px"].view(BT, 4, 2))
+        r.render(None, ti, views=False, norm_nhwc=True, minv=minv, out={"norm_nhwc": tb["x"]})
+        r.render(None, ti, views=False, att=True, minv=minv, out={"att": tb["att"]})
+        teng = vm.engine(BT, 224, 224, dev)
+        DN._trunk_forward(vm, teng, tb["x"], False, out=tb["frames"])
+        eng = vln.train_engine(B, L, T, dev)
+        eng.forward(tb["frames"].view(BT, NCH, NSP), deg, cls, lang, 0.0, 0)
+        tr = lambda a: a.float().transpose(0, 1).contiguous()          # [B,T,...] -> step-major [T,B,...]
+        att_t = tb["att"].view(B, T, 224, 224).transpose(0, 1).contiguous()
+        nss_r = int(getattr(self.args, "nss_r", 0))
+        total = torch.zeros(1, dtype=torch.float64, device=dev)
+        eng.loss(tr(batch["gt_xy"]), tr(batch["gt_alt"]), tr(batch["gt_prog"]), att_t, self.nss_w, nss_r,
+                 float(self.train_ml) / B, total)
+        outs.extend(eng.output[t].clone() for t in range(T))
+        metrics = torch.empty((T, B, 4), dtype=torch.float64, device=dev)
+        _lib.call("avdn_saliency_metrics", ptr(eng.h_sali), ptr(att_t), BT, nss_r, ptr(metrics))
+        self.launches += 5
+        mh = metrics.cpu().numpy()
+        for t in range(T):
+            for i in range(B):
+                if mh[t, i, 3] > 0:                          # the sample's fixation map is not empty
+                    traj[i].setdefault("human_att_performance", []).append([float(mh[t, i, 0]), float(mh[t, i, 1])])
+                    traj[i].setdefault("nss", []).append(float(mh[t, i, 2]))
+        self._ctx_eval = (eng, att_t)
+        return total
+
+    # ------------------------------------------------------------- checkpoints
+    def _checkpoint_items(self):
+        """The trunk, the policy (its ``vision_model.*`` keys are the trunk's: written once, under ``vision_model``)
+        and, when attached, the language model -- see the module docstring."""
+        items = [("vision_model", self.vision_model, self.vision_model_optimizer, None),
+                 ("vln_model", self.vln_model, self.policy_optimizer, ("vision_model.",))]
+        if self.lang_model is not None:
+            items.insert(0, ("lang_model", self.lang_model, self.lang_optimizer, None))
+        return items

@@ -573,6 +573,14 @@ int avdn_loss(const float* output, const float* h_sali, const float* gt_xy, cons
 int avdn_upsample_saliency(const float* h_sali, int B, float* pred, avdn_stream_t stream);
 /* adjoint: d_h_sali [B,64] = upsample^T d_pred [B,1,224,224] (overwrites). */
 int avdn_upsample_saliency_bwd(const float* d_pred, int B, float* d_h_sali, avdn_stream_t stream);
+/* Human-attention validation scores of N rows (xview_et/agent.py:683-693, evaluated per sample): with
+ * sal = avdn_upsample_saliency(h_sali[n]) (the same device code, bit-identical pixels), gt = att[n] / 255 and
+ * p = clip(sal, 0, 1), out[n] = (precision = sum p*gt / sum p (0 when sum p == 0), recall = sum p*gt / sum gt
+ * (0 when sum gt == 0), nss = NSS(sal, gt) of the row (agent.py:256-270: unbiased std, nss_r in {-1,0,1},
+ * sum gt + 0.001), fixation sum = sum gt).  h_sali [N,64] f32, att [N,224,224] u8, out [N,4] f64.
+ * float64 sums, one CTA per row, a fixed reduction order: results repeat bit for bit.                       */
+int avdn_saliency_metrics(const float* h_sali, const uint8_t* att, int N, int nss_r, double* out,
+                          avdn_stream_t stream);
 /* agent.py:637-653,738,745-752: normalise xy, clamp altitude / progress, discretise.
  *   output [B,4] f32, edge_len [B] f64 (= |c0-c1|) -> angle_deg [B] i32,
  *   dist [B] f64, altitude_m [B] i32, stop [B] u8, xy_norm [B,2] f32 (or NULL). */
