@@ -94,6 +94,7 @@ _SIGNATURES = {
     "avdn_dropout_bf16": [c_void_p, c_i64, c_f32, C.c_uint64, C.c_uint32, c_void_p],
     "avdn_dropout_f32": [c_void_p, c_void_p, c_i64, c_f32, C.c_uint64, C.c_uint32, c_void_p],
     "avdn_add_dropout_f32": [c_void_p, c_void_p, c_void_p, c_i64, c_f32, C.c_uint64, C.c_uint32, c_void_p],
+    "avdn_add_dropout_f32_at": [c_void_p, c_void_p, c_void_p, c_i64, c_i64, c_f32, C.c_uint64, C.c_uint32, c_void_p],
     "avdn_dropout_keep_scale": [c_void_p, c_i64, c_f32, C.c_uint64, C.c_uint32, c_void_p],
     "avdn_heads_fwd_drop": [c_void_p, c_int, c_int, c_int, c_int] + [c_void_p] * 12 + [c_f32, C.c_uint64, C.c_uint32,
                                                                                      c_void_p],

@@ -484,13 +484,7 @@ def rollout_trunk_forward(agent, x, B, T, frames_out, bn_per_step=None):
         l0 = teng.launches
         DN._trunk_forward(vm, teng, x, True, out=frames_out)
         return teng, None, l0, 0
-    key = ("rollout_steps", B, T)
-    sb = agent._bufs.get(key)
-    if sb is None:
-        sb = dict(x=[torch.empty((B, 224, 224, 4), dtype=torch.bfloat16, device=dev) for _ in range(T)],
-                  f=torch.empty((B, 512, 7, 7), dtype=torch.float32, device=dev),
-                  df=torch.empty((B, 512, 7, 7), dtype=torch.float32, device=dev))
-        agent._bufs[key] = sb
+    sb = rollout_step_bufs(agent, B, T)
     tengs = [vm.engine(B, 224, 224, dev, slot=1 + t) for t in range(T)]
     l0 = sum(e.launches for e in tengs)
     x5 = x.view(B, T, 224, 224, 4)
@@ -502,22 +496,38 @@ def rollout_trunk_forward(agent, x, B, T, frames_out, bn_per_step=None):
     return tengs[0], tengs, l0, 2 * T
 
 
-def rollout_trunk_backward(agent, teng, tengs, l0, d_frames, B, T, after_layer=None, flush_layers=None):
+def rollout_step_bufs(agent, B, T):
+    """Buffers of the per-step trunk passes of a rollout of B episodes and T steps: the views of every step, one
+    step's features and their gradient."""
+    key = ("rollout_steps", B, T)
+    sb = agent._bufs.get(key)
+    if sb is None:
+        dev = agent.device
+        sb = dict(x=[torch.empty((B, 224, 224, 4), dtype=torch.bfloat16, device=dev) for _ in range(T)],
+                  f=torch.empty((B, 512, 7, 7), dtype=torch.float32, device=dev),
+                  df=torch.empty((B, 512, 7, 7), dtype=torch.float32, device=dev))
+        agent._bufs[key] = sb
+    return sb
+
+
+def rollout_trunk_backward(agent, teng, tengs, l0, d_frames, B, T, after_layer=None, flush_layers=None, steps=None):
     """Backward of ``rollout_trunk_forward`` from ``d_frames`` [B*T,512,49]; parameter gradients accumulate into
     the trunk's arena.  With per-step passes every pass runs back through its own activations and the last one
-    (step 0) carries ``after_layer`` / ``flush_layers`` (the data-parallel buckets).  Returns the launches."""
+    (step 0) carries ``after_layer`` / ``flush_layers`` (the data-parallel buckets); ``steps`` (default T): only
+    the passes of the first ``steps`` steps ran (a rollout that ended early).  Returns the launches."""
     vm = agent.vision_model
     if tengs is None:
         DN._trunk_backward(vm, teng, d_frames.view(-1, 512, 7, 7), after_layer=after_layer, flush_layers=flush_layers)
         return teng.launches - l0
     sb = agent._bufs[("rollout_steps", B, T)]
     d5 = d_frames.view(B, T, 512, 49)
-    for t in reversed(range(T)):
+    steps = T if steps is None else int(steps)
+    for t in reversed(range(steps)):
         sb["df"].view(B, 512, 49).copy_(d5[:, t])
         last = (t == 0)
         DN._trunk_backward(vm, tengs[t], sb["df"], after_layer=after_layer if last else None,
                            flush_layers=flush_layers if last else None)
-    return T + sum(e.launches for e in tengs) - l0
+    return steps + sum(e.launches for e in tengs) - l0
 
 
 def student_rollout_targets(agent, batch, res, gt_path_corners):

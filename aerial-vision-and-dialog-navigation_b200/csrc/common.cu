@@ -48,7 +48,7 @@ bool pdl_enabled() {
 
 extern "C" const char* avdn_last_error_string(void) { return avdn::err_buf(); }
 
-extern "C" int avdn_abi_version(void) { return 10; }
+extern "C" int avdn_abi_version(void) { return 11; }
 
 extern "C" int avdn_device_supported(void) {
   int n = 0;

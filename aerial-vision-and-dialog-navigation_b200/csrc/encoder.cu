@@ -797,13 +797,15 @@ __global__ void __launch_bounds__(256) dropout_f32_kernel(float* __restrict__ x,
   }
 }
 
-// out = dropout'(a + b): the gradient entering a dropout site whose output fed two consumers
+// out = dropout'(a + b): the gradient entering a dropout site whose output fed two consumers.  Element i draws the
+// mask of element idx0 + i of its site, so a slice of a larger tensor gets that tensor's mask.
 __global__ void __launch_bounds__(256) add_dropout_f32_kernel(const float* __restrict__ a, const float* __restrict__ b,
-                                                              float* __restrict__ out, long long n, unsigned int dthr,
-                                                              float dscale, unsigned long long seed, unsigned int site) {
+                                                              float* __restrict__ out, long long n, unsigned long long idx0,
+                                                              unsigned int dthr, float dscale, unsigned long long seed,
+                                                              unsigned int site) {
   for (long long i = blockIdx.x * 256LL + threadIdx.x; i < n; i += (long long)gridDim.x * 256) {
     const float v = a[i] + (b ? b[i] : 0.f);
-    out[i] = (!dthr || avdn_drop_keep(seed, site, (unsigned long long)i, dthr)) ? v * dscale : 0.f;
+    out[i] = (!dthr || avdn_drop_keep(seed, site, idx0 + (unsigned long long)i, dthr)) ? v * dscale : 0.f;
   }
 }
 
@@ -991,15 +993,29 @@ extern "C" int avdn_dropout_f32(float* x, void* x16, long long n, float p, unsig
   return avdn::check_launch("avdn_dropout_f32");
 }
 
+static void add_dropout_f32_launch(const float* a, const float* b, float* out, long long n, long long idx0, float p,
+                                   unsigned long long seed, unsigned int site, avdn_stream_t stream) {
+  long long blocks = (n + 255) / 256;
+  if (blocks > 148 * 16) blocks = 148 * 16;
+  add_dropout_f32_kernel<<<(unsigned)blocks, 256, 0, avdn::to_cuda(stream)>>>(
+      a, b, out, n, (unsigned long long)idx0, avdn_drop_thresh(p), p == 0.f ? 1.f : drop_scale(p), seed, site);
+}
+
 extern "C" int avdn_add_dropout_f32(const float* a, const float* b, float* out, long long n, float p,
                                     unsigned long long seed, unsigned int site, avdn_stream_t stream) {
   AVDN_REQUIRE(a && out && n >= 0 && drop_ok(p), "avdn_add_dropout_f32: bad argument");
   if (n == 0) return AVDN_OK;
-  long long blocks = (n + 255) / 256;
-  if (blocks > 148 * 16) blocks = 148 * 16;
-  add_dropout_f32_kernel<<<(unsigned)blocks, 256, 0, avdn::to_cuda(stream)>>>(a, b, out, n, avdn_drop_thresh(p),
-                                                                            p == 0.f ? 1.f : drop_scale(p), seed, site);
+  add_dropout_f32_launch(a, b, out, n, 0, p, seed, site, stream);
   return avdn::check_launch("avdn_add_dropout_f32");
+}
+
+extern "C" int avdn_add_dropout_f32_at(const float* a, const float* b, float* out, long long n, long long idx0,
+                                       float p, unsigned long long seed, unsigned int site, avdn_stream_t stream) {
+  AVDN_REQUIRE(a && out, "avdn_add_dropout_f32_at: null pointer");
+  AVDN_REQUIRE(n >= 0 && idx0 >= 0 && drop_ok(p), "avdn_add_dropout_f32_at: bad argument");
+  if (n == 0) return AVDN_OK;
+  add_dropout_f32_launch(a, b, out, n, idx0, p, seed, site, stream);
+  return avdn::check_launch("avdn_add_dropout_f32_at");
 }
 
 extern "C" int avdn_dropout_keep_scale(float* out, long long n, float p, unsigned long long seed, unsigned int site,

@@ -133,59 +133,127 @@ class _TrainEngine:
         self.p, self.seed = float(p), int(seed)
         self._in = (frames.contiguous(), cls_hidden.contiguous(), lang_feature.contiguous())
         frames, cls, lang = self._in
-        av, al, dec, fc = m.attention_layer_vision, m.attention_layer_lang, m.decoder_2_action_full, m.fc
+        av = m.attention_layer_vision
         # input_lstm_0 of every step (vln_model.py:219)
         call("avdn_frame_attn_fwd", ptr(frames), ptr(cls), ptr(av.linear_in.weight), ptr(av.linear_out.weight), None,
              None, B, T, ptr(self.attn512), ptr(self.wc), ptr(self.e49), None)
         self.e49_t.copy_(self.e49.view(B, T, NSP).transpose(0, 1))
         call("avdn_add_dropout_f32", ptr(self.e49_t), None, ptr(self.e49d), BT * NSP, self.p, self.seed, SITE_INPUT)
-        # pred_saliency's fc reads the undropped input_lstm_0 (vln_model.py:244)
-        m._linear(self.e49_t.view(BT, NSP), fc[0].weight, fc[0].bias, self.s0.view(BT, 128), act=1)
-        call("avdn_dropout_f32", ptr(self.s0), None, BT * 128, self.p, self.seed, SITE_FC)
-        m._linear(self.s0.view(BT, 128), fc[3].weight, fc[3].bias, self.h_sali.view(BT, 64), act=1)
         # direction_embedding of every step (vln_model.py:228-229)
         self.deg.copy_(deg.t())
         call("avdn_direction_embed", ptr(self.deg), ptr(m.direction_embedding.weight), ptr(m.direction_embedding.bias),
              ptr(self.dir_emb), BT, 32)
-        n = 6
         for t in range(T):
-            cat = self.cat2[t]
-            prev = self.cat2[t - 1] if t > 0 else None
-            # hh_1, cc_1 = vision_lstm(drop(input_lstm_0), (hh_0, cc_0))                vln_model.py:220-226
-            m._lstm(m.vision_lstm, self.e49d[t], prev[:, HID + 192:] if t else None, self.c_v[t - 1] if t else None,
-                    self.gates_v[t], cat[:, HID + 192:], self.c_v[t])
-            m._lstm(m.direct_lstm, self.dir_emb[t], prev[:, HID:HID + 192] if t else None,
-                    self.c_d[t - 1] if t else None, self.gates_d[t], cat[:, HID:HID + 192], self.c_d[t])
-            # action_module_input = SoftDotAttention(768)(cat(h_1, hh_1), lang_feature)  vln_model.py:238-239
-            m._linear(cat[:, HID:], al.linear_in.weight, None, self.target[t])
-            call("avdn_lang_attn_fwd", ptr(lang), ptr(self.target[t]), B, L, HID, ptr(self.attn[t]), ptr(cat),
-                 cat.stride(0))
-            m._linear(cat, al.linear_out.weight, None, self.act_in[t], act=2)
-            # output = decoder_2_action_full(action_module_input)                       vln_model.py:248
-            m._linear(self.act_in[t], dec[0].weight, dec[0].bias, self.m0[t], act=1)
-            call("avdn_dropout_f32", ptr(self.m0[t]), None, B * 256, self.p, self.seed, SITE_DEC + 2 * t)
-            m._linear(self.m0[t], dec[3].weight, dec[3].bias, self.m1[t], act=1)
-            call("avdn_dropout_f32", ptr(self.m1[t]), None, B * 32, self.p, self.seed, SITE_DEC + 2 * t + 1)
-            m._linear(self.m1[t], dec[6].weight, dec[6].bias, self.output[t])
-            n += 3
-        self.launches += n + (m.launches - l0)
+            self._step_body(t, lang)
+        self._saliency(T)
+        self.launches += 6 + 3 * T + (m.launches - l0)
         return self.output, self.h_sali
 
-    def loss(self, gt_xy, gt_alt, gt_prog, att, nss_w, nss_r, scale, loss_total):
+    def begin(self, cls_hidden, lang_feature, p=0.0, seed=0):
+        """Start a step-wise forward (``step`` per time step, then ``finish``): the same activations as ``forward``,
+        for a rollout whose frames and headings of step t+1 depend on the output of step t.  Arguments as for
+        ``forward``."""
+        self.p, self.seed = float(p), int(seed)
+        if getattr(self, "_frames", None) is None:
+            f = lambda *s: torch.zeros(s, dtype=torch.float32, device=self.deg.device)
+            self._frames = f(self.B * self.T, NCH, NSP)                 # frame-major input, read by backward
+            self._st = (f(self.B, NCH), f(self.B, NSP), f(self.B, NSP))  # attn512 / wc / e49 of one step
+        self._in = (self._frames, cls_hidden.contiguous(), lang_feature.contiguous())
+        self.n_run = 0
+
+    def step(self, t, frames_t, deg_t):
+        """Policy step ``t`` (0, 1, ... in order) of a ``begin``-started forward on the B frames ``frames_t``
+        [B,512,49] f32 and headings ``deg_t`` [B] (degrees).  Returns ``output[t]`` [B,4] (a view, valid until the
+        engine's next forward)."""
+        m, B, T = self.m, self.B, self.T
+        call, ptr = _lib.call, _lib.ptr
+        if t != self.n_run or t >= T:
+            raise ValueError(f"step {t}: expected step {self.n_run} of {T}")
+        l0 = m.launches
+        _, cls, lang = self._in
+        av = m.attention_layer_vision
+        imf = frames_t.contiguous()
+        attn512, wc, e49 = self._st
+        call("avdn_frame_attn_fwd", ptr(imf), ptr(cls), ptr(av.linear_in.weight), ptr(av.linear_out.weight), None,
+             None, B, 1, ptr(attn512), ptr(wc), ptr(e49), None)
+        # the frame-major rows b*T + t of step t
+        self.attn512.view(B, T, NCH)[:, t].copy_(attn512)
+        self.wc.view(B, T, NSP)[:, t].copy_(wc)
+        self.e49.view(B, T, NSP)[:, t].copy_(e49)
+        self._frames.view(B, T, NCH, NSP)[:, t].copy_(imf.view(B, NCH, NSP))
+        self.e49_t[t].copy_(e49)
+        # step t's slice of the [T,B,49] input dropout: the mask forward draws over the whole rollout
+        call("avdn_add_dropout_f32_at", ptr(self.e49_t[t]), None, ptr(self.e49d[t]), B * NSP, t * B * NSP, self.p,
+             self.seed, SITE_INPUT)
+        self.deg[t].copy_(deg_t.reshape(B))
+        call("avdn_direction_embed", ptr(self.deg[t]), ptr(m.direction_embedding.weight),
+             ptr(m.direction_embedding.bias), ptr(self.dir_emb[t]), B, 32)
+        self._step_body(t, lang)
+        self.n_run = t + 1
+        self.launches += 12 + (m.launches - l0)
+        return self.output[t]
+
+    def finish(self):
+        """End a step-wise forward: the saliency branch of the steps that ran.  Returns ``output`` [T,B,4] and
+        ``h_sali`` [T,B,64] (rows of the first ``n_run`` steps)."""
+        l0 = self.m.launches
+        self._saliency(self.n_run)
+        self.launches += 1 + (self.m.launches - l0)
+        return self.output, self.h_sali
+
+    def _saliency(self, n):
+        """pred_saliency's fc over the first n steps; it reads the undropped input_lstm_0 (vln_model.py:244)."""
+        m, call, ptr = self.m, _lib.call, _lib.ptr
+        fc, nB = m.fc, n * self.B
+        m._linear(self.e49_t[:n].view(nB, NSP), fc[0].weight, fc[0].bias, self.s0[:n].view(nB, 128), act=1)
+        call("avdn_dropout_f32", ptr(self.s0), None, nB * 128, self.p, self.seed, SITE_FC)
+        m._linear(self.s0[:n].view(nB, 128), fc[3].weight, fc[3].bias, self.h_sali[:n].view(nB, 64), act=1)
+
+    def _step_body(self, t, lang):
+        """The recurrent part of step t on ``e49d[t]`` and ``dir_emb[t]``: the two LSTM cells, the language attention
+        and the action head (3 launches of its own besides the linear layers)."""
+        m, B, L = self.m, self.B, self.L
+        call, ptr = _lib.call, _lib.ptr
+        al, dec = m.attention_layer_lang, m.decoder_2_action_full
+        cat = self.cat2[t]
+        prev = self.cat2[t - 1] if t > 0 else None
+        # hh_1, cc_1 = vision_lstm(drop(input_lstm_0), (hh_0, cc_0))                vln_model.py:220-226
+        m._lstm(m.vision_lstm, self.e49d[t], prev[:, HID + 192:] if t else None, self.c_v[t - 1] if t else None,
+                self.gates_v[t], cat[:, HID + 192:], self.c_v[t])
+        m._lstm(m.direct_lstm, self.dir_emb[t], prev[:, HID:HID + 192] if t else None,
+                self.c_d[t - 1] if t else None, self.gates_d[t], cat[:, HID:HID + 192], self.c_d[t])
+        # action_module_input = SoftDotAttention(768)(cat(h_1, hh_1), lang_feature)  vln_model.py:238-239
+        m._linear(cat[:, HID:], al.linear_in.weight, None, self.target[t])
+        call("avdn_lang_attn_fwd", ptr(lang), ptr(self.target[t]), B, L, HID, ptr(self.attn[t]), ptr(cat),
+             cat.stride(0))
+        m._linear(cat, al.linear_out.weight, None, self.act_in[t], act=2)
+        # output = decoder_2_action_full(action_module_input)                       vln_model.py:248
+        m._linear(self.act_in[t], dec[0].weight, dec[0].bias, self.m0[t], act=1)
+        call("avdn_dropout_f32", ptr(self.m0[t]), None, B * 256, self.p, self.seed, SITE_DEC + 2 * t)
+        m._linear(self.m0[t], dec[3].weight, dec[3].bias, self.m1[t], act=1)
+        call("avdn_dropout_f32", ptr(self.m1[t]), None, B * 32, self.p, self.seed, SITE_DEC + 2 * t + 1)
+        m._linear(self.m1[t], dec[6].weight, dec[6].bias, self.output[t])
+
+    def loss(self, gt_xy, gt_alt, gt_prog, att, nss_w, nss_r, scale, loss_total, n_steps=None):
         """``avdn_loss`` of every step in one launch (T*B independent rows; jitter 0, src/xview_lstm/agent.py:636):
         ``loss_total`` += scale * sum of the step losses; ``d_output`` / ``d_h_sali`` receive their gradients.
-        ``gt_xy`` [T,B,2], ``gt_alt`` / ``gt_prog`` [T,B] f32, ``att`` u8 [T,B,224,224] or None."""
+        ``gt_xy`` [T,B,2], ``gt_alt`` / ``gt_prog`` [T,B] f32, ``att`` u8 [T,B,224,224] or None.  ``n_steps`` (default
+        T): only the first n_steps steps count (a rollout that ended early); the targets then hold n_steps rows."""
         ptr = _lib.ptr
+        n = self.T if n_steps is None else int(n_steps)
         _lib.call("avdn_loss", ptr(self.output), ptr(self.h_sali), ptr(gt_xy), ptr(gt_alt), ptr(gt_prog), ptr(att),
-                  None, self.B * self.T, float(nss_w), int(nss_r), float(scale), ptr(loss_total), ptr(self.loss_i),
+                  None, self.B * n, float(nss_w), int(nss_r), float(scale), ptr(loss_total), ptr(self.loss_i),
                   ptr(self.d_output), ptr(self.d_h_sali))
         self.launches += 1
 
-    def backward(self, d_lang=None, d_cls=None):
+    def backward(self, d_lang=None, d_cls=None, n_steps=None):
         """Backward through time from ``d_output`` / ``d_h_sali`` (written by ``loss``).  Overwrites ``d_frames``
         [B*T,512,49] (returned); accumulates every parameter gradient into ``G`` and, when given, the gradients of
-        ``lang_feature`` into ``d_lang`` [B,L,768] and of ``cls_hidden`` into ``d_cls`` [B,49] (+=)."""
-        m, B, L, T = self.m, self.B, self.L, self.T
+        ``lang_feature`` into ``d_lang`` [B,L,768] and of ``cls_hidden`` into ``d_cls`` [B,49] (+=).  ``n_steps``
+        (default T, as given to ``loss``): the steps the rollout ran; the rows of later steps get zero ``d_frames``
+        and contribute nothing."""
+        m, B, L = self.m, self.B, self.L
+        T = self.T if n_steps is None else int(n_steps)
         call, ptr = _lib.call, _lib.ptr
         BT = B * T
         l0 = m.launches
@@ -193,7 +261,7 @@ class _TrainEngine:
         frames, cls, lang = self._in
         av, al, dec, fc = m.attention_layer_vision, m.attention_layer_lang, m.decoder_2_action_full, m.fc
         vl, dl = m.vision_lstm, m.direct_lstm
-        r = lambda a: a.view(BT, a.shape[-1])
+        r = lambda a: a[:T].view(BT, a.shape[-1])          # step-major: the first T steps are the first B*T rows
         n = 0
         # ---- the action head of every step (nothing recurrent), down to d cat2 = [d weighted | d h | d hh] ----
         self._lin_bwd(r(self.m1), dec[6].weight, r(self.d_output), r(self.d_output), 0, r(self.d_m1),
@@ -241,7 +309,7 @@ class _TrainEngine:
             if T > 1:                      # step 0 ran from the zero state: W_hh saw h = 0 there
                 H = cell.hidden_size
                 h_prev = self.cat2[:T - 1].view((T - 1) * B, 2 * HID)[:, lo:lo + H]
-                dg1 = dg[1:].view((T - 1) * B, 4 * H)
+                dg1 = dg[1:T].view((T - 1) * B, 4 * H)
                 _lib.call("avdn_linear_f32_bwd", ptr(h_prev), h_prev.stride(0), ptr(cell.weight_hh), ptr(dg1),
                           ptr(dg1), (T - 1) * B, 4 * H, H, 0, None, 0, 0, ptr(G[name + ".weight_hh"]), None)
                 n += 1
@@ -254,9 +322,11 @@ class _TrainEngine:
         self._lin_bwd(r(self.s0), fc[3].weight, r(self.h_sali), r(self.d_h_sali), 1, r(self.d_s0), "fc.3")
         call("avdn_dropout_f32", ptr(self.d_s0), None, BT * 128, p, seed, SITE_FC)
         self._lin_bwd(r(self.e49_t), fc[0].weight, r(self.s0), r(self.d_s0), 1, r(self.d_e49), "fc.0", dx_accumulate=1)
-        self.d_e49_bt.view(B, T, NSP).copy_(self.d_e49.transpose(0, 1))
+        if T < self.T:                     # steps that did not run: no gradient reaches their frames
+            self.d_e49[T:].zero_()
+        self.d_e49_bt.view(B, self.T, NSP).copy_(self.d_e49.transpose(0, 1))
         call("avdn_frame_attn_bwd_cls", ptr(frames), ptr(cls), ptr(av.linear_in.weight), ptr(av.linear_out.weight),
-             None, B, T, ptr(self.attn512), ptr(self.wc), ptr(self.e49), ptr(self.d_e49_bt), ptr(self.d_frames),
+             None, B, self.T, ptr(self.attn512), ptr(self.wc), ptr(self.e49), ptr(self.d_e49_bt), ptr(self.d_frames),
              ptr(self.G["attention_layer_vision.linear_in.weight"]), ptr(self.G["attention_layer_vision.linear_out.weight"]),
              None, None, ptr(d_cls))
         n += 10

@@ -15,6 +15,13 @@ with every per-step stage on the device and no host round trip inside the loop:
 The language side (BERT -> ``lang_feature`` [B,L,768], ``cls_hidden`` = linear_cls [B,49],
 agent.py:527-543) is an input of the path (SURVEY.md §8f N1).
 
+Student-feedback training runs in one of two ways.  By default (``rollout``, ``student_batch``) a no-grad
+``rollout_greedy`` in eval mode fixes the poses and ``train_rollout_step`` then trains on them.  With
+``args.on_policy_student`` ``rollout`` calls ``student_rollout_step`` instead, the reference's single pass
+(agent.py:518-774): every step renders the current views, runs its own train-mode trunk pass (per-step batch
+statistics) and ``_TrainEngine.step`` with dropout on, and the simulator moves by that train-mode output; the targets,
+loss and backward through time follow once the loop has ended.
+
 Training: one ``FusedAdamW`` over ``vln_model.used_parameters()`` (gradients clipped to a global norm of 40) and one
 over the trunk (unclipped), built here before any rollout captures a CUDA graph of the trunk (the arenas re-home
 the parameter storage).  AdamW is elementwise, so two optimisers update as one would; the clipping mirrors the ET
@@ -36,8 +43,8 @@ import numpy as np
 import torch
 
 from .. import _lib
-from ..agent_common import (RolloutTrainer, render_rollout_views, rollout_trunk_backward, rollout_trunk_forward,
-                            steps_until_all_ended, student_rollout_targets)
+from ..agent_common import (RolloutTrainer, render_rollout_views, rollout_step_bufs, rollout_trunk_backward,
+                            rollout_trunk_forward, steps_until_all_ended, student_rollout_targets)
 from ..env import ViewRenderer
 from ..models import dark_net as DN
 from ..models.dark_net import Darknet
@@ -88,8 +95,11 @@ class NavCMTAgent(RolloutTrainer):
         self.launches = 0
         self._bufs = {}
 
-    def _get_bufs(self, B, T):
-        b = self._bufs.get((B, T))
+    def _get_bufs(self, B, T, kind=None):
+        """Pose and simulator buffers of a rollout of B episodes and T steps; ``kind`` keeps the greedy rollout's
+        (None) and the on-policy training rollout's ('on_policy') apart."""
+        key = (B, T) if kind is None else (kind, B, T)
+        b = self._bufs.get(key)
         if b is None:
             dev = self.device
             b = dict(x=torch.empty((B, 224, 224, 4), dtype=torch.bfloat16, device=dev),
@@ -106,7 +116,7 @@ class NavCMTAgent(RolloutTrainer):
                      angle=torch.empty((T, B), dtype=torch.int32, device=dev),
                      altitude=torch.empty((T, B), dtype=torch.int32, device=dev),
                      dist=torch.empty((T, B), dtype=torch.float64, device=dev))
-            self._bufs[(B, T)] = b
+            self._bufs[key] = b
         return b
 
     @torch.no_grad()
@@ -259,6 +269,134 @@ class NavCMTAgent(RolloutTrainer):
                    directions=res["directions"][:T].float().t().contiguous())
         return out
 
+    def student_rollout_step(self, batch, gt_path_corners, max_action_len=None, nss_w=None, train_ml=None, zero=True,
+                             step=True, sync_loss=False, collect=None, bn_per_step=None):
+        """One on-policy student-feedback training rollout, as the reference runs it (src/xview_lstm/agent.py:518-774):
+        every step runs the policy in train mode -- the trunk on the step's own batch statistics, the four Dropout(0.2)
+        sites active -- and the simulator moves by that same train-mode prediction (stop threshold 0.25).  The loop
+        stops after the step at which every sample has ended (one host read of the B stop flags per step).  Then one
+        ``teacher_action`` launch gives the target of every visited pose, and the loss, the backward through time,
+        the trunk backward of the executed per-step passes, the BERT backward and (``step``) the optimiser step run
+        as in ``train_rollout_step``.
+
+        ``batch`` as for ``rollout_greedy``; with an attached language model it may carry ``input_ids`` /
+        ``attention_mask`` (and ``cls_*``) instead of ``lang_feature`` / ``cls_hidden``: BERT then runs once in train
+        mode, and its outputs both steer the rollout and receive the gradients.  ``gt_path_corners``: per sample the
+        ``[n_i,4,2]`` ground-truth view corners.  The per-step trunk passes are required (``bn_per_step`` false
+        raises ``ValueError``): the views of step t+1 depend on step t's features.  What the rollout visited is kept
+        in ``self._last_rollout``."""
+        if bn_per_step is None:
+            bn_per_step = bool(getattr(self.args, "bn_per_step", True))
+        if not bn_per_step:
+            raise ValueError("an on-policy student rollout needs one trunk pass per step (bn_per_step): the views of "
+                             "step t+1 depend on the features of step t")
+        with self._weights(nss_w, train_ml):
+            return self._student_rollout_step(batch, gt_path_corners, max_action_len, zero, step, sync_loss, collect)
+
+    def _student_rollout_step(self, batch, gt_path_corners, max_action_len, zero, step, sync_loss, collect):
+        T = int(max_action_len if max_action_len is not None else getattr(self.args, "max_action_len", 20))
+        ptr, call = _lib.ptr, _lib.call
+        dev = self.device
+        n = 0
+        if zero:
+            for opt in self.optimizers:
+                opt.zero_grad()
+            n += 2
+        leng = leng2 = None
+        if "input_ids" in batch:
+            seq, lin, leng, leng2 = self._lang_train_forward(batch)
+            batch = dict(batch, lang_feature=seq, cls_hidden=lin)
+        lang, cls = batch["lang_feature"].contiguous().float(), batch["cls_hidden"].contiguous().float()
+        B, L = lang.shape[0], lang.shape[1]
+        vln, vm, r = self.vln_model, self.vision_model, self.renderer
+        vln.train(not getattr(self.args, "no_dropout", False))
+        vm.train()
+        eng = vln.train_engine(B, L, T, dev)
+        e0 = eng.launches
+        eng.begin(cls, lang, *vln.dropout_config())
+        bf = self._get_bufs(B, T, "on_policy")
+        sb = rollout_step_bufs(self, B, T)
+        geo = batch["geo"].contiguous()
+        bounds = geo[:, :4].contiguous()
+        ti = batch.get("tile_idx")
+        bf["corners"].copy_(batch["corners_gps"])
+        bf["cur_dir"].copy_(batch["directions"])
+        bf["ended"].zero_()
+        ended_h = torch.empty(B, dtype=torch.uint8, pin_memory=True)
+        tengs, l0 = [], 0
+        steps = T
+        for t in range(T):
+            bf["corners_hist"][t].copy_(bf["corners"])
+            bf["dir_hist"][t].copy_(bf["cur_dir"])
+            # ---- observation of the current pose (agent.py:742) ----
+            call("avdn_gps_to_pixels", ptr(bf["corners"]), ptr(geo), B, ptr(bf["px"]))
+            call("avdn_homography_from_corners", ptr(bf["px"]), B, ptr(bf["minv"]))
+            r.render(None, ti, views=False, norm_nhwc=True, minv=bf["minv"], out={"norm_nhwc": sb["x"][t]})
+            # ---- train-mode policy step (agent.py:592-602): its own trunk pass, kept for the backward ----
+            teng = vm.engine(B, 224, 224, dev, slot=1 + t)
+            l0 += teng.launches
+            tengs.append(teng)
+            DN._trunk_forward(vm, teng, sb["x"][t], True, out=sb["f"])
+            output = eng.step(t, sb["f"].view(B, NCH, NSP), bf["cur_dir"])
+            # ---- the simulator moves by the train-mode prediction (agent.py:607-626,700-730) ----
+            call("avdn_waypoint_step", ptr(output), ptr(bf["corners"]), ptr(bounds), ptr(bf["cur_dir"]),
+                 ptr(bf["ended"]), B, float(STOP_THRESHOLD_STUDENT), int(t == T - 1), ptr(bf["angle"][t]),
+                 ptr(bf["dist"][t]), ptr(bf["altitude"][t]))
+            bf["ended_hist"][t].copy_(bf["ended"])
+            n += 9
+            if t < T - 1:                                # agent.py:773-774: stop once every sample has ended
+                ended_h.copy_(bf["ended"])
+                if bool(ended_h.numpy().all()):
+                    steps = t + 1
+                    break
+        bf["corners_hist"][steps].copy_(bf["corners"])
+        bf["dir_hist"][steps].copy_(bf["cur_dir"])
+        eng.finish()
+        # ---- the teacher's target at every visited pose, one launch (agent.py:655-661) ----
+        res = dict(corners=bf["corners_hist"], ended=bf["ended_hist"], steps=steps)
+        tgt, _, _ = student_rollout_targets(self, batch, res, gt_path_corners)
+        sm = lambda a: a.transpose(0, 1).contiguous()                  # [B,steps,...] -> step-major
+        att = None
+        if self.nss_w != 0:
+            key = ("on_policy_att", B, T)
+            if key not in self._bufs:
+                self._bufs[key] = torch.empty((T * B, 224, 224), dtype=torch.uint8, device=dev)
+            att = self._bufs[key][:steps * B]
+            minv = r.homography(sm(tgt["corners_px"]).view(steps * B, 4, 2))
+            r.render(None, None if ti is None else ti.repeat(steps), views=False, att=True, minv=minv,
+                     out={"att": att})
+            att = att.view(steps, B, 224, 224)
+            n += 2
+        self.loss_total.zero_()
+        eng.loss(sm(tgt["gt_xy"]), sm(tgt["gt_alt"]), sm(tgt["gt_prog"]), att, self.nss_w,
+                 int(getattr(self.args, "nss_r", 0)), float(self.train_ml) / B, self.loss_total, n_steps=steps)
+        n += 6
+        if collect is not None:
+            collect.extend(eng.output[t].clone() for t in range(steps))
+        if leng is None:
+            eng.backward(n_steps=steps)
+        else:
+            d_lang = torch.zeros((B, L, 768), dtype=torch.float32, device=dev)
+            d_cls = torch.zeros((B, 49), dtype=torch.float32, device=dev)
+            eng.backward(d_lang, d_cls, n_steps=steps)
+            self._lang_train_backward(leng, leng2, d_lang, d_cls)
+        trunk_launches = rollout_trunk_backward(self, tengs[0], tengs, l0, eng.d_frames, B, T, steps=steps)
+        self._ctx = (tengs[0], tengs, eng, sb)
+        # what the rollout visited (inspection / tests): poses before every step and after the last, stop flags,
+        # train-mode outputs, targets, and the teacher-forced batch of the same poses
+        tr = {k: tgt[k] for k in ("corners_px", "tile_idx", "gt_xy", "gt_alt", "gt_prog")}
+        self._last_rollout = dict(
+            corners=bf["corners_hist"][:steps + 1].clone(), directions=bf["dir_hist"][:steps + 1].clone(),
+            ended=bf["ended_hist"][:steps].clone(), output=eng.output[:steps].clone(), steps=steps,
+            tgt_xy=sm(tgt["gt_xy"]), tgt_alt=sm(tgt["gt_alt"]), tgt_prog=sm(tgt["gt_prog"]),
+            batch=dict(batch, directions=bf["dir_hist"][:steps].float().t().contiguous(), **tr))
+        if step:
+            for opt in self.optimizers:
+                n += opt.step()
+        self.launches += n + trunk_launches + (eng.launches - e0)
+        self._log_loss()
+        return float(self.loss_total.item()) if sync_loss else self.loss_total
+
     @staticmethod
     def trajectories(res):
         """Host view of a rollout result: per sample the list of (corners [4,2], direction) the
@@ -285,6 +423,9 @@ class NavCMTAgent(RolloutTrainer):
         * Poses: teacher feedback from the ground-truth actions (``_teacher_rollout_poses``), student feedback from a
           no-grad greedy rollout on BERT's eval-mode features, with the ``teacher_action`` target of every pose.  The
           loop stops after the step at which every sample has ended (agent.py:773-774).
+        * ``args.on_policy_student`` (default false): a student-feedback training rollout is instead one
+          ``student_rollout_step``, the reference's single pass -- the poses follow the train-mode predictions that
+          are trained (trunk on per-step batch statistics, dropout on), as in agent.py:518-774.
         * Training (``not_in_train`` false): ``train_rollout_step`` over the poses with BERT in train mode -- the loss
           ``ml_loss * train_ml / B`` is added to ``self.loss`` and the gradients to the arenas (the reference's
           ``self.loss.backward()`` in ``train``; ``train`` then only clips and steps).  The LSTM has no ``lenths``: a
@@ -299,6 +440,9 @@ class NavCMTAgent(RolloutTrainer):
         has_gt = "test" not in self.env_name
         prev_r, self.renderer = self.renderer, env.renderer
         try:
+            if self.feedback == "student" and not not_in_train and getattr(self.args, "on_policy_student", False):
+                self._on_policy_rollout(lb, gps0, dirs0, geo, tidx, gt_paths, traj, T, train_ml, nss_w, has_gt)
+                return traj
             if self.feedback == "teacher":
                 H, steps = self._teacher_rollout_poses(torch.from_numpy(gps0), dirs0, geo, gt_paths, T)
                 corners, ended, heads = H["corners"][:steps], H["ended"][:steps], H["dirs"][:steps]
@@ -352,6 +496,21 @@ class NavCMTAgent(RolloutTrainer):
         finally:
             self.renderer = prev_r
         return traj
+
+    def _on_policy_rollout(self, lb, gps0, dirs0, geo, tidx, gt_paths, traj, T, train_ml, nss_w, has_gt):
+        """The student-feedback training rollout of ``rollout`` with ``args.on_policy_student``: one
+        ``student_rollout_step`` (BERT, trunk and policy in train mode; the poses follow the train-mode predictions).
+        The trajectory dicts log the outputs and poses the rollout used."""
+        outs = []
+        batch = dict(lb, corners_gps=torch.from_numpy(gps0).to(self.device), directions=dirs0, geo=geo, tile_idx=tidx)
+        loss = self.student_rollout_step(batch, gt_paths, max_action_len=T, nss_w=float(nss_w),
+                                         train_ml=train_ml if train_ml is not None else 0.0, zero=False, step=False,
+                                         collect=outs)
+        lr = self._last_rollout
+        tgt = (lr["tgt_xy"].cpu().numpy(), lr["tgt_alt"].cpu().numpy(), lr["tgt_prog"].cpu().numpy()) if has_gt else None
+        self._log_traj(traj, torch.stack(outs).cpu().numpy(), tgt, lr["ended"].cpu().numpy().astype(bool),
+                       lr["corners"].cpu().numpy(), lr["directions"].cpu().numpy(), lr["steps"])
+        self._add_rollout_loss(loss, train_ml)
 
     @torch.no_grad()
     def _eval_rollout(self, batch, traj, outs):

@@ -476,6 +476,10 @@ int avdn_dropout_f32(float* x, void* x16, long long n, float p, unsigned long lo
                      avdn_stream_t stream);
 int avdn_add_dropout_f32(const float* a, const float* b, float* out, long long n, float p, unsigned long long seed,
                          unsigned int site, avdn_stream_t stream);
+/* avdn_add_dropout_f32 over a slice that starts at element idx0 of a larger tensor of the same site: element i
+ * draws the mask of element idx0 + i (one time step of ViT_LSTM's input dropout, drawn as over the whole rollout). */
+int avdn_add_dropout_f32_at(const float* a, const float* b, float* out, long long n, long long idx0, float p,
+                            unsigned long long seed, unsigned int site, avdn_stream_t stream);
 int avdn_heads_fwd_drop(const float* x, int B, int S, int row_vis, int row_dir, const float* w0, const float* b0,
                         const float* w1, const float* b1, const float* w2, const float* b2, const float* wf,
                         const float* bf, float* h0, float* h1, float* output, float* h_sali, float p,
