@@ -98,18 +98,11 @@ class RolloutTrainer:
         B = c.shape[0]
         packed = isinstance(gt_path_corners, tuple) and len(gt_path_corners) == 2 and torch.is_tensor(gt_path_corners[0])
         if isinstance(gt_path_corners, (list, tuple)) and not packed:
-            lens = [len(g) for g in gt_path_corners]
-            pmax = max(lens)
-            gt = np.zeros((B, pmax, 4, 2), dtype=np.float64)
-            for i, g in enumerate(gt_path_corners):
-                gt[i, :lens[i]] = np.asarray(g, dtype=np.float64)
-            gt_t = torch.from_numpy(gt).to(dev)
-            len_t = torch.tensor(lens, dtype=torch.int32, device=dev)
-        else:
-            gt_t, len_t = gt_path_corners
-            gt_t = gt_t.to(dev, torch.float64).contiguous()
-            len_t = len_t.to(dev, torch.int32).contiguous()
-            pmax = gt_t.shape[1]
+            gt_path_corners = pack_gt_paths(gt_path_corners, dev)
+        gt_t, len_t = gt_path_corners
+        gt_t = gt_t.to(dev, torch.float64).contiguous()
+        len_t = len_t.to(dev, torch.int32).contiguous()
+        pmax = gt_t.shape[1]
         e = torch.as_tensor(np.asarray(ended, dtype=np.uint8) if not torch.is_tensor(ended) else ended).to(dev, torch.uint8).contiguous()
         ratio = torch.empty((B, 2), dtype=torch.float32, device=dev)
         alt = torch.empty(B, dtype=torch.float32, device=dev)
@@ -228,12 +221,7 @@ class RolloutTrainer:
                  ended=torch.empty((T, B), dtype=torch.uint8, device=dev), xy=torch.empty((T, B, 2), device=dev),
                  alt=torch.empty((T, B), device=dev), prog=torch.empty((T, B), device=dev))
         ang = torch.empty(B, dtype=i32, device=dev); dist = torch.empty(B, dtype=f64, device=dev); alt_i = torch.empty(B, dtype=i32, device=dev)
-        gts = [gt_paths[i] for i in range(B)]
-        lens = [len(g) for g in gts]
-        gt = np.zeros((B, max(lens), 4, 2), dtype=np.float64)
-        for i, g in enumerate(gts):
-            gt[i, :lens[i]] = np.asarray(g, dtype=np.float64)
-        gt_pack = (torch.from_numpy(gt).to(dev), torch.tensor(lens, dtype=i32, device=dev))
+        gt_pack = pack_gt_paths([gt_paths[i] for i in range(B)], dev)
         for t in range(T):
             H["corners"][t].copy_(corners); H["dirs"][t].copy_(cur)
             xy, alt, prog = self.teacher_action(corners, gt_pack, ended, feedback="teacher")
@@ -438,6 +426,16 @@ class RolloutTrainer:
                                      "format) cannot be resumed -- load with resume_optimizer=False")
                 opt.m.copy_(o["m"]); opt.v.copy_(o["v"]); opt.step_count = int(o["step"])
         return states.get("vln_model", {}).get("epoch", 0) - 1
+
+
+def pack_gt_paths(gt_path_corners, device):
+    """Per sample ``[n_i,4,2]`` ground-truth view corners -> the ``(gt [B,max n_i,4,2] f64, lengths [B] i32)`` device
+    pair ``teacher_action`` takes (zero-padded), so a loop of ``teacher_action`` launches packs them once."""
+    lens = [len(g) for g in gt_path_corners]
+    gt = np.zeros((len(lens), max(lens), 4, 2), dtype=np.float64)
+    for i, g in enumerate(gt_path_corners):
+        gt[i, :lens[i]] = np.asarray(g, dtype=np.float64)
+    return torch.from_numpy(gt).to(device), torch.tensor(lens, dtype=torch.int32, device=device)
 
 
 def steps_until_all_ended(ended):

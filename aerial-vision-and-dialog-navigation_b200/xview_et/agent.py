@@ -26,6 +26,11 @@ What is here
   tokenizer -> ``CustomBERTModel`` -> poses of the rollout (teacher: ground-truth actions, ``avdn_teacher_action`` +
   ``avdn_waypoint_step`` on the device; student: a no-grad greedy rollout) -> ``train_rollout_step`` (views, trunk,
   T encoder passes with loss and backward) -> trajectory dicts, ``self.loss``, ``self.logs['IL_loss']``.
+
+* ``student_rollout_step`` (``rollout`` with ``args.on_policy_student``): the reference's on-policy student-feedback
+  training rollout in one pass -- every step renders the current views, runs its own train-mode trunk pass and the
+  ET in train mode over the history, takes the step's loss and backward, and moves the simulator by that same
+  train-mode prediction.
 """
 from __future__ import annotations
 
@@ -41,8 +46,8 @@ from ..models import dark_net as DN
 from ..models.dark_net import Darknet
 from ..optim import FusedAdamW
 from .. import parallel
-from ..agent_common import (RolloutTrainer, render_rollout_views, rollout_trunk_backward,
-                            rollout_trunk_forward, student_rollout_targets)
+from ..agent_common import (RolloutTrainer, pack_gt_paths, render_rollout_views, rollout_step_bufs,
+                            rollout_trunk_backward, rollout_trunk_forward, student_rollout_targets)
 
 PI_REF = 3.14159
 
@@ -469,6 +474,228 @@ class NavCMTAgent(RolloutTrainer):
                    lenths=np.maximum(lens, 1).tolist())
         return out
 
+    _LANG_KEYS = ("lang", "lang_cls", "input_ids", "attention_mask", "cls_input_ids", "cls_attention_mask")
+
+    def student_rollout_step(self, batch, gt_path_corners, max_action_len=None, nss_w=None, train_ml=None, zero=True,
+                             step=True, sync_loss=False, collect=None, bn_per_step=None):
+        """One on-policy student-feedback training rollout, as the reference runs it (src/xview_et/agent.py:580-760):
+        every step runs the trunk and the ET in train mode, takes the step's loss, and the simulator moves by that
+        same train-mode prediction (stop threshold 0.5), so the model is trained on the states its own train-mode
+        policy visits.  Step t: render the B current views into trunk slot ``1 + t`` and run a train-mode pass on
+        the step's own batch statistics (kept for the backward) -> the features and the heading join the history,
+        ``lenths`` grows for the samples that have not ended (agent.py:603-620) -> the ET over the history
+        ``[:t+1]`` with fresh dropout masks -> the ``teacher_action`` target at the pose -> ``avdn_loss`` ->
+        ``avdn_waypoint_step`` -> the ET backward of the step, its frame gradients added into the history's.  One
+        host read of the B stop flags per step gives the next step's ``lenths``; the loop stops after the step at
+        which every sample has ended (agent.py:773-774).  Then the BERT backward, the trunk backward of the executed
+        passes and (``step``) the data-parallel reduction and the optimiser step, as in ``train_rollout_step``.
+
+        ``batch`` as for ``rollout_greedy``; with an attached language model it may carry ``input_ids`` /
+        ``attention_mask`` (and ``cls_*``) instead of ``lang`` / ``lang_cls``: BERT then runs once in train mode,
+        its outputs steer the rollout and one backward receives the gradients of every step.  ``gt_path_corners``:
+        per sample the ``[n_i,4,2]`` ground-truth view corners.  The per-step trunk passes are required
+        (``bn_per_step`` false raises ``ValueError``): the views of step t+1 depend on the features of step t.  What
+        the rollout visited, and the ``train_rollout_step`` batch of those poses, is kept in ``self._last_rollout``."""
+        if bn_per_step is None:
+            bn_per_step = bool(getattr(self.args, "bn_per_step", True))
+        if not bn_per_step:
+            raise ValueError("an on-policy student rollout needs one trunk pass per step (bn_per_step): the views of "
+                             "step t+1 depend on the features of step t")
+        with self._weights(nss_w, train_ml):
+            return self._student_rollout_step(batch, gt_path_corners, max_action_len, zero, step, sync_loss, collect)
+
+    def _on_policy_bufs(self, B, T):
+        """Pose, history and gradient buffers of an on-policy training rollout of B episodes and T steps."""
+        key = ("on_policy", B, T)
+        b = self._bufs.get(key)
+        if b is None:
+            dev = self.device
+            f64, i32, f32 = torch.float64, torch.int32, torch.float32
+            b = dict(corners=torch.empty((B, 4, 2), dtype=f64, device=dev),
+                     cur_dir=torch.empty(B, dtype=f64, device=dev),
+                     ended=torch.empty(B, dtype=torch.uint8, device=dev),
+                     minv=torch.empty((B, 3, 3), dtype=f64, device=dev),
+                     att=torch.empty((B, 224, 224), dtype=torch.uint8, device=dev),
+                     corners_hist=torch.empty((T + 1, B, 4, 2), dtype=f64, device=dev),
+                     dir_hist=torch.empty((T + 1, B), dtype=f64, device=dev),
+                     px_hist=torch.empty((T, B, 4, 2), dtype=i32, device=dev),
+                     ended_before=torch.zeros((T, B), dtype=torch.uint8, device=dev),
+                     ended_hist=torch.empty((T, B), dtype=torch.uint8, device=dev),
+                     output_hist=torch.empty((T, B, 4), dtype=f32, device=dev),
+                     tgt_xy=torch.empty((T, B, 2), dtype=f32, device=dev),
+                     tgt_alt=torch.empty((T, B), dtype=f32, device=dev),
+                     tgt_prog=torch.empty((T, B), dtype=f32, device=dev),
+                     frames=torch.empty((B, T, 512, 49), dtype=f32, device=dev),
+                     dirs=torch.empty((B, T, 2), dtype=f32, device=dev),
+                     d_frames=torch.empty((B, T, 512, 49), dtype=f32, device=dev),
+                     d_frames_t=torch.empty((B * T, 512, 49), dtype=f32, device=dev),
+                     d_output=torch.empty((B, 4), dtype=f32, device=dev),
+                     d_h_sali=torch.empty((B, 64), dtype=f32, device=dev),
+                     loss_i=torch.empty(B, dtype=f64, device=dev),
+                     angle=torch.empty((T, B), dtype=i32, device=dev),
+                     altitude=torch.empty((T, B), dtype=i32, device=dev),
+                     dist=torch.empty((T, B), dtype=f64, device=dev),
+                     ended_h=torch.empty(B, dtype=torch.uint8, pin_memory=True))
+            self._bufs[key] = b
+        return b
+
+    def _student_rollout_step(self, batch, gt_path_corners, max_action_len, zero, step, sync_loss, collect):
+        ptr, call = _lib.ptr, _lib.call
+        T = int(max_action_len if max_action_len is not None else getattr(self.args, "max_action_len", 20))
+        dev = self.device
+        n = 0
+        if zero:
+            for opt in self.optimizers:
+                opt.zero_grad()
+            n += 2
+        lang_in = {k: batch[k] for k in self._LANG_KEYS if k in batch}
+        leng = leng2 = None
+        if "input_ids" in batch:
+            # the language encoder runs once per rollout (agent.py:519-538): its train-mode outputs steer the rollout
+            seq, lin, leng, leng2 = self._lang_train_forward(batch)
+            batch = dict(batch, lang=seq, lang_cls=lin)
+        lang, lang_cls = batch["lang"].contiguous().float(), batch["lang_cls"].contiguous().float()
+        B, L = lang.shape[0], lang.shape[1]
+        vm, et, r = self.vision_model, self.vln_model, self.renderer
+        vm.train()
+        et.train(not getattr(self.args, "no_dropout", False))
+        bf = self._on_policy_bufs(B, T)
+        sb = rollout_step_bufs(self, B, T)
+        geo = batch["geo"].contiguous()
+        bounds = geo[:, :4].contiguous()
+        ti = batch.get("tile_idx")
+        gt_pack = pack_gt_paths(gt_path_corners, dev)              # once: the loop does no host packing
+        bf["corners"].copy_(batch["corners_gps"])
+        bf["cur_dir"].copy_(batch["directions"])
+        bf["ended"].zero_()
+        bf["d_frames"].zero_()
+        no_dir = bool(getattr(self.args, "no_direction", False))
+        if no_dir:
+            bf["dirs"].zero_()
+        self.loss_total.zero_()
+        scale = float(self.train_ml) / B                               # agent.py:883-885
+        nss_w, nss_r = float(self.nss_w), int(getattr(self.args, "nss_r", 0))
+        thr = float(self.STOP_THRESHOLD)
+        pe = et.encoder_vl.enc_pos.pe[0]
+        if leng is not None:
+            d_lang_sum = torch.zeros((B, L, 768), dtype=torch.float32, device=dev)
+            d_cls_sum = torch.zeros((B, 49), dtype=torch.float32, device=dev)      # every step adds into it
+        lens = [0] * B
+        lens_hist = []                                                 # [steps][B]: history length seen at step t
+        ended_host = np.zeros(B, dtype=bool)
+        tengs, l0, et_launches = [], 0, 0
+        steps = T
+        for t in range(T):
+            Tc = t + 1
+            # ---- 1. the pose and its observation (agent.py:742): the views into this step's trunk slot ----
+            bf["corners_hist"][t].copy_(bf["corners"])
+            bf["dir_hist"][t].copy_(bf["cur_dir"])
+            if t > 0:
+                bf["ended_before"][t].copy_(bf["ended"])
+            px = bf["px_hist"][t]
+            call("avdn_gps_to_pixels", ptr(bf["corners"]), ptr(geo), B, ptr(px))
+            call("avdn_homography_from_corners", ptr(px), B, ptr(bf["minv"]))
+            r.render(None, ti, views=False, norm_nhwc=True, minv=bf["minv"], out={"norm_nhwc": sb["x"][t]})
+            att = None
+            if nss_w != 0:
+                r.render(None, ti, views=False, att=True, minv=bf["minv"], out={"att": bf["att"]})
+                att = bf["att"]
+                n += 1
+            # ---- 2. train-mode trunk pass on the step's own batch statistics (agent.py:593), kept for the backward ----
+            teng = vm.engine(B, 224, 224, dev, slot=1 + t)
+            l0 += teng.launches
+            tengs.append(teng)
+            DN._trunk_forward(vm, teng, sb["x"][t], True, out=sb["f"])
+            bf["frames"][:, t].copy_(sb["f"].view(B, 512, 49))
+            # ---- 3. heading of the step (agent.py:605-606) and the history lengths (agent.py:603-620) ----
+            if not no_dir:
+                rad = bf["cur_dir"].float() / 180 * PI_REF
+                bf["dirs"][:, t, 0] = torch.sin(rad)
+                bf["dirs"][:, t, 1] = torch.cos(rad)
+            for i in range(B):
+                if not ended_host[i]:
+                    lens[i] += 1
+            lens_hist.append(list(lens))
+            # ---- 4. the ET over the history [:t+1], train mode, fresh dropout masks ----
+            eng = et.engine(B, L, Tc, dev)
+            e0 = eng.launches
+            eng.set_dropout(*et.dropout_config())
+            f_t = bf["frames"][:, :Tc].contiguous().view(B * Tc, 512, 49)
+            output, h_sali = eng.forward(f_t, lang, lang_cls, bf["dirs"][:, :Tc].contiguous(), lens, pe)
+            # ---- 5. the teacher's target at the pose (agent.py:655-661) and 6. the step's loss ----
+            xy, alt, prog = self.teacher_action(bf["corners"], gt_pack, bf["ended_before"][t], feedback="student")
+            call("avdn_loss", ptr(output), ptr(h_sali), ptr(xy), ptr(alt), ptr(prog), ptr(att), None, B, nss_w, nss_r,
+                 scale, ptr(self.loss_total), ptr(bf["loss_i"]), ptr(bf["d_output"]), ptr(bf["d_h_sali"]))
+            bf["tgt_xy"][t].copy_(xy)
+            bf["tgt_alt"][t].copy_(alt)
+            bf["tgt_prog"][t].copy_(prog)
+            # ---- 7. the simulator moves by the train-mode prediction (agent.py:637-653,736-760) ----
+            bf["output_hist"][t].copy_(output)
+            if collect is not None:
+                collect.append(output.detach().clone())
+            call("avdn_waypoint_step", ptr(output), ptr(bf["corners"]), ptr(bounds), ptr(bf["cur_dir"]),
+                 ptr(bf["ended"]), B, thr, int(t == T - 1), ptr(bf["angle"][t]), ptr(bf["dist"][t]),
+                 ptr(bf["altitude"][t]))
+            bf["ended_hist"][t].copy_(bf["ended"])
+            # ---- 8. the step's backward straight away: one encoder's activations are alive at a time ----
+            if leng is None:
+                df, _ = eng.backward(bf["d_output"], bf["d_h_sali"], d_frames=bf["d_frames_t"][:B * Tc])
+            else:
+                df, d_lang = eng.backward(bf["d_output"], bf["d_h_sali"], d_frames=bf["d_frames_t"][:B * Tc],
+                                          need_lang_grad=True, d_lang_cls=d_cls_sum)
+                d_lang_sum += d_lang.view(B, L, 768)
+                n += 1
+            bf["d_frames"][:, :Tc] += df.view(B, Tc, 512, 49)
+            et_launches += eng.launches - e0
+            n += 20                                 # the step's kernels outside the trunk and ET engines
+            # ---- 9. the step's only host read: the stop flags (next lenths; agent.py:773-774 early exit) ----
+            if t < T - 1:
+                bf["ended_h"].copy_(bf["ended"])
+                ended_host = bf["ended_h"].numpy().astype(bool)
+                if ended_host.all():
+                    steps = t + 1
+                    break
+        bf["corners_hist"][steps].copy_(bf["corners"])
+        bf["dir_hist"][steps].copy_(bf["cur_dir"])
+        if leng is not None:
+            self._lang_train_backward(leng, leng2, d_lang_sum, d_cls_sum)
+        self._ctx = (tengs[0], eng, bf, l0, eng.launches - et_launches)
+        dp = self.world > 1 and step               # gradients are reduced once, after the iteration's last rollout
+        if dp:
+            if self.lang_optimizer is not None:
+                self._allreduce_async(self.lang_optimizer.g, 0, self.lang_optimizer.n)
+            self._allreduce_async(self.et_optimizer.g, 0, self.et_optimizer.n)
+            buckets = {c: (lo, hi) for c, lo, hi in self._trunk_buckets(tengs[0])}
+            hook = lambda li: (self._allreduce_async(self.vision_model_optimizer.g, *buckets[li])
+                               if li in buckets else None)
+        else:
+            hook = None
+        trunk_launches = rollout_trunk_backward(self, tengs[0], tengs, l0, bf["d_frames"], B, T, after_layer=hook,
+                                                flush_layers=set(buckets) if dp else None, steps=steps)
+        if dp:
+            self._wait_comm()
+        if step:
+            gs = 1.0 / self.world
+            for opt in self.optimizers:
+                n += opt.step(grad_scale=gs)
+        self.launches += n + trunk_launches + et_launches
+        self._log_loss()
+        # what the rollout visited (inspection / tests): poses before every step and after the last, stop flags,
+        # train-mode outputs, targets, and the teacher-forced batch of the same poses
+        # [steps,B,...] -> [B,steps,...], always a copy: the buffers are rewritten by the next rollout
+        tb = lambda a: a[:steps].transpose(0, 1).clone(memory_format=torch.contiguous_format)
+        lenths = np.array(lens_hist, dtype=np.int64).T                 # [B, steps]
+        rb = dict(lang_in, corners_px=tb(bf["px_hist"]),
+                  directions=bf["dirs"][:, :steps].clone(memory_format=torch.contiguous_format),
+                  tile_idx=None if ti is None else ti.view(B, 1).expand(B, steps).contiguous(),
+                  gt_xy=tb(bf["tgt_xy"]), gt_alt=tb(bf["tgt_alt"]), gt_prog=tb(bf["tgt_prog"]), lenths=lenths.tolist())
+        self._last_rollout = dict(
+            corners=bf["corners_hist"][:steps + 1].clone(), directions=bf["dir_hist"][:steps + 1].clone(),
+            ended=bf["ended_hist"][:steps].clone(), output=bf["output_hist"][:steps].clone(), steps=steps,
+            lenths=lenths, tgt_xy=bf["tgt_xy"][:steps].clone(), tgt_alt=bf["tgt_alt"][:steps].clone(),
+            tgt_prog=bf["tgt_prog"][:steps].clone(), batch=rb)
+        return float(self.loss_total.item()) if sync_loss else self.loss_total
+
     # ----------------------------------------------------------------- inference
     STOP_THRESHOLD = 0.5               # agent.py:738-745 (the LSTM agent uses 0.25)
 
@@ -713,6 +940,9 @@ class NavCMTAgent(RolloutTrainer):
           inside it and ``train`` only clips and steps.  Teacher feedback: the poses come from the ground-truth
           actions; student feedback: from a no-grad greedy rollout (``student_batch``).  Language: tokenizer +
           ``CustomBERTModel``, trained in the loop.
+        * ``args.on_policy_student`` (default false): a student-feedback training rollout is instead one
+          ``student_rollout_step``, the reference's single pass -- the poses follow the train-mode predictions that
+          are trained (trunk on per-step batch statistics, dropout on), as in agent.py:580-760.
         * ``not_in_train``: no gradients; student feedback is ``rollout_greedy``; teacher feedback additionally logs
           ``human_att_performance`` / ``nss`` per step (agent.py:683-693)."""
         env = self.env
@@ -741,6 +971,9 @@ class NavCMTAgent(RolloutTrainer):
                     tgt = (xy.view(steps, B, 2).cpu().numpy(), alt.view(steps, B).cpu().numpy(),
                            pr.view(steps, B).cpu().numpy())
                 self._log_traj(traj, outs, tgt, ended, c_h, d_h, steps)
+                return traj
+            if self.feedback == "student" and not not_in_train and getattr(self.args, "on_policy_student", False):
+                self._on_policy_rollout(lb, gps0, dirs0, geo, tidx, gt_paths, traj, T, train_ml, nss_w, has_gt)
                 return traj
             # ---- poses of the rollout ----
             if self.feedback == "teacher":
@@ -800,6 +1033,21 @@ class NavCMTAgent(RolloutTrainer):
         finally:
             self.renderer = prev_r
         return traj
+
+    def _on_policy_rollout(self, lb, gps0, dirs0, geo, tidx, gt_paths, traj, T, train_ml, nss_w, has_gt):
+        """The student-feedback training rollout of ``rollout`` with ``args.on_policy_student``: one
+        ``student_rollout_step`` (BERT, trunk and ET in train mode; the poses follow the train-mode predictions).
+        The trajectory dicts log the outputs and poses the rollout used."""
+        outs = []
+        batch = dict(lb, corners_gps=torch.from_numpy(gps0).to(self.device), directions=dirs0, geo=geo, tile_idx=tidx)
+        loss = self.student_rollout_step(batch, gt_paths, max_action_len=T, nss_w=float(nss_w),
+                                         train_ml=train_ml if train_ml is not None else 0.0, zero=False, step=False,
+                                         collect=outs)
+        lr = self._last_rollout
+        tgt = (lr["tgt_xy"].cpu().numpy(), lr["tgt_alt"].cpu().numpy(), lr["tgt_prog"].cpu().numpy()) if has_gt else None
+        self._log_traj(traj, torch.stack(outs).cpu().numpy(), tgt, lr["ended"].cpu().numpy().astype(bool),
+                       lr["corners"].cpu().numpy(), lr["directions"].cpu().numpy(), lr["steps"])
+        self._add_rollout_loss(loss, train_ml)
 
     @torch.no_grad()
     def _eval_rollout(self, batch, traj, outs):
