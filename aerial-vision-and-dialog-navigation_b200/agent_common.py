@@ -2,8 +2,9 @@
 the batch-level training API (``RolloutTrainer``: loss weights, ``train_rollout_step``, ``train_iteration``, the
 loss log, ``teacher_action``), the model-independent parts of the reference's agent loop (tokenizer, BERT passes,
 teacher poses, trajectory dicts, ``train``, ``test``, ``save`` / ``load``), the views and trunk passes of a
-teacher-forced training rollout, and the targets of a student-feedback rollout.  Each agent supplies
-``_train_rollout_step`` (its policy's forward, loss and backward), ``rollout`` and ``_checkpoint_items``."""
+teacher-forced training rollout, the targets of the poses a student-feedback rollout visited (``student_targets``)
+and the pose batch of a rollout (``rollout_pose_batch``).  Each agent supplies ``_train_rollout_step`` (its policy's
+forward, loss and backward), ``rollout`` and ``_checkpoint_items``."""
 from __future__ import annotations
 
 import os
@@ -155,6 +156,8 @@ class RolloutTrainer:
         """BERT in eval mode over a ``_language_batch``: (sequence output, ``linear_cls``) -- the latter from the
         second pass over ``pre_dialogs + instructions`` when the batch has one (agent.py:519-538)."""
         lm, dev = self.lang_model, self.device
+        if lm is None:
+            raise RuntimeError("batch carries input_ids but no language model is attached (attach_lang_model)")
         lm.eval()
         leng = lm.engine(lb["input_ids"].shape[0], lb["input_ids"].shape[1], dev)
         leng.set_dropout(*lm.dropout_config())
@@ -528,25 +531,30 @@ def rollout_trunk_backward(agent, teng, tengs, l0, d_frames, B, T, after_layer=N
     return steps + sum(e.launches for e in tengs) - l0
 
 
-def student_rollout_targets(agent, batch, res, gt_path_corners):
-    """Training targets of a no-grad greedy rollout ``res`` (``rollout_greedy``'s result for ``batch``): the
-    ``teacher_action`` target of every step in one launch (student feedback, agent.py:655-661) and the pixel corners
-    of every pose.  Returns (dict of [B,T,...] tensors ``corners_px``, ``tile_idx``, ``gt_xy``, ``gt_alt``,
-    ``gt_prog``; ``ended_before`` [T,B] u8 -- the sample had stopped before step t; T)."""
-    T = int(res.get("steps", res["ended"].shape[0]))
-    corners = res["corners"][:T]                                   # [T,B,4,2] gps
-    B = corners.shape[1]
+def student_targets(agent, corners, ended, gt_path_corners):
+    """The ``teacher_action`` target of every pose a student-feedback rollout visited (agent.py:655-661), in one
+    launch.  ``corners`` [T,B,4,2] f64 (lat,lng) the pose before each step; ``ended`` [T,B] the sticky stop flags
+    after each step -- the teacher sees at step t whether the sample had stopped before it; ``gt_path_corners``: per
+    sample the ``[n_i,4,2]`` ground-truth view corners.  Returns ``(xy [T,B,2], alt [T,B], prog [T,B])`` f32."""
+    T, B = corners.shape[0], corners.shape[1]
     ended_before = torch.zeros((T, B), dtype=torch.uint8, device=agent.device)
-    ended_before[1:] = res["ended"][:T - 1]
-    tgt_xy, tgt_alt, prog = agent.teacher_action(corners.reshape(T * B, 4, 2),
-                                                 [gt_path_corners[k % B] for k in range(T * B)],
-                                                 ended_before.reshape(-1), feedback="student")
-    geo = batch["geo"].contiguous()
-    px = torch.empty((T * B, 4, 2), dtype=torch.int32, device=agent.device)
+    ended_before[1:] = ended[:T - 1]
+    xy, alt, prog = agent.teacher_action(corners.reshape(T * B, 4, 2), [gt_path_corners[k % B] for k in range(T * B)],
+                                         ended_before.reshape(-1), feedback="student")
+    return xy.view(T, B, 2), alt.view(T, B), prog.view(T, B)
+
+
+def rollout_pose_batch(corners, geo, tile_idx, targets):
+    """The poses of a ``train_rollout_step`` batch: a rollout that visited ``corners`` [T,B,4,2] (f64 lat,lng) on the
+    maps ``geo`` [B,5] (``tile_idx`` i32 [B] or None), with ``targets`` = ``(xy [T,B,2], alt [T,B], prog [T,B])``.
+    Returns a dict of [B,T,...] tensors ``corners_px`` (i32 pixel corners), ``tile_idx`` (or None), ``gt_xy``,
+    ``gt_alt`` and ``gt_prog``."""
+    T, B = corners.shape[0], corners.shape[1]
+    px = torch.empty((T * B, 4, 2), dtype=torch.int32, device=corners.device)
     _lib.call("avdn_gps_to_pixels", _lib.ptr(corners.reshape(T * B, 4, 2).contiguous()),
               _lib.ptr(geo.repeat(T, 1).contiguous()), T * B, _lib.ptr(px))
-    tb = lambda a: a.view(T, B, *a.shape[1:]).transpose(0, 1).contiguous()
-    ti = batch.get("tile_idx")
-    out = dict(corners_px=tb(px), tile_idx=None if ti is None else ti.view(B, 1).expand(B, T).contiguous(),
-               gt_xy=tb(tgt_xy.float()), gt_alt=tb(tgt_alt.float()), gt_prog=tb(prog.float()))
-    return out, ended_before, T
+    tb = lambda a: a.transpose(0, 1).contiguous()                  # step-major [T,B,...] -> [B,T,...]
+    xy, alt, prog = targets
+    return dict(corners_px=tb(px.view(T, B, 4, 2)),
+                tile_idx=None if tile_idx is None else tile_idx.view(B, 1).expand(B, T).contiguous(),
+                gt_xy=tb(xy.float()), gt_alt=tb(alt.float()), gt_prog=tb(prog.float()))

@@ -31,6 +31,10 @@ What is here
   training rollout in one pass -- every step renders the current views, runs its own train-mode trunk pass and the
   ET in train mode over the history, takes the step's loss and backward, and moves the simulator by that same
   train-mode prediction.
+
+Both training rollouts run each step of their ET pass as ``_history_step_forward`` and ``_history_step_backward``;
+``train_step`` and both rollouts end in ``_finish_backward`` (BERT backward, all-reduce, trunk backward, optimiser).
+``history_lengths`` gives the ``lenths`` of a rollout whose poses are known in advance.
 """
 from __future__ import annotations
 
@@ -46,8 +50,8 @@ from ..models import dark_net as DN
 from ..models.dark_net import Darknet
 from ..optim import FusedAdamW
 from .. import parallel
-from ..agent_common import (RolloutTrainer, pack_gt_paths, render_rollout_views, rollout_step_bufs,
-                            rollout_trunk_backward, rollout_trunk_forward, student_rollout_targets)
+from ..agent_common import (RolloutTrainer, pack_gt_paths, render_rollout_views, rollout_pose_batch,
+                            rollout_step_bufs, rollout_trunk_backward, rollout_trunk_forward, student_targets)
 
 PI_REF = 3.14159
 
@@ -62,6 +66,15 @@ def get_direction(start, end):
     else:
         ang = 90 if np.sign(vec[0]) == 1 else 270
     return (360 - ang + 90) % 360
+
+
+def history_lengths(ended):
+    """The ``lenths`` of a rollout (agent.py:603-620): the history length each sample's ET sees at step t -- it grows
+    by one every step until the sample has ended, then stays.  ``ended`` host bool [T,B]: the sticky stop flags after
+    each step.  Returns int64 [B,T]."""
+    alive = np.ones(ended.shape, dtype=bool)
+    alive[1:] = ~ended[:-1]
+    return np.cumsum(alive, axis=0).T
 
 
 class NavCMTAgent(RolloutTrainer):
@@ -190,31 +203,17 @@ class NavCMTAgent(RolloutTrainer):
         bf16 [B*T,224,224,4] (pre-rendered, normalised NHWC); ``tile_idx`` i32 [B,T] or None;
         ``lang`` f32 [B,L,768]; ``lang_cls`` f32 [B,49]; ``directions`` f32 [B,T,2];
         ``lenths`` host list[int]; ``gt_xy`` [B,2], ``gt_alt`` [B], ``gt_prog`` [B] f32;
-        optional ``att`` u8 [B,224,224], ``jitter`` f32 [B]."""
+        optional ``att`` u8 [B,224,224], ``jitter`` f32 [B]; or, with an attached language model, ``input_ids`` /
+        ``attention_mask`` (and optionally ``cls_input_ids`` / ``cls_attention_mask``) instead of ``lang`` /
+        ``lang_cls``.  Sets ``self._ctx = (trunk engine, ET engine, buffers)``; returns ``(output, h_sali, BERT
+        engines of the training pass or None, trunk launch count before the pass, ET launch count before the pass)``."""
         ptr = _lib.ptr
-        self._lang_eng = None
+        lengs = None
         if "input_ids" in batch:
-            if self.lang_model is None:
-                raise RuntimeError("batch carries input_ids but no language model is attached (attach_lang_model)")
-            lm = self.lang_model
-            lm.train(bool(train) and not getattr(self.args, "no_dropout", False))
-            ids, am = batch["input_ids"], batch["attention_mask"]
-            leng = lm.engine(ids.shape[0], ids.shape[1], self.device)
-            leng.set_dropout(*lm.dropout_config())
-            l0l = leng.launches
-            seq, lin, _ = leng.forward(ids.long(), am)
-            self.launches += leng.launches - l0l
-            self._lang_eng = leng
-            self._lang_eng_cls = None
-            if "cls_input_ids" in batch:
-                # agent.py:530-538: ``linear_cls`` comes from a second pass over pre_dialogs + instructions
-                ids2, am2 = batch["cls_input_ids"], batch["cls_attention_mask"]
-                leng2 = lm.engine(ids2.shape[0], ids2.shape[1], self.device, slot=1)
-                leng2.set_dropout(*lm.dropout_config())
-                l0l = leng2.launches
-                _, lin, _ = leng2.forward(ids2.long(), am2)
-                self.launches += leng2.launches - l0l
-                self._lang_eng_cls = leng2
+            if train:
+                seq, lin, *lengs = self._lang_train_forward(batch)
+            else:
+                seq, lin = self._lang_eval_forward(batch)
             batch = dict(batch, lang=seq, lang_cls=lin)
         lang, lang_cls, dirs = batch["lang"], batch["lang_cls"], batch["directions"]
         B, T = dirs.shape[0], dirs.shape[1]
@@ -258,14 +257,14 @@ class NavCMTAgent(RolloutTrainer):
                   int(getattr(self.args, "nss_r", 0)), scale, ptr(self.loss_total), ptr(bufs["loss_i"]),
                   ptr(bufs["d_output"]), ptr(bufs["d_h_sali"]))
         n += 2
-        self._ctx = (teng, eng, bufs, l0, e0)
+        self._ctx = (teng, eng, bufs)
         self.launches += n
-        return output, h_sali
+        return output, h_sali, lengs, l0, e0
 
     def forward_loss(self, batch):
         """Validation: forward + loss (trunk in eval mode).  Returns (loss, output, h_sali)."""
         self.vision_model.eval()
-        output, h_sali = self._forward(batch, False)
+        output, h_sali, _, _, _ = self._forward(batch, False)
         return self.loss_total.clone(), output, h_sali
 
     def train_step(self, batch, sync_loss=False):
@@ -275,47 +274,51 @@ class NavCMTAgent(RolloutTrainer):
         for opt in self.optimizers:
             opt.zero_grad()
         self.launches += 2
-        self._forward(batch, True)
-        teng, eng, bufs, l0, e0 = self._ctx
-        leng = self._lang_eng
-        if leng is None:
+        _, _, lengs, l0, e0 = self._forward(batch, True)
+        teng, eng, bufs = self._ctx
+        lang = None
+        if lengs is None:
             eng.backward(bufs["d_output"], bufs["d_h_sali"], d_frames=bufs["d_frames"])
         else:
             d_cls = torch.zeros((eng.B, 49), dtype=torch.float32, device=self.device)
             _, d_lang = eng.backward(bufs["d_output"], bufs["d_h_sali"], d_frames=bufs["d_frames"], need_lang_grad=True,
                                      d_lang_cls=d_cls)
-            leng2 = self._lang_eng_cls
-            l0l = leng.launches
-            if leng2 is None:
-                leng.backward(d_lang, d_cls, None)
-            else:                          # both passes accumulate into the one gradient arena
-                leng.backward(d_lang, None, None)
-                l1 = leng2.launches
-                leng2.backward(None, d_cls, None)
-                self.launches += leng2.launches - l1
-            self.launches += leng.launches - l0l
-        dp = self.world > 1
+            lang = (*lengs, d_lang, d_cls)
+        n = self._finish_backward(lang, teng, None, l0, bufs["d_frames"], eng.B, eng.T)
+        self.launches += n + (eng.launches - e0)
+        self._log_loss()
+        if sync_loss:
+            return float(self.loss_total.item())
+        return self.loss_total
+
+    def _finish_backward(self, lang, teng, tengs, l0, d_frames, B, T, steps=None, step=True):
+        """What follows the ET backward of ``train_step`` and both training rollouts: BERT's backward of ``lang`` =
+        (engine, cls engine, d_lang, d_cls) from ``_lang_train_forward``, or None; with ``step`` on more than one GPU
+        the all-reduce of the language and ET arenas and of the trunk's gradient buckets as the trunk backward
+        completes them (gradients are reduced once, after the iteration's last rollout); ``rollout_trunk_backward``
+        (arguments as there); then, with ``step``, every optimiser with ``grad_scale = 1/world``.  Returns the
+        launches of the trunk, forward included, and of the optimisers."""
+        if lang is not None:
+            self._lang_train_backward(*lang)
+        dp = self.world > 1 and step
+        hook = flush = None
         if dp:
-            if leng is not None:
+            if self.lang_optimizer is not None:
                 self._allreduce_async(self.lang_optimizer.g, 0, self.lang_optimizer.n)
             self._allreduce_async(self.et_optimizer.g, 0, self.et_optimizer.n)
             buckets = {c: (lo, hi) for c, lo, hi in self._trunk_buckets(teng)}
             hook = lambda li: (self._allreduce_async(self.vision_model_optimizer.g, *buckets[li])
                                if li in buckets else None)
-        else:
-            hook = None
-        DN._trunk_backward(self.vision_model, teng, bufs["d_frames"].view(-1, 512, 7, 7), after_layer=hook,
-                           flush_layers=set(buckets) if dp else None)
+            flush = set(buckets)
+        n = rollout_trunk_backward(self, teng, tengs, l0, d_frames, B, T, after_layer=hook, flush_layers=flush,
+                                   steps=steps)
         if dp:
             self._wait_comm()
-        gs = 1.0 / self.world
-        for opt in self.optimizers:
-            self.launches += opt.step(grad_scale=gs)
-        self.launches += (teng.launches - l0) + (eng.launches - e0)
-        self._log_loss()
-        if sync_loss:
-            return float(self.loss_total.item())
-        return self.loss_total
+        if step:
+            gs = 1.0 / self.world
+            for opt in self.optimizers:
+                n += opt.step(grad_scale=gs)
+        return n
 
     def _wait_comm(self):
         """The optimiser waits for the last gradient bucket; with ``exposed_events`` set (bench) the wait is bracketed
@@ -357,23 +360,21 @@ class NavCMTAgent(RolloutTrainer):
         ``bn_per_step`` (default ``args.bn_per_step``, false): the reference's BatchNorm semantics -- one train-mode
         trunk pass per time step over that step's B views (its own batch statistics, one running-statistics update
         per step, agent.py:593), each pass kept for its own backward -- instead of one pass over all B*T views."""
-        ptr = _lib.ptr
         self.vision_model.train()
         n = 0
         if zero:
             for opt in self.optimizers:
                 opt.zero_grad()
             n += 2
-        leng = leng2 = None
+        lengs = None
         if "input_ids" in batch:
             # the language encoder runs once per rollout (agent.py:519-538) and collects the gradients of all steps
-            seq, lin, leng, leng2 = self._lang_train_forward(batch)
+            seq, lin, *lengs = self._lang_train_forward(batch)
             batch = dict(batch, lang=seq, lang_cls=lin)
         dirs = batch["directions"].contiguous().float()
         B, T = dirs.shape[0], dirs.shape[1]
         BT = B * T
         lang, lang_cls = batch["lang"].contiguous().float(), batch["lang_cls"].contiguous().float()
-        L = lang.shape[1]
         dev = self.device
         bufs = self._get_bufs(B, T)
         key = ("rollout_train", B, T)
@@ -384,7 +385,6 @@ class NavCMTAgent(RolloutTrainer):
             self._bufs[key] = xb
         x, att, k = render_rollout_views(self, batch, BT, bufs["x"], xb["att"])
         n += k
-        vm, et = self.vision_model, self.vln_model
         teng, tengs, l0, k = rollout_trunk_forward(self, x, B, T, bufs["frames"], bn_per_step)
         n += k
         # ---- step t: the encoder over the history [:t+1], its loss, and straight back (the loss is a sum over steps,
@@ -400,63 +400,62 @@ class NavCMTAgent(RolloutTrainer):
         jit = None if jit is None else jit.float().transpose(0, 1).contiguous()
         att_t = None if att is None else att.view(B, T, 224, 224).transpose(0, 1).contiguous()
         n += 6
-        et.train(not getattr(self.args, "no_dropout", False))
+        self.vln_model.train(not getattr(self.args, "no_dropout", False))
         self.loss_total.zero_()
-        scale = float(self.train_ml) / B                               # agent.py:883-885
-        pe = et.encoder_vl.enc_pos.pe[0]
+        d_lang = None                              # the sums of every step's lang / lang_cls gradients
+        if lengs is not None:
+            d_lang = (torch.zeros((B, lang.shape[1], 768), dtype=torch.float32, device=dev),
+                      torch.zeros((B, 49), dtype=torch.float32, device=dev))
         et_launches = 0
-        if leng is not None:
-            d_lang_sum = torch.zeros((B, L, 768), dtype=torch.float32, device=dev)
-            d_cls_sum = torch.zeros((B, 49), dtype=torch.float32, device=dev)      # every step adds into it
         for t in range(T):
-            Tc = t + 1
-            eng = et.engine(B, L, Tc, dev)
-            e0 = eng.launches
-            eng.set_dropout(*et.dropout_config())
-            f_t = frames[:, :Tc].contiguous().view(B * Tc, 512, 49)
-            output, h_sali = eng.forward(f_t, lang, lang_cls, dirs[:, :Tc].contiguous(),
-                                         [int(lens[i][t]) for i in range(B)] if lens is not None else [Tc] * B, pe)
-            _lib.call("avdn_loss", ptr(output), ptr(h_sali), ptr(gt_xy[t]), ptr(gt_alt[t]), ptr(gt_prog[t]),
-                      ptr(None if att_t is None else att_t[t]), ptr(None if jit is None else jit[t]), B,
-                      float(self.nss_w), int(getattr(self.args, "nss_r", 0)), scale, ptr(self.loss_total),
-                      ptr(bufs["loss_i"]), ptr(bufs["d_output"]), ptr(bufs["d_h_sali"]))
+            lens_t = [int(lens[i][t]) for i in range(B)] if lens is not None else [t + 1] * B
+            eng, e0, output = self._history_step_forward(t, frames, dirs, lang, lang_cls, lens_t,
+                                                         (gt_xy[t], gt_alt[t], gt_prog[t]),
+                                                         None if att_t is None else att_t[t],
+                                                         None if jit is None else jit[t], bufs)
             if collect is not None:
                 collect.append(output.detach().clone())
-            if leng is None:
-                df, _ = eng.backward(bufs["d_output"], bufs["d_h_sali"], d_frames=xb["d_frames"][:B * Tc])
-            else:
-                df, d_lang = eng.backward(bufs["d_output"], bufs["d_h_sali"], d_frames=xb["d_frames"][:B * Tc],
-                                          need_lang_grad=True, d_lang_cls=d_cls_sum)
-                d_lang_sum += d_lang.view(B, L, 768)
-                n += 1
-            d_frames[:, :Tc] += df.view(B, Tc, 512, 49)
-            n += 5
-            et_launches += eng.launches - e0
-        e0 = eng.launches - et_launches
-        if leng is not None:
-            self._lang_train_backward(leng, leng2, d_lang_sum, d_cls_sum)
-        self._ctx = (teng, eng, bufs, l0, e0)
-        dp = self.world > 1 and step               # gradients are reduced once, after the iteration's last rollout
-        if dp:
-            if self.lang_optimizer is not None:
-                self._allreduce_async(self.lang_optimizer.g, 0, self.lang_optimizer.n)
-            self._allreduce_async(self.et_optimizer.g, 0, self.et_optimizer.n)
-            buckets = {c: (lo, hi) for c, lo, hi in self._trunk_buckets(teng)}
-            hook = lambda li: (self._allreduce_async(self.vision_model_optimizer.g, *buckets[li])
-                               if li in buckets else None)
-        else:
-            hook = None
-        trunk_launches = rollout_trunk_backward(self, teng, tengs, l0, bufs["d_frames"], B, T, after_layer=hook,
-                                                flush_layers=set(buckets) if dp else None)
-        if dp:
-            self._wait_comm()
-        if step:
-            gs = 1.0 / self.world
-            for opt in self.optimizers:
-                n += opt.step(grad_scale=gs)
-        self.launches += n + trunk_launches + (eng.launches - e0)
+            et_launches += self._history_step_backward(eng, e0, bufs, xb["d_frames"], d_frames, d_lang)
+            n += 4
+        self._ctx = (teng, eng, bufs)
+        n += self._finish_backward(None if lengs is None else (*lengs, *d_lang), teng, tengs, l0, bufs["d_frames"],
+                                   B, T, step=step)
+        self.launches += n + et_launches
         self._log_loss()
         return float(self.loss_total.item()) if sync_loss else self.loss_total
+
+    def _history_step_forward(self, t, frames, dirs, lang, lang_cls, lens, targets, att, jitter, gb):
+        """Step t of a training rollout's ET pass: the ET over the history ``[:t+1]`` of ``frames`` [B,T,512,49] /
+        ``dirs`` [B,T,2] (fresh dropout masks) with the history lengths ``lens``, then the step's ``avdn_loss`` against
+        ``targets`` = (xy [B,2], alt [B], prog [B]) into ``loss_total`` and ``gb``'s output gradients.  Returns
+        (engine, its launch count before the step, output [B,4])."""
+        ptr = _lib.ptr
+        et = self.vln_model
+        B, L, Tc = lang.shape[0], lang.shape[1], t + 1
+        eng = et.engine(B, L, Tc, self.device)
+        e0 = eng.launches
+        eng.set_dropout(*et.dropout_config())
+        output, h_sali = eng.forward(frames[:, :Tc].contiguous().view(B * Tc, 512, 49), lang, lang_cls,
+                                     dirs[:, :Tc].contiguous(), lens, et.encoder_vl.enc_pos.pe[0])
+        xy, alt, prog = targets
+        _lib.call("avdn_loss", ptr(output), ptr(h_sali), ptr(xy), ptr(alt), ptr(prog), ptr(att), ptr(jitter), B,
+                  float(self.nss_w), int(getattr(self.args, "nss_r", 0)), float(self.train_ml) / B,   # agent.py:883-885
+                  ptr(self.loss_total), ptr(gb["loss_i"]), ptr(gb["d_output"]), ptr(gb["d_h_sali"]))
+        return eng, e0, output
+
+    def _history_step_backward(self, eng, e0, gb, d_frames_t, d_frames, d_lang):
+        """The backward of ``_history_step_forward``'s step: the frame gradients (into the scratch ``d_frames_t``) are
+        added into the history's ``d_frames`` [B,T,512,49], and with ``d_lang`` = (sum [B,L,768], sum [B,49]) the
+        language gradients into it.  Returns the step's launches since ``e0``."""
+        B, L, Tc = eng.B, eng.L, eng.T
+        if d_lang is None:
+            df, _ = eng.backward(gb["d_output"], gb["d_h_sali"], d_frames=d_frames_t[:B * Tc])
+        else:
+            df, dl = eng.backward(gb["d_output"], gb["d_h_sali"], d_frames=d_frames_t[:B * Tc], need_lang_grad=True,
+                                  d_lang_cls=d_lang[1])
+            d_lang[0].add_(dl.view(B, L, 768))
+        d_frames[:, :Tc] += df.view(B, Tc, 512, 49)
+        return eng.launches - e0 + 1 + (d_lang is not None)
 
     @torch.no_grad()
     def student_batch(self, batch, gt_path_corners, max_action_len=None):
@@ -465,13 +464,14 @@ class NavCMTAgent(RolloutTrainer):
         result is a ``train_rollout_step`` batch.  ``batch`` as for ``rollout_greedy``; returns the training batch
         (device tensors; ``lenths`` from the steps each sample was alive)."""
         res = self.rollout_greedy(batch, max_action_len=max_action_len)
-        out, ended_before, T = student_rollout_targets(self, batch, res, gt_path_corners)
+        T = int(res["steps"])
+        corners, ended = res["corners"][:T], res["ended"][:T]
+        out = rollout_pose_batch(corners, batch["geo"], batch.get("tile_idx"),
+                                 student_targets(self, corners, ended, gt_path_corners))
         rad = res["directions"][:T].float() / 180 * PI_REF
-        alive = (ended_before == 0).cpu().numpy()
-        lens = np.cumsum(alive, axis=0).T                              # [B,T]: history length seen at step t
         out.update(lang=batch["lang"], lang_cls=batch["lang_cls"],
                    directions=torch.stack([torch.sin(rad), torch.cos(rad)], -1).transpose(0, 1).contiguous(),
-                   lenths=np.maximum(lens, 1).tolist())
+                   lenths=history_lengths(ended.cpu().numpy().astype(bool)).tolist())
         return out
 
     _LANG_KEYS = ("lang", "lang_cls", "input_ids", "attention_mask", "cls_input_ids", "cls_attention_mask")
@@ -483,12 +483,13 @@ class NavCMTAgent(RolloutTrainer):
         same train-mode prediction (stop threshold 0.5), so the model is trained on the states its own train-mode
         policy visits.  Step t: render the B current views into trunk slot ``1 + t`` and run a train-mode pass on
         the step's own batch statistics (kept for the backward) -> the features and the heading join the history,
-        ``lenths`` grows for the samples that have not ended (agent.py:603-620) -> the ET over the history
-        ``[:t+1]`` with fresh dropout masks -> the ``teacher_action`` target at the pose -> ``avdn_loss`` ->
-        ``avdn_waypoint_step`` -> the ET backward of the step, its frame gradients added into the history's.  One
-        host read of the B stop flags per step gives the next step's ``lenths``; the loop stops after the step at
-        which every sample has ended (agent.py:773-774).  Then the BERT backward, the trunk backward of the executed
-        passes and (``step``) the data-parallel reduction and the optimiser step, as in ``train_rollout_step``.
+        ``lenths`` grows for the samples that have not ended (agent.py:603-620) -> the ``teacher_action`` target at
+        the pose -> the ET over the history ``[:t+1]`` with fresh dropout masks and ``avdn_loss``
+        (``_history_step_forward``) -> ``avdn_waypoint_step`` -> the ET backward of the step, its frame gradients
+        added into the history's (``_history_step_backward``).  One host read of the B stop flags per step gives the
+        next step's ``lenths``; the loop stops after the step at which every sample has ended (agent.py:773-774).
+        Then ``_finish_backward``, as in ``train_rollout_step``: the BERT backward, the trunk backward of the executed
+        passes and (``step``) the data-parallel reduction and the optimiser step.
 
         ``batch`` as for ``rollout_greedy``; with an attached language model it may carry ``input_ids`` /
         ``attention_mask`` (and ``cls_*``) instead of ``lang`` / ``lang_cls``: BERT then runs once in train mode,
@@ -549,10 +550,10 @@ class NavCMTAgent(RolloutTrainer):
                 opt.zero_grad()
             n += 2
         lang_in = {k: batch[k] for k in self._LANG_KEYS if k in batch}
-        leng = leng2 = None
+        lengs = None
         if "input_ids" in batch:
             # the language encoder runs once per rollout (agent.py:519-538): its train-mode outputs steer the rollout
-            seq, lin, leng, leng2 = self._lang_train_forward(batch)
+            seq, lin, *lengs = self._lang_train_forward(batch)
             batch = dict(batch, lang=seq, lang_cls=lin)
         lang, lang_cls = batch["lang"].contiguous().float(), batch["lang_cls"].contiguous().float()
         B, L = lang.shape[0], lang.shape[1]
@@ -573,20 +574,17 @@ class NavCMTAgent(RolloutTrainer):
         if no_dir:
             bf["dirs"].zero_()
         self.loss_total.zero_()
-        scale = float(self.train_ml) / B                               # agent.py:883-885
-        nss_w, nss_r = float(self.nss_w), int(getattr(self.args, "nss_r", 0))
         thr = float(self.STOP_THRESHOLD)
-        pe = et.encoder_vl.enc_pos.pe[0]
-        if leng is not None:
-            d_lang_sum = torch.zeros((B, L, 768), dtype=torch.float32, device=dev)
-            d_cls_sum = torch.zeros((B, 49), dtype=torch.float32, device=dev)      # every step adds into it
+        d_lang = None                              # the sums of every step's lang / lang_cls gradients
+        if lengs is not None:
+            d_lang = (torch.zeros((B, L, 768), dtype=torch.float32, device=dev),
+                      torch.zeros((B, 49), dtype=torch.float32, device=dev))
         lens = [0] * B
         lens_hist = []                                                 # [steps][B]: history length seen at step t
         ended_host = np.zeros(B, dtype=bool)
         tengs, l0, et_launches = [], 0, 0
         steps = T
         for t in range(T):
-            Tc = t + 1
             # ---- 1. the pose and its observation (agent.py:742): the views into this step's trunk slot ----
             bf["corners_hist"][t].copy_(bf["corners"])
             bf["dir_hist"][t].copy_(bf["cur_dir"])
@@ -597,7 +595,7 @@ class NavCMTAgent(RolloutTrainer):
             call("avdn_homography_from_corners", ptr(px), B, ptr(bf["minv"]))
             r.render(None, ti, views=False, norm_nhwc=True, minv=bf["minv"], out={"norm_nhwc": sb["x"][t]})
             att = None
-            if nss_w != 0:
+            if self.nss_w != 0:
                 r.render(None, ti, views=False, att=True, minv=bf["minv"], out={"att": bf["att"]})
                 att = bf["att"]
                 n += 1
@@ -616,16 +614,11 @@ class NavCMTAgent(RolloutTrainer):
                 if not ended_host[i]:
                     lens[i] += 1
             lens_hist.append(list(lens))
-            # ---- 4. the ET over the history [:t+1], train mode, fresh dropout masks ----
-            eng = et.engine(B, L, Tc, dev)
-            e0 = eng.launches
-            eng.set_dropout(*et.dropout_config())
-            f_t = bf["frames"][:, :Tc].contiguous().view(B * Tc, 512, 49)
-            output, h_sali = eng.forward(f_t, lang, lang_cls, bf["dirs"][:, :Tc].contiguous(), lens, pe)
-            # ---- 5. the teacher's target at the pose (agent.py:655-661) and 6. the step's loss ----
+            # ---- 4. the teacher's target at the pose (agent.py:655-661), 5. the ET over the history [:t+1] (train
+            #      mode, fresh dropout masks) and 6. the step's loss ----
             xy, alt, prog = self.teacher_action(bf["corners"], gt_pack, bf["ended_before"][t], feedback="student")
-            call("avdn_loss", ptr(output), ptr(h_sali), ptr(xy), ptr(alt), ptr(prog), ptr(att), None, B, nss_w, nss_r,
-                 scale, ptr(self.loss_total), ptr(bf["loss_i"]), ptr(bf["d_output"]), ptr(bf["d_h_sali"]))
+            eng, e0, output = self._history_step_forward(t, bf["frames"], bf["dirs"], lang, lang_cls, lens,
+                                                         (xy, alt, prog), att, None, bf)
             bf["tgt_xy"][t].copy_(xy)
             bf["tgt_alt"][t].copy_(alt)
             bf["tgt_prog"][t].copy_(prog)
@@ -638,16 +631,8 @@ class NavCMTAgent(RolloutTrainer):
                  ptr(bf["altitude"][t]))
             bf["ended_hist"][t].copy_(bf["ended"])
             # ---- 8. the step's backward straight away: one encoder's activations are alive at a time ----
-            if leng is None:
-                df, _ = eng.backward(bf["d_output"], bf["d_h_sali"], d_frames=bf["d_frames_t"][:B * Tc])
-            else:
-                df, d_lang = eng.backward(bf["d_output"], bf["d_h_sali"], d_frames=bf["d_frames_t"][:B * Tc],
-                                          need_lang_grad=True, d_lang_cls=d_cls_sum)
-                d_lang_sum += d_lang.view(B, L, 768)
-                n += 1
-            bf["d_frames"][:, :Tc] += df.view(B, Tc, 512, 49)
-            et_launches += eng.launches - e0
-            n += 20                                 # the step's kernels outside the trunk and ET engines
+            et_launches += self._history_step_backward(eng, e0, bf, bf["d_frames_t"], bf["d_frames"], d_lang)
+            n += 19                                 # the step's other kernels outside the trunk and ET engines
             # ---- 9. the step's only host read: the stop flags (next lenths; agent.py:773-774 early exit) ----
             if t < T - 1:
                 bf["ended_h"].copy_(bf["ended"])
@@ -657,28 +642,10 @@ class NavCMTAgent(RolloutTrainer):
                     break
         bf["corners_hist"][steps].copy_(bf["corners"])
         bf["dir_hist"][steps].copy_(bf["cur_dir"])
-        if leng is not None:
-            self._lang_train_backward(leng, leng2, d_lang_sum, d_cls_sum)
-        self._ctx = (tengs[0], eng, bf, l0, eng.launches - et_launches)
-        dp = self.world > 1 and step               # gradients are reduced once, after the iteration's last rollout
-        if dp:
-            if self.lang_optimizer is not None:
-                self._allreduce_async(self.lang_optimizer.g, 0, self.lang_optimizer.n)
-            self._allreduce_async(self.et_optimizer.g, 0, self.et_optimizer.n)
-            buckets = {c: (lo, hi) for c, lo, hi in self._trunk_buckets(tengs[0])}
-            hook = lambda li: (self._allreduce_async(self.vision_model_optimizer.g, *buckets[li])
-                               if li in buckets else None)
-        else:
-            hook = None
-        trunk_launches = rollout_trunk_backward(self, tengs[0], tengs, l0, bf["d_frames"], B, T, after_layer=hook,
-                                                flush_layers=set(buckets) if dp else None, steps=steps)
-        if dp:
-            self._wait_comm()
-        if step:
-            gs = 1.0 / self.world
-            for opt in self.optimizers:
-                n += opt.step(grad_scale=gs)
-        self.launches += n + trunk_launches + et_launches
+        self._ctx = (tengs[0], eng, bf)
+        n += self._finish_backward(None if lengs is None else (*lengs, *d_lang), tengs[0], tengs, l0, bf["d_frames"],
+                                   B, T, steps, step)
+        self.launches += n + et_launches
         self._log_loss()
         # what the rollout visited (inspection / tests): poses before every step and after the last, stop flags,
         # train-mode outputs, targets, and the teacher-forced batch of the same poses
@@ -948,8 +915,7 @@ class NavCMTAgent(RolloutTrainer):
         env = self.env
         dev = self.device
         T = int(getattr(self.args, "max_action_len", 15))
-        items, lb, gps0, geo, tidx, dirs0, gt_paths, traj = self._rollout_setup()
-        B = len(items)
+        _, lb, gps0, geo, tidx, dirs0, gt_paths, traj = self._rollout_setup()
         has_gt = "test" not in self.env_name
         prev_r, self.renderer = self.renderer, env.renderer
         try:
@@ -958,19 +924,13 @@ class NavCMTAgent(RolloutTrainer):
                 res = self.rollout_greedy(dict(corners_gps=torch.from_numpy(gps0).to(dev), directions=dirs0, geo=geo,
                                                tile_idx=tidx, lang=seq.float(), lang_cls=lin.float()), max_action_len=T)
                 steps = int(res["steps"])
-                ended = res["ended"][:steps].cpu().numpy().astype(bool)
-                c_h, d_h = res["corners"].cpu().numpy(), res["directions"].cpu().numpy()
-                outs = res["output"][:steps].cpu().numpy()
                 tgt = None
                 if has_gt:
-                    flat = res["corners"][:steps].reshape(steps * B, 4, 2)
-                    eb = np.zeros((steps, B), dtype=np.uint8)
-                    eb[1:] = ended[:steps - 1]
-                    xy, alt, pr = self.teacher_action(flat, [gt_paths[k % B] for k in range(steps * B)], eb.reshape(-1),
-                                                      feedback="student")
-                    tgt = (xy.view(steps, B, 2).cpu().numpy(), alt.view(steps, B).cpu().numpy(),
-                           pr.view(steps, B).cpu().numpy())
-                self._log_traj(traj, outs, tgt, ended, c_h, d_h, steps)
+                    tgt = tuple(a.cpu().numpy() for a in student_targets(self, res["corners"][:steps],
+                                                                         res["ended"][:steps], gt_paths))
+                self._log_traj(traj, res["output"][:steps].cpu().numpy(), tgt,
+                               res["ended"][:steps].cpu().numpy().astype(bool), res["corners"].cpu().numpy(),
+                               res["directions"].cpu().numpy(), steps)
                 return traj
             if self.feedback == "student" and not not_in_train and getattr(self.args, "on_policy_student", False):
                 self._on_policy_rollout(lb, gps0, dirs0, geo, tidx, gt_paths, traj, T, train_ml, nss_w, has_gt)
@@ -978,10 +938,8 @@ class NavCMTAgent(RolloutTrainer):
             # ---- poses of the rollout ----
             if self.feedback == "teacher":
                 Hh, steps = self._teacher_rollout_poses(torch.from_numpy(gps0), dirs0, geo, gt_paths, T)
-                corners = Hh["corners"][:steps]
-                ended = Hh["ended"][:steps]
-                tgt_xy, tgt_alt, tgt_prog = Hh["xy"][:steps], Hh["alt"][:steps], Hh["prog"][:steps]
-                heads = Hh["dirs"][:steps]
+                corners, ended, heads = Hh["corners"][:steps], Hh["ended"][:steps], Hh["dirs"][:steps]
+                tgt = (Hh["xy"][:steps], Hh["alt"][:steps], Hh["prog"][:steps])
                 c_all, d_all = Hh["corners"], Hh["dirs"]
             elif self.feedback == "student":
                 # the student's own (no-grad, eval-mode) greedy rollout fixes the poses; the teacher supplies the
@@ -994,26 +952,14 @@ class NavCMTAgent(RolloutTrainer):
                 steps = int(res["steps"])
                 corners, ended, heads = res["corners"][:steps], res["ended"][:steps], res["directions"][:steps]
                 c_all, d_all = res["corners"], res["directions"]
-                eb = torch.zeros((steps, B), dtype=torch.uint8, device=dev)
-                eb[1:] = ended[:steps - 1]
-                xy, alt, pr = self.teacher_action(corners.reshape(steps * B, 4, 2),
-                                                  [gt_paths[k % B] for k in range(steps * B)], eb.reshape(-1),
-                                                  feedback="student")
-                tgt_xy, tgt_alt, tgt_prog = xy.view(steps, B, 2), alt.view(steps, B), pr.view(steps, B)
+                tgt = student_targets(self, corners, ended, gt_paths)
             else:
                 raise SystemExit("Invalid feedback option")
             ended_h = ended.cpu().numpy().astype(bool)
-            alive = np.ones((steps, B), dtype=bool)
-            alive[1:] = ~ended_h[:steps - 1]
-            lens = np.maximum(np.cumsum(alive, axis=0).T, 1)             # [B, steps]: history length seen at step t
-            px = torch.empty((steps * B, 4, 2), dtype=torch.int32, device=dev)
-            _lib.call("avdn_gps_to_pixels", _lib.ptr(corners.reshape(steps * B, 4, 2).contiguous()),
-                      _lib.ptr(geo.repeat(steps, 1).contiguous()), steps * B, _lib.ptr(px))
+            lens = history_lengths(ended_h)
             rad = heads.float() / 180 * PI_REF                            # agent.py:605-606
-            tb = lambda a: a.reshape(steps, B, *a.shape[2:]).transpose(0, 1).contiguous()
-            batch = dict(lb, corners_px=tb(px.view(steps, B, 4, 2)), tile_idx=tidx.view(B, 1).expand(B, steps).contiguous(),
-                         directions=tb(torch.stack([torch.sin(rad), torch.cos(rad)], -1)),
-                         gt_xy=tb(tgt_xy.float()), gt_alt=tb(tgt_alt.float()), gt_prog=tb(tgt_prog.float()),
+            batch = dict(lb, **rollout_pose_batch(corners, geo, tidx, tgt),
+                         directions=torch.stack([torch.sin(rad), torch.cos(rad)], -1).transpose(0, 1).contiguous(),
                          lenths=lens.tolist())
             if getattr(self.args, "no_direction", False):
                 batch["directions"] = torch.zeros_like(batch["directions"])
@@ -1024,11 +970,12 @@ class NavCMTAgent(RolloutTrainer):
                 loss = self.train_rollout_step(batch, zero=False, step=False, nss_w=float(nss_w),
                                                train_ml=train_ml if train_ml is not None else 0.0, collect=outs,
                                                bn_per_step=bool(getattr(self.args, "bn_per_step", True)))
-            tgt = (tgt_xy.cpu().numpy(), tgt_alt.cpu().numpy(), tgt_prog.cpu().numpy()) if has_gt else None
             # what the rollout was made of (inspection / tests): poses, stop flags, targets, the training batch
-            self._last_rollout = dict(corners=corners, ended=ended, steps=steps, tgt_xy=tgt_xy, tgt_alt=tgt_alt,
-                                      tgt_prog=tgt_prog, batch=batch, lenths=lens)
-            self._log_traj(traj, torch.stack(outs).cpu().numpy(), tgt, ended_h, c_all.cpu().numpy(), d_all.cpu().numpy(), steps)
+            self._last_rollout = dict(corners=corners, ended=ended, steps=steps, tgt_xy=tgt[0], tgt_alt=tgt[1],
+                                      tgt_prog=tgt[2], batch=batch, lenths=lens)
+            tgt_h = tuple(a.cpu().numpy() for a in tgt) if has_gt else None
+            self._log_traj(traj, torch.stack(outs).cpu().numpy(), tgt_h, ended_h, c_all.cpu().numpy(), d_all.cpu().numpy(),
+                           steps)
             self._add_rollout_loss(loss, train_ml)
         finally:
             self.renderer = prev_r

@@ -20,7 +20,8 @@ Student-feedback training runs in one of two ways.  By default (``rollout``, ``s
 ``args.on_policy_student`` ``rollout`` calls ``student_rollout_step`` instead, the reference's single pass
 (agent.py:518-774): every step renders the current views, runs its own train-mode trunk pass (per-step batch
 statistics) and ``_TrainEngine.step`` with dropout on, and the simulator moves by that train-mode output; the targets,
-loss and backward through time follow once the loop has ended.
+loss and backward through time follow once the loop has ended.  Both training rollouts end in ``_finish_backward``
+(backward through time, BERT backward, trunk backward, optimiser).
 
 Training: one ``FusedAdamW`` over ``vln_model.used_parameters()`` (gradients clipped to a global norm of 40) and one
 over the trunk (unclipped), built here before any rollout captures a CUDA graph of the trunk (the arenas re-home
@@ -43,8 +44,8 @@ import numpy as np
 import torch
 
 from .. import _lib
-from ..agent_common import (RolloutTrainer, render_rollout_views, rollout_step_bufs, rollout_trunk_backward,
-                            rollout_trunk_forward, steps_until_all_ended, student_rollout_targets)
+from ..agent_common import (RolloutTrainer, render_rollout_views, rollout_pose_batch, rollout_step_bufs,
+                            rollout_trunk_backward, rollout_trunk_forward, steps_until_all_ended, student_targets)
 from ..env import ViewRenderer
 from ..models import dark_net as DN
 from ..models.dark_net import Darknet
@@ -216,9 +217,9 @@ class NavCMTAgent(RolloutTrainer):
             for opt in self.optimizers:
                 opt.zero_grad()
             n += 2
-        leng = leng2 = None
+        lengs = None
         if "input_ids" in batch:
-            seq, lin, leng, leng2 = self._lang_train_forward(batch)
+            seq, lin, *lengs = self._lang_train_forward(batch)
             batch = dict(batch, lang_feature=seq, cls_hidden=lin)
         lang, cls = batch["lang_feature"].contiguous().float(), batch["cls_hidden"].contiguous().float()
         L = lang.shape[1]
@@ -241,21 +242,30 @@ class NavCMTAgent(RolloutTrainer):
         n += 5
         if collect is not None:
             collect.extend(eng.output[t].clone() for t in range(T))
-        if leng is None:
-            eng.backward()
-        else:
-            d_lang = torch.zeros((B, L, 768), dtype=torch.float32, device=dev)
-            d_cls = torch.zeros((B, 49), dtype=torch.float32, device=dev)
-            eng.backward(d_lang, d_cls)
-            self._lang_train_backward(leng, leng2, d_lang, d_cls)
-        trunk_launches = rollout_trunk_backward(self, teng, tengs, l0, eng.d_frames, B, T)
+        n += self._finish_backward(eng, lengs, teng, tengs, l0, T, step)
         self._ctx = (teng, tengs, eng, tb)
+        self.launches += n + (eng.launches - e0)
+        self._log_loss()
+        return float(self.loss_total.item()) if sync_loss else self.loss_total
+
+    def _finish_backward(self, eng, lengs, teng, tengs, l0, steps, step):
+        """What follows the loss of both training rollouts: the backward through time over the first ``steps`` steps
+        (with ``lengs``, ``_lang_train_forward``'s engines, it also sums the ``lang_feature`` / ``cls_hidden``
+        gradients for BERT's backward), ``rollout_trunk_backward`` and, with ``step``, the optimiser step.  Returns
+        the launches outside the policy engine."""
+        B, L, T = eng.B, eng.L, eng.T
+        if lengs is None:
+            eng.backward(n_steps=steps)
+        else:
+            d_lang = torch.zeros((B, L, 768), dtype=torch.float32, device=self.device)
+            d_cls = torch.zeros((B, 49), dtype=torch.float32, device=self.device)
+            eng.backward(d_lang, d_cls, n_steps=steps)
+            self._lang_train_backward(*lengs, d_lang, d_cls)
+        n = rollout_trunk_backward(self, teng, tengs, l0, eng.d_frames, B, T, steps=steps)
         if step:
             for opt in self.optimizers:
                 n += opt.step()
-        self.launches += n + trunk_launches + (eng.launches - e0)
-        self._log_loss()
-        return float(self.loss_total.item()) if sync_loss else self.loss_total
+        return n
 
     @torch.no_grad()
     def student_batch(self, batch, gt_path_corners, max_action_len=None):
@@ -264,7 +274,10 @@ class NavCMTAgent(RolloutTrainer):
         ``train_rollout_step`` batch.  ``batch`` as for ``rollout_greedy``; ``gt_path_corners``: per sample the
         ``[n_i,4,2]`` ground-truth view corners."""
         res = self.rollout_greedy(batch, max_action_len=max_action_len)
-        out, _, T = student_rollout_targets(self, batch, res, gt_path_corners)
+        T = res["ended"].shape[0]
+        corners = res["corners"][:T]
+        out = rollout_pose_batch(corners, batch["geo"], batch.get("tile_idx"),
+                                 student_targets(self, corners, res["ended"], gt_path_corners))
         out.update(lang_feature=batch["lang_feature"], cls_hidden=batch["cls_hidden"],
                    directions=res["directions"][:T].float().t().contiguous())
         return out
@@ -275,9 +288,9 @@ class NavCMTAgent(RolloutTrainer):
         every step runs the policy in train mode -- the trunk on the step's own batch statistics, the four Dropout(0.2)
         sites active -- and the simulator moves by that same train-mode prediction (stop threshold 0.25).  The loop
         stops after the step at which every sample has ended (one host read of the B stop flags per step).  Then one
-        ``teacher_action`` launch gives the target of every visited pose, and the loss, the backward through time,
-        the trunk backward of the executed per-step passes, the BERT backward and (``step``) the optimiser step run
-        as in ``train_rollout_step``.
+        ``teacher_action`` launch gives the target of every visited pose, and the loss and ``_finish_backward`` (the
+        backward through time, the BERT backward, the trunk backward of the executed per-step passes and (``step``)
+        the optimiser step) run as in ``train_rollout_step``.
 
         ``batch`` as for ``rollout_greedy``; with an attached language model it may carry ``input_ids`` /
         ``attention_mask`` (and ``cls_*``) instead of ``lang_feature`` / ``cls_hidden``: BERT then runs once in train
@@ -302,9 +315,9 @@ class NavCMTAgent(RolloutTrainer):
             for opt in self.optimizers:
                 opt.zero_grad()
             n += 2
-        leng = leng2 = None
+        lengs = None
         if "input_ids" in batch:
-            seq, lin, leng, leng2 = self._lang_train_forward(batch)
+            seq, lin, *lengs = self._lang_train_forward(batch)
             batch = dict(batch, lang_feature=seq, cls_hidden=lin)
         lang, cls = batch["lang_feature"].contiguous().float(), batch["cls_hidden"].contiguous().float()
         B, L = lang.shape[0], lang.shape[1]
@@ -353,47 +366,36 @@ class NavCMTAgent(RolloutTrainer):
         bf["dir_hist"][steps].copy_(bf["cur_dir"])
         eng.finish()
         # ---- the teacher's target at every visited pose, one launch (agent.py:655-661) ----
-        res = dict(corners=bf["corners_hist"], ended=bf["ended_hist"], steps=steps)
-        tgt, _, _ = student_rollout_targets(self, batch, res, gt_path_corners)
-        sm = lambda a: a.transpose(0, 1).contiguous()                  # [B,steps,...] -> step-major
+        corners = bf["corners_hist"][:steps]
+        tgt = student_targets(self, corners, bf["ended_hist"][:steps], gt_path_corners)
+        poses = rollout_pose_batch(corners, geo, ti, tgt)
         att = None
         if self.nss_w != 0:
             key = ("on_policy_att", B, T)
             if key not in self._bufs:
                 self._bufs[key] = torch.empty((T * B, 224, 224), dtype=torch.uint8, device=dev)
             att = self._bufs[key][:steps * B]
-            minv = r.homography(sm(tgt["corners_px"]).view(steps * B, 4, 2))
+            minv = r.homography(poses["corners_px"].transpose(0, 1).reshape(steps * B, 4, 2))
             r.render(None, None if ti is None else ti.repeat(steps), views=False, att=True, minv=minv,
                      out={"att": att})
             att = att.view(steps, B, 224, 224)
             n += 2
         self.loss_total.zero_()
-        eng.loss(sm(tgt["gt_xy"]), sm(tgt["gt_alt"]), sm(tgt["gt_prog"]), att, self.nss_w,
-                 int(getattr(self.args, "nss_r", 0)), float(self.train_ml) / B, self.loss_total, n_steps=steps)
+        eng.loss(*tgt, att, self.nss_w, int(getattr(self.args, "nss_r", 0)), float(self.train_ml) / B, self.loss_total,
+                 n_steps=steps)
         n += 6
         if collect is not None:
             collect.extend(eng.output[t].clone() for t in range(steps))
-        if leng is None:
-            eng.backward(n_steps=steps)
-        else:
-            d_lang = torch.zeros((B, L, 768), dtype=torch.float32, device=dev)
-            d_cls = torch.zeros((B, 49), dtype=torch.float32, device=dev)
-            eng.backward(d_lang, d_cls, n_steps=steps)
-            self._lang_train_backward(leng, leng2, d_lang, d_cls)
-        trunk_launches = rollout_trunk_backward(self, tengs[0], tengs, l0, eng.d_frames, B, T, steps=steps)
+        n += self._finish_backward(eng, lengs, tengs[0], tengs, l0, steps, step)
         self._ctx = (tengs[0], tengs, eng, sb)
         # what the rollout visited (inspection / tests): poses before every step and after the last, stop flags,
         # train-mode outputs, targets, and the teacher-forced batch of the same poses
-        tr = {k: tgt[k] for k in ("corners_px", "tile_idx", "gt_xy", "gt_alt", "gt_prog")}
         self._last_rollout = dict(
             corners=bf["corners_hist"][:steps + 1].clone(), directions=bf["dir_hist"][:steps + 1].clone(),
             ended=bf["ended_hist"][:steps].clone(), output=eng.output[:steps].clone(), steps=steps,
-            tgt_xy=sm(tgt["gt_xy"]), tgt_alt=sm(tgt["gt_alt"]), tgt_prog=sm(tgt["gt_prog"]),
-            batch=dict(batch, directions=bf["dir_hist"][:steps].float().t().contiguous(), **tr))
-        if step:
-            for opt in self.optimizers:
-                n += opt.step()
-        self.launches += n + trunk_launches + (eng.launches - e0)
+            tgt_xy=tgt[0], tgt_alt=tgt[1], tgt_prog=tgt[2],
+            batch=dict(batch, directions=bf["dir_hist"][:steps].float().t().contiguous(), **poses))
+        self.launches += n + (eng.launches - e0)
         self._log_loss()
         return float(self.loss_total.item()) if sync_loss else self.loss_total
 
@@ -435,8 +437,7 @@ class NavCMTAgent(RolloutTrainer):
         env = self.env
         dev = self.device
         T = int(getattr(self.args, "max_action_len", 20))
-        items, lb, gps0, geo, tidx, dirs0, gt_paths, traj = self._rollout_setup()
-        B = len(items)
+        _, lb, gps0, geo, tidx, dirs0, gt_paths, traj = self._rollout_setup()
         has_gt = "test" not in self.env_name
         prev_r, self.renderer = self.renderer, env.renderer
         try:
@@ -446,7 +447,7 @@ class NavCMTAgent(RolloutTrainer):
             if self.feedback == "teacher":
                 H, steps = self._teacher_rollout_poses(torch.from_numpy(gps0), dirs0, geo, gt_paths, T)
                 corners, ended, heads = H["corners"][:steps], H["ended"][:steps], H["dirs"][:steps]
-                tgt_xy, tgt_alt, tgt_prog = H["xy"][:steps], H["alt"][:steps], H["prog"][:steps]
+                tgt = (H["xy"][:steps], H["alt"][:steps], H["prog"][:steps])
                 c_all, d_all = H["corners"], H["dirs"]
             elif self.feedback == "student":
                 seq, lin = self._lang_eval_forward(lb)
@@ -456,30 +457,18 @@ class NavCMTAgent(RolloutTrainer):
                 steps = steps_until_all_ended(res["ended"])
                 corners, ended, heads = res["corners"][:steps], res["ended"][:steps], res["directions"][:steps]
                 c_all, d_all = res["corners"], res["directions"]
-                tgt_xy = tgt_alt = tgt_prog = None
+                tgt = None
                 if has_gt or not not_in_train:
-                    # the teacher's target at every visited pose (agent.py:655-661)
-                    eb = torch.zeros((steps, B), dtype=torch.uint8, device=dev)
-                    eb[1:] = ended[:steps - 1]
-                    xy, alt, pr = self.teacher_action(corners.reshape(steps * B, 4, 2),
-                                                      [gt_paths[k % B] for k in range(steps * B)], eb.reshape(-1),
-                                                      feedback="student")
-                    tgt_xy, tgt_alt, tgt_prog = xy.view(steps, B, 2), alt.view(steps, B), pr.view(steps, B)
+                    tgt = student_targets(self, corners, ended, gt_paths)
             else:
                 raise SystemExit("Invalid feedback option")
             ended_h = ended.cpu().numpy().astype(bool)
-            tgt = (tgt_xy.cpu().numpy(), tgt_alt.cpu().numpy(), tgt_prog.cpu().numpy()) if has_gt else None
+            tgt_h = tuple(a.cpu().numpy() for a in tgt) if has_gt else None
             if not_in_train and self.feedback == "student":
-                self._log_traj(traj, res["output"][:steps].cpu().numpy(), tgt, ended_h, c_all.cpu().numpy(),
+                self._log_traj(traj, res["output"][:steps].cpu().numpy(), tgt_h, ended_h, c_all.cpu().numpy(),
                                d_all.cpu().numpy(), steps)
                 return traj
-            px = torch.empty((steps * B, 4, 2), dtype=torch.int32, device=dev)
-            _lib.call("avdn_gps_to_pixels", _lib.ptr(corners.reshape(steps * B, 4, 2).contiguous()),
-                      _lib.ptr(geo.repeat(steps, 1).contiguous()), steps * B, _lib.ptr(px))
-            tb = lambda a: a.reshape(steps, B, *a.shape[2:]).transpose(0, 1).contiguous()
-            batch = dict(lb, corners_px=tb(px.view(steps, B, 4, 2)), tile_idx=tidx.view(B, 1).expand(B, steps).contiguous(),
-                         directions=tb(heads.float()), gt_xy=tb(tgt_xy.float()), gt_alt=tb(tgt_alt.float()),
-                         gt_prog=tb(tgt_prog.float()))
+            batch = dict(lb, **rollout_pose_batch(corners, geo, tidx, tgt), directions=heads.float().t().contiguous())
             outs = []
             if not_in_train:
                 loss = self._eval_rollout(batch, traj, outs)
@@ -488,10 +477,10 @@ class NavCMTAgent(RolloutTrainer):
                                                train_ml=train_ml if train_ml is not None else 0.0, collect=outs,
                                                bn_per_step=bool(getattr(self.args, "bn_per_step", True)))
             # what the rollout was made of (inspection / tests): poses, stop flags, targets, the training batch
-            self._last_rollout = dict(corners=corners, ended=ended, steps=steps, tgt_xy=tgt_xy, tgt_alt=tgt_alt,
-                                      tgt_prog=tgt_prog, batch=batch)
-            self._log_traj(traj, torch.stack(outs).cpu().numpy(), tgt, ended_h, c_all.cpu().numpy(), d_all.cpu().numpy(),
-                           steps)
+            self._last_rollout = dict(corners=corners, ended=ended, steps=steps, tgt_xy=tgt[0], tgt_alt=tgt[1],
+                                      tgt_prog=tgt[2], batch=batch)
+            self._log_traj(traj, torch.stack(outs).cpu().numpy(), tgt_h, ended_h, c_all.cpu().numpy(),
+                           d_all.cpu().numpy(), steps)
             self._add_rollout_loss(loss, train_ml)
         finally:
             self.renderer = prev_r
