@@ -17,6 +17,7 @@ from torch import nn
 
 from .. import _lib
 from ._et_engine import ETEngine, ETDecodeState, E, NCH, NSP
+from ._lease import EnginePool, lease_slot
 from .enc_vl import EncoderVL
 
 
@@ -48,6 +49,7 @@ class ET(nn.Module):
         self.fc2 = nn.Linear(49, 768)
         self.init_weights()
         self._engines = {}
+        self._pool = EnginePool(self._pool_engine)
         self._grad_arena = None          # name -> tensor, set by the optimiser arena (xview_et.agent)
 
     def init_weights(self, init_range=0.1):
@@ -59,8 +61,9 @@ class ET(nn.Module):
         skip = ("dec_action.", "attention_layer_vision.c.")
         return {n: p for n, p in self.named_parameters() if not n.startswith(skip)}
 
-    def engine(self, B, L, T, device):
-        key = (B, L, T, str(device))
+    def engine(self, B, L, T, device, slot=0):
+        """``slot`` separates engines of equal shape whose activations must coexist (pending forwards)."""
+        key = (B, L, T, str(device)) if slot == 0 else (B, L, T, str(device), slot)
         eng = self._engines.get(key)
         if eng is None:
             a = self.args
@@ -68,6 +71,9 @@ class ET(nn.Module):
                            grads=self._grad_arena)
             self._engines[key] = eng
         return eng
+
+    def _pool_engine(self, key, slot):
+        return self.engine(*key, slot=lease_slot(slot))
 
     def decoder(self, B, L, Tmax, device):
         """Incremental inference state of a greedy rollout (``_et_engine.ETDecodeState``)."""
@@ -103,9 +109,10 @@ class ET(nn.Module):
         if tuple(frames.shape[2:]) != (NCH, NSP):
             raise ValueError("frames must be [B,T,512,49] (src/xview_et/agent.py:594,615)")
         lenths = [int(x) for x in inputs["lenths"]]
-        eng = self.engine(B, L, T, frames.device)
+        # with grad enabled the engine is held until this forward's backward (``_lease.EnginePool``)
+        eng, lease = self._pool.acquire((B, L, T, frames.device), torch.is_grad_enabled())
         eng.set_dropout(*self.dropout_config())
-        return _ETFn.apply(self, eng, lenths, frames, lang, lang_cls, dirs, *self.used_parameters().values())
+        return _ETFn.apply(self, eng, lease, lenths, frames, lang, lang_cls, dirs, *self.used_parameters().values())
 
     def forward(self, **inputs):
         """src/models/ET_haa.py:121-184: keys ``directions [B,T,2]``, ``frames [B,T,512,49]``,
@@ -117,13 +124,14 @@ class ET(nn.Module):
 
 class _ETFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, mod, eng, lenths, frames, lang, lang_cls, dirs, *params):
+    def forward(ctx, mod, eng, lease, lenths, frames, lang, lang_cls, dirs, *params):
         f = frames.detach().contiguous().float().view(-1, NCH, NSP)
         lg = lang.detach().contiguous().float()
         lc = lang_cls.detach().contiguous().float()
         dr = dirs.detach().contiguous().float()
         output, h_sali = eng.forward(f, lg, lc, dr, lenths, mod.encoder_vl.enc_pos.pe[0])
         ctx.mod, ctx.eng = mod, eng
+        ctx.save_for_backward(lease)
         ctx.frames_shape = frames.shape
         ctx.need_lang = lang.requires_grad
         ctx.need_cls = lang_cls.requires_grad
@@ -144,7 +152,7 @@ class _ETFn(torch.autograd.Function):
             grads = [eng.G[n].clone() for n in mod.used_parameters()]
         else:                            # gradients were accumulated straight into the optimiser arena
             grads = [None] * len(mod.used_parameters())
-        return (None, None, None, d_frames.view(ctx.frames_shape) if ctx.need_frames else None, d_lang, d_cls, None,
+        return (None, None, None, None, d_frames.view(ctx.frames_shape) if ctx.need_frames else None, d_lang, d_cls, None,
                 *grads)
 
 

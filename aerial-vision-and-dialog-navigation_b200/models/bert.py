@@ -26,6 +26,7 @@ from torch import nn
 
 from .. import _lib
 from .. import gemm as G
+from ._lease import EnginePool, lease_slot
 
 E = 768
 LN_EPS = 1e-12
@@ -337,6 +338,7 @@ class CustomBERTModel(nn.Module):
             raise NotImplementedError("only the bert-base geometry (768 wide, 64-wide heads, erf-GELU) is implemented")
         self.linears = nn.Sequential(nn.Linear(768, 64), nn.ReLU(), nn.Dropout(0.2), nn.Linear(64, 49), nn.ReLU())
         self._engines = {}
+        self._pool = EnginePool(self._pool_engine)
         self._grad_arena = None          # name -> tensor, set by the optimiser arena (xview_et.agent.attach_lang_model)
         self._drop_step = 0
 
@@ -365,21 +367,26 @@ class CustomBERTModel(nn.Module):
             self._engines[key] = e
         return e
 
+    def _pool_engine(self, key, slot):
+        return self.engine(*key, slot=lease_slot(slot))
+
     def forward(self, ids, mask):
         _lib.require_cuda(ids, mask)
         B, S = ids.shape
         if S > self.bert.config.max_position_embeddings:
             raise ValueError("sequence longer than the position table")
-        eng = self.engine(B, S, ids.device)
+        # with grad enabled the engine is held until this forward's backward (``_lease.EnginePool``)
+        eng, lease = self._pool.acquire((B, S, ids.device), torch.is_grad_enabled())
         eng.set_dropout(*self.dropout_config())
-        return _BertFn.apply(self, eng, ids, mask, *self.used_parameters().values())
+        return _BertFn.apply(self, eng, lease, ids, mask, *self.used_parameters().values())
 
 
 class _BertFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, mod, eng, ids, mask, *params):
+    def forward(ctx, mod, eng, lease, ids, mask, *params):
         seq, lin, pooled = eng.forward(ids.long(), mask)
         ctx.mod, ctx.eng = mod, eng
+        ctx.save_for_backward(lease)
         return seq.clone(), lin.clone(), pooled.clone()
 
     @staticmethod
@@ -388,4 +395,4 @@ class _BertFn(torch.autograd.Function):
         eng.zero_grads()
         eng.backward(None if d_seq is None else d_seq.contiguous().float(), d_lin,
                      None if d_pooled is None else d_pooled.contiguous().float())
-        return (None, None, None, None, *[eng.G[n].clone() for n in ctx.mod.used_parameters()])
+        return (None, None, None, None, None, *[eng.G[n].clone() for n in ctx.mod.used_parameters()])

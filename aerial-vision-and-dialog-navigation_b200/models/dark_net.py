@@ -25,6 +25,7 @@ import torch.nn as nn
 
 from .. import _lib
 from .. import gemm as G
+from ._lease import EnginePool, lease_slot
 
 LEAKY_SLOPE = 0.01      # nn.LeakyReLU() default, dark_net.py:33
 # AVDN_FUSE_BNB=1: BatchNorm-backward reductions fused into the epilogue of the data-gradient convolution that
@@ -513,9 +514,10 @@ def _trunk_backward(net, eng, dout, after_layer=None, flush_layers=None):
 
 class _TrunkFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, net, eng, x_nhwc4, train, *params):
+    def forward(ctx, net, eng, lease, x_nhwc4, train, *params):
         out = _trunk_forward(net, eng, x_nhwc4, train)
         ctx.net, ctx.eng, ctx.train = net, eng, train
+        ctx.save_for_backward(lease)     # holds the engine's activations until this node's graph is freed
         return out
 
     @staticmethod
@@ -532,7 +534,7 @@ class _TrunkFn(torch.autograd.Function):
         flat = []
         for L in eng.layers:
             flat += [L.dw.clone(), L.dgamma.clone(), L.dbeta.clone()] if own else [None, None, None]
-        return (None, None, None, None, *flat)
+        return (None, None, None, None, None, *flat)
 
 
 class Darknet(nn.Module):
@@ -546,6 +548,7 @@ class Darknet(nn.Module):
         self.img_size = img_size
         self.loss_names = ["loss", "x", "y", "w", "h", "conf", "cls", "nGT", "TP", "FP", "FPe", "FN", "TC"]
         self._engines = {}
+        self._pool = EnginePool(self._pool_engine)
         self._grad_arena = None          # name -> tensor, set by the optimiser arena (xview_et.agent)
         self._pending_batches = 0
         self.register_state_dict_pre_hook(lambda m, prefix, keep_vars: m._flush_batches_tracked())
@@ -582,14 +585,19 @@ class Darknet(nn.Module):
             self._engines[key] = e
         return e
 
+    def _pool_engine(self, key, slot):
+        return self._engine(*key, slot=lease_slot(slot))
+
     def forward_nhwc4(self, x_nhwc4):
         """Fast path: ``x`` is the renderer's ``norm_nhwc`` output ``[N,H,W,4]`` bf16
-        (R,G,B,0).  Returns ``[N, C_last, H/32, W/32]`` float32."""
+        (R,G,B,0).  Returns ``[N, C_last, H/32, W/32]`` float32.  A train-mode forward with grad enabled
+        keeps its engine (and so its activations) until its backward: pending forwards of one shape each
+        run on an engine of their own (``_lease.EnginePool``)."""
         _lib.require_cuda(x_nhwc4)
         assert x_nhwc4.dtype == torch.bfloat16 and x_nhwc4.shape[-1] == 4 and x_nhwc4.is_contiguous()
         N, H, W, _ = x_nhwc4.shape
-        eng = self._engine(N, H, W, x_nhwc4.device)
-        return _TrunkFn.apply(self, eng, x_nhwc4, self.training, *self._params())
+        eng, lease = self._pool.acquire((N, H, W, x_nhwc4.device), self.training and torch.is_grad_enabled())
+        return _TrunkFn.apply(self, eng, lease, x_nhwc4, self.training, *self._params())
 
     def forward(self, x, targets=None, requestPrecision=False, weight=None, epoch=None):
         """Reference signature (dark_net.py:212): ``x`` is ``[N,3,H,W]`` float32 NCHW."""

@@ -8,6 +8,7 @@ from torch import nn
 from .. import _lib
 from . import model_util
 from ._et_engine import ETEngine, E
+from ._lease import EnginePool, lease_slot
 from .encodings import PosEncoding
 
 
@@ -27,6 +28,18 @@ class EncoderVL(nn.Module):
         self.enc_dropout = nn.Dropout(args.dropout_emb, inplace=True)
         self.n_heads, self.n_layers, self.d_ff = args.encoder_heads, args.encoder_layers, args.demb
         self._engines = {}
+        self._pool = EnginePool(self._pool_engine)
+
+    def _pool_engine(self, key, slot):
+        B, L, T, device = key
+        key = (B, L, T, str(device)) if slot == 0 else (B, L, T, str(device), lease_slot(slot))
+        eng = self._engines.get(key)
+        if eng is None:
+            params = {"encoder_vl." + n: p for n, p in self.named_parameters()}
+            eng = ETEngine(params, self.n_heads, self.n_layers, self.d_ff, B, L, T, device,
+                           with_frame_attn=False, with_heads=False)
+            self._engines[key] = eng
+        return eng
 
     def _dropout_config(self):
         """Train mode: nn.TransformerEncoderLayer's dropout p at its four sites (stateless hash masks,
@@ -45,26 +58,22 @@ class EncoderVL(nn.Module):
         _lib.require_cuda(emb_lang, emb_frames, emb_directions)
         B, L, _ = emb_lang.shape
         T = emb_frames.shape[1]
-        key = (B, L, T, str(emb_lang.device))
-        eng = self._engines.get(key)
-        if eng is None:
-            params = {"encoder_vl." + n: p for n, p in self.named_parameters()}
-            eng = ETEngine(params, self.n_heads, self.n_layers, self.d_ff, B, L, T, emb_lang.device,
-                           with_frame_attn=False, with_heads=False)
-            self._engines[key] = eng
+        # with grad enabled the engine is held until this forward's backward (``_lease.EnginePool``)
+        eng, lease = self._pool.acquire((B, L, T, emb_lang.device), torch.is_grad_enabled())
         eng.set_dropout(*self._dropout_config())
-        out = _EncoderFn.apply(self, eng, list(lengths), emb_lang, emb_frames, emb_directions,
+        out = _EncoderFn.apply(self, eng, lease, list(lengths), emb_lang, emb_frames, emb_directions,
                                *[p for _, p in self.named_parameters()])
         return out, model_util.generate_pad_mask(lengths, L, emb_lang.device)
 
 
 class _EncoderFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, mod, eng, lengths, lang, frames, dirs, *params):
+    def forward(ctx, mod, eng, lease, lengths, lang, frames, dirs, *params):
         eng.set_lengths(lengths)
         lang, frames, dirs = (t.detach().contiguous().float() for t in (lang, frames, dirs))
         x = eng.encode(lang, frames, dirs, True, mod.enc_pos.pe[0])
         ctx.mod, ctx.eng = mod, eng
+        ctx.save_for_backward(lease)
         return x.view(eng.B, eng.S, E).clone()
 
     @staticmethod
@@ -76,4 +85,4 @@ class _EncoderFn(torch.autograd.Function):
         dv0 = eng.backward_encoder(d_out.contiguous().float()).view(eng.B, eng.S, E)
         L, T = eng.L, eng.T
         grads = [eng.G["encoder_vl." + n].clone() for n, _ in mod.named_parameters()]
-        return (None, None, None, dv0[:, :L].clone(), dv0[:, L:L + T].clone(), dv0[:, L + T:].clone(), *grads)
+        return (None, None, None, None, dv0[:, :L].clone(), dv0[:, L:L + T].clone(), dv0[:, L + T:].clone(), *grads)

@@ -7,9 +7,11 @@ the same ``state_dict`` keys (including the ``pos_embedding`` and
 same ``forward(current_direct, im_input, pos_input, cls_hidden, lang_feature, h_0, c_0,
 hh_0, cc_0) -> (h_1, c_1, hh_1, cc_1, output, pred_saliency)``.
 
-``step`` / ``forward`` are the inference step (the rollout of ``agent.test``,
+``step`` / eval-mode ``forward`` are the inference step (the rollout of ``agent.test``,
 src/xview_lstm/agent.py:191-206, runs under ``.eval()``): dropout is the identity and the trunk uses its
-running statistics; ``.train()`` + ``step`` raises.
+running statistics; ``.train()`` + ``step`` raises.  A train-mode ``forward`` with grad enabled is differentiable
+(the reference's training loop written with module calls, src/xview_lstm/agent.py:546-550,592-602): the trunk runs
+through autograd and the policy step on a one-step ``_TrainEngine`` of its own until its backward.
 
 Device work per step: trunk (tcgen05 convs, eval-mode BN folded into the apply pass),
 ``avdn_frame_attn_fwd`` (SoftDotAttention(49) over the 512 channels), ``avdn_linear_f32`` +
@@ -28,6 +30,8 @@ import torch
 from torch import nn
 
 from .. import _lib
+from ._lease import EnginePool, lease_slot
+from .ET_haa import _UpsampleFn
 
 NCH, NSP, HID = 512, 49, 768
 
@@ -112,6 +116,7 @@ class _TrainEngine:
         self.d_e49_bt, self.d_frames = f(BT, NSP), f(BT, NCH, NSP)
         self.G = grads if grads is not None else {n: torch.zeros_like(p) for n, p in model.used_parameters().items()}
         self.p, self.seed = 0.0, 0
+        self._state = None               # (h_0, c_0, hh_0, cc_0) before step 0; None: the zero state
         self.launches = 0
 
     def _lin_bwd(self, x, w, y, dy, act, dx, name, bias=True, dx_accumulate=0):
@@ -122,15 +127,18 @@ class _TrainEngine:
                   dy.shape[1], K, act, _lib.ptr(dx), dx.stride(0) if dx is not None else 0, dx_accumulate,
                   _lib.ptr(G[name + ".weight"] if bias else G[name]), _lib.ptr(G[name + ".bias"]) if bias else None)
 
-    def forward(self, frames, deg, cls_hidden, lang_feature, p=0.0, seed=0):
+    def forward(self, frames, deg, cls_hidden, lang_feature, p=0.0, seed=0, state=None):
         """The T policy steps on trunk features ``frames`` [B*T,512,49] f32 (episode-major, as the trunk emits them)
         with headings ``deg`` [B,T] (degrees), ``cls_hidden`` [B,49], ``lang_feature`` [B,L,768]; dropout ``p`` with
-        hash seed ``seed`` (``ViT_LSTM.dropout_config``).  Returns ``output`` [T,B,4] and ``h_sali`` [T,B,64]."""
+        hash seed ``seed`` (``ViT_LSTM.dropout_config``).  ``state``: the recurrent state ``(h_0 [B,192], c_0 [B,192],
+        hh_0 [B,576], cc_0 [B,576])`` step 0 starts from (default: zero, src/xview_lstm/agent.py:546-550); its
+        gradients are ``d_state0`` after ``backward``.  Returns ``output`` [T,B,4] and ``h_sali`` [T,B,64]."""
         m, B, L, T = self.m, self.B, self.L, self.T
         call, ptr = _lib.call, _lib.ptr
         BT = B * T
         l0 = m.launches
         self.p, self.seed = float(p), int(seed)
+        self._state = None if state is None else tuple(x.contiguous().float() for x in state)
         self._in = (frames.contiguous(), cls_hidden.contiguous(), lang_feature.contiguous())
         frames, cls, lang = self._in
         av = m.attention_layer_vision
@@ -154,6 +162,7 @@ class _TrainEngine:
         for a rollout whose frames and headings of step t+1 depend on the output of step t.  Arguments as for
         ``forward``."""
         self.p, self.seed = float(p), int(seed)
+        self._state = None
         if getattr(self, "_frames", None) is None:
             f = lambda *s: torch.zeros(s, dtype=torch.float32, device=self.deg.device)
             self._frames = f(self.B * self.T, NCH, NSP)                 # frame-major input, read by backward
@@ -216,12 +225,14 @@ class _TrainEngine:
         call, ptr = _lib.call, _lib.ptr
         al, dec = m.attention_layer_lang, m.decoder_2_action_full
         cat = self.cat2[t]
-        prev = self.cat2[t - 1] if t > 0 else None
+        if t:
+            prev = self.cat2[t - 1]
+            h, c, hh, cc = prev[:, HID:HID + 192], self.c_d[t - 1], prev[:, HID + 192:], self.c_v[t - 1]
+        else:
+            h, c, hh, cc = self._state if self._state is not None else (None,) * 4
         # hh_1, cc_1 = vision_lstm(drop(input_lstm_0), (hh_0, cc_0))                vln_model.py:220-226
-        m._lstm(m.vision_lstm, self.e49d[t], prev[:, HID + 192:] if t else None, self.c_v[t - 1] if t else None,
-                self.gates_v[t], cat[:, HID + 192:], self.c_v[t])
-        m._lstm(m.direct_lstm, self.dir_emb[t], prev[:, HID:HID + 192] if t else None,
-                self.c_d[t - 1] if t else None, self.gates_d[t], cat[:, HID:HID + 192], self.c_d[t])
+        m._lstm(m.vision_lstm, self.e49d[t], hh, cc, self.gates_v[t], cat[:, HID + 192:], self.c_v[t])
+        m._lstm(m.direct_lstm, self.dir_emb[t], h, c, self.gates_d[t], cat[:, HID:HID + 192], self.c_d[t])
         # action_module_input = SoftDotAttention(768)(cat(h_1, hh_1), lang_feature)  vln_model.py:238-239
         m._linear(cat[:, HID:], al.linear_in.weight, None, self.target[t])
         call("avdn_lang_attn_fwd", ptr(lang), ptr(self.target[t]), B, L, HID, ptr(self.attn[t]), ptr(cat),
@@ -246,12 +257,14 @@ class _TrainEngine:
                   ptr(self.d_output), ptr(self.d_h_sali))
         self.launches += 1
 
-    def backward(self, d_lang=None, d_cls=None, n_steps=None):
+    def backward(self, d_lang=None, d_cls=None, n_steps=None, d_state=None):
         """Backward through time from ``d_output`` / ``d_h_sali`` (written by ``loss``).  Overwrites ``d_frames``
         [B*T,512,49] (returned); accumulates every parameter gradient into ``G`` and, when given, the gradients of
         ``lang_feature`` into ``d_lang`` [B,L,768] and of ``cls_hidden`` into ``d_cls`` [B,49] (+=).  ``n_steps``
         (default T, as given to ``loss``): the steps the rollout ran; the rows of later steps get zero ``d_frames``
-        and contribute nothing."""
+        and contribute nothing.  ``d_state``: the gradients ``(d h, d c, d hh, d cc)`` of the recurrent state after
+        the last step (None entries: zero), for a caller that carries the state on.  A forward given ``state``
+        leaves the gradients of that state in ``d_state0`` = ``(d h_0, d c_0, d hh_0, d cc_0)``."""
         m, B, L = self.m, self.B, self.L
         T = self.T if n_steps is None else int(n_steps)
         call, ptr = _lib.call, _lib.ptr
@@ -276,6 +289,17 @@ class _TrainEngine:
         self._lin_bwd(r(self.cat2), al.linear_out.weight, r(self.act_in), r(self.d_act_in), 2, r(self.d_cat2),
                       "attention_layer_lang.linear_out.weight", bias=False)
         n += 4 + 2 * T
+        carry = d_state is not None      # gradients of the state after step T-1 enter as for a step T
+        if carry:
+            d_h, d_c, d_hh, d_cc = d_state
+            dlast = self.d_cat2[T - 1]
+            if d_h is not None:
+                dlast[:, HID:HID + 192].add_(d_h)
+            if d_hh is not None:
+                dlast[:, HID + 192:].add_(d_hh)
+            self.dc_d.zero_() if d_c is None else self.dc_d.copy_(d_c)
+            self.dc_v.zero_() if d_cc is None else self.dc_v.copy_(d_cc)
+        s0 = self._state
         # ---- backward through time: the data gradients that cross steps ----
         w_in_t = al.linear_in.weight.t().contiguous()           # d hcat = d target W_in  (linear_f32: x w^T)
         w_hh_v_t, w_hh_d_t = vl.weight_hh.t().contiguous(), dl.weight_hh.t().contiguous()
@@ -284,11 +308,14 @@ class _TrainEngine:
             call("avdn_lang_attn_bwd", ptr(lang), ptr(self.target[t]), ptr(self.attn[t]), ptr(dcat), dcat.stride(0),
                  B, L, HID, ptr(self.d_target[t]), ptr(d_lang))
             m._linear(self.d_target[t], w_in_t, None, dcat[:, HID:], accumulate=1)
-            first, last = t == 0, t == T - 1
-            call("avdn_lstm_cell_bwd", ptr(self.gates_d[t]), None if first else ptr(self.c_d[t - 1]), ptr(self.c_d[t]),
+            first, last = t == 0, t == T - 1 and not carry
+            # the cell state before step 0 is c_0 / cc_0 when given: then dc_prev of step 0 is its gradient
+            c_d_prev = self.c_d[t - 1] if not first else (s0[1] if s0 is not None else None)
+            c_v_prev = self.c_v[t - 1] if not first else (s0[3] if s0 is not None else None)
+            call("avdn_lstm_cell_bwd", ptr(self.gates_d[t]), ptr(c_d_prev), ptr(self.c_d[t]),
                  ptr(dcat[:, HID:HID + 192]), dcat.stride(0), None if last else ptr(self.dc_d), ptr(self.dg_d[t]),
                  ptr(self.dc_d), B, 192)
-            call("avdn_lstm_cell_bwd", ptr(self.gates_v[t]), None if first else ptr(self.c_v[t - 1]), ptr(self.c_v[t]),
+            call("avdn_lstm_cell_bwd", ptr(self.gates_v[t]), ptr(c_v_prev), ptr(self.c_v[t]),
                  ptr(dcat[:, HID + 192:]), dcat.stride(0), None if last else ptr(self.dc_v), ptr(self.dg_v[t]),
                  ptr(self.dc_v), B, 576)
             n += 3
@@ -296,6 +323,11 @@ class _TrainEngine:
                 prev = self.d_cat2[t - 1]
                 m._linear(self.dg_d[t], w_hh_d_t, None, prev[:, HID:HID + 192], accumulate=1)
                 m._linear(self.dg_v[t], w_hh_v_t, None, prev[:, HID + 192:], accumulate=1)
+            elif s0 is not None:           # ... and h_0 / hh_0 fed step 0's
+                self.d_state0 = (torch.empty_like(s0[0]), self.dc_d.clone(), torch.empty_like(s0[2]),
+                                 self.dc_v.clone())
+                m._linear(self.dg_d[0], w_hh_d_t, None, self.d_state0[0])
+                m._linear(self.dg_v[0], w_hh_v_t, None, self.d_state0[2])
         # ---- weight gradients over all T*B rows ----
         cat = r(self.cat2)
         self._lin_bwd(cat[:, HID:], al.linear_in.weight, r(self.d_target), r(self.d_target), 0, None,
@@ -306,12 +338,17 @@ class _TrainEngine:
             _lib.call("avdn_linear_f32_bwd", ptr(r(x)), x.shape[-1], ptr(cell.weight_ih), ptr(r(dg)), ptr(r(dg)), BT,
                       dg.shape[-1], x.shape[-1], 0, ptr(dx), dx.shape[-1], 0, ptr(G[name + ".weight_ih"]),
                       ptr(G[name + ".bias_ih"]))
+            H = cell.hidden_size
             if T > 1:                      # step 0 ran from the zero state: W_hh saw h = 0 there
-                H = cell.hidden_size
                 h_prev = self.cat2[:T - 1].view((T - 1) * B, 2 * HID)[:, lo:lo + H]
                 dg1 = dg[1:T].view((T - 1) * B, 4 * H)
                 _lib.call("avdn_linear_f32_bwd", ptr(h_prev), h_prev.stride(0), ptr(cell.weight_hh), ptr(dg1),
                           ptr(dg1), (T - 1) * B, 4 * H, H, 0, None, 0, 0, ptr(G[name + ".weight_hh"]), None)
+                n += 1
+            if s0 is not None:             # ... unless a state was given: W_hh saw h_0 / hh_0
+                h0 = s0[0] if lo == HID else s0[2]
+                _lib.call("avdn_linear_f32_bwd", ptr(h0), h0.stride(0), ptr(cell.weight_hh), ptr(dg[0]), ptr(dg[0]),
+                          B, 4 * H, H, 0, None, 0, 0, ptr(G[name + ".weight_hh"]), None)
                 n += 1
             call("avdn_colsum", ptr(dg), 1, BT, dg.shape[-1], dg.shape[-1], ptr(G[name + ".bias_hh"]))
             n += 2
@@ -356,6 +393,7 @@ class ViT_LSTM(nn.Module):
                                 nn.ReLU())
         self._bufs = {}
         self._train_engines = {}
+        self._pool = EnginePool(self._pool_engine)
         self._grad_arena = None          # name -> tensor, set by the optimiser arena (xview_lstm.agent)
         self.launches = 0
 
@@ -375,14 +413,29 @@ class ViT_LSTM(nn.Module):
                 + 0x9E3779B97F4A7C15 * int(getattr(self, "drop_rank", 0))) & 0xFFFFFFFFFFFFFFFF
         return DROP_P, seed
 
-    def train_engine(self, B, L, T, device):
+    def train_engine(self, B, L, T, device, slot=0):
         """The training-rollout engine of (B episodes, L tokens, T steps) (``_TrainEngine``); parameter gradients go
-        to the attached optimiser arena, or to engine-owned buffers ``engine.G`` when there is none."""
-        key = (B, L, T, str(device))
+        to the attached optimiser arena, or to engine-owned buffers ``engine.G`` when there is none.  ``slot``
+        separates engines of equal shape whose activations must coexist (pending train-mode forwards)."""
+        key = (B, L, T, str(device)) if slot == 0 else (B, L, T, str(device), slot)
         eng = self._train_engines.get(key)
         if eng is None:
             eng = self._train_engines[key] = _TrainEngine(self, B, L, T, device, self._grad_arena)
         return eng
+
+    def _pool_engine(self, key, slot):
+        B, L, device = key
+        return self.train_engine(B, L, 1, device, slot=lease_slot(slot))
+
+    def _step_dropout(self):
+        """(p, seed) of one train-mode ``forward``: a fresh seed per call (``dropout_config``) and the p of the four
+        nn.Dropout sites, 0 where they are in eval mode (the kernels take one p for all four)."""
+        _, seed = self.dropout_config()
+        sites = (self.drop, self.decoder_2_action_full[2], self.decoder_2_action_full[5], self.fc[2])
+        ps = {float(d.p) if d.training else 0.0 for d in sites}
+        if len(ps) != 1:
+            raise NotImplementedError("the four nn.Dropout sites of ViT_LSTM must share one p (or all be in eval mode)")
+        return ps.pop(), seed
 
     # ------------------------------------------------------------------ pieces
     def _linear(self, x, w, b, y, act=0, accumulate=0):
@@ -477,13 +530,20 @@ class ViT_LSTM(nn.Module):
 
     def forward(self, current_direct, im_input, pos_input, cls_hidden, lang_feature, h_0=None, c_0=None, hh_0=None,
                 cc_0=None):
-        """Reference signature (vln_model.py:213).  ``im_input`` [B,3,224,224] f32 normalised."""
+        """Reference signature (vln_model.py:213).  ``im_input`` [B,3,224,224] f32 normalised.
+
+        In train mode with grad enabled the step is differentiable: ``vision_model(im_input)`` runs through autograd
+        (a ``Darknet`` with batch statistics), the policy step with train-mode dropout (a fresh seed per call), and
+        the backward reaches every used parameter (``.grad``, or the attached optimiser arena), the trunk, and
+        ``cls_hidden``, ``lang_feature`` and ``h_0, c_0, hh_0, cc_0`` where they require grad."""
+        given = [x is not None for x in (h_0, c_0, hh_0, cc_0)]
+        if any(given) and not all(given):
+            raise ValueError("pass all four recurrent states or none")
+        if self.training and torch.is_grad_enabled():
+            return self._train_forward(current_direct, im_input, cls_hidden, lang_feature, h_0, c_0, hh_0, cc_0)
         with torch.no_grad():
             feat = self.vision_model(im_input)                                      # [B,512,7,7]
             B, L = feat.shape[0], lang_feature.shape[1]
-            given = [x is not None for x in (h_0, c_0, hh_0, cc_0)]
-            if any(given) and not all(given):
-                raise ValueError("pass all four recurrent states or none")
             bf = self.reset_state(B, L, feat.device)
             if all(given):                         # load the caller's state into the 'previous' buffers
                 p = bf.k ^ 1
@@ -494,3 +554,56 @@ class ViT_LSTM(nn.Module):
             _lib.call("avdn_upsample_saliency", _lib.ptr(h_sali), B, _lib.ptr(pred))
             h1, c1, hh1, cc1 = self.state(B, L, feat.device)
         return h1, c1, hh1, cc1, output.clone(), pred
+
+    def _train_forward(self, current_direct, im_input, cls_hidden, lang_feature, h_0, c_0, hh_0, cc_0):
+        feat = self.vision_model(im_input)                                          # [B,512,7,7], through autograd
+        _lib.require_cuda(feat, cls_hidden, lang_feature)
+        B, L = feat.shape[0], lang_feature.shape[1]
+        p, seed = self._step_dropout()
+        eng, lease = self._pool.lease((B, L, feat.device))
+        h1, c1, hh1, cc1, output, h_sali = _StepFn.apply(self, eng, lease, p, seed, feat, current_direct, cls_hidden,
+                                                         lang_feature, h_0, c_0, hh_0, cc_0,
+                                                         *self.used_parameters().values())
+        return h1, c1, hh1, cc1, output, _UpsampleFn.apply(h_sali)
+
+
+class _StepFn(torch.autograd.Function):
+    """One train-mode policy step on a leased one-step ``_TrainEngine``: the step's activations stay in the engine
+    until this node's backward (``_lease.EnginePool``)."""
+
+    @staticmethod
+    def forward(ctx, mod, eng, lease, p, seed, feat, current_direct, cls_hidden, lang_feature, h_0, c_0, hh_0, cc_0,
+                *params):
+        B = feat.shape[0]
+        frames = feat.reshape(B, NCH, NSP).contiguous().float()
+        state = None if h_0 is None else (h_0, c_0, hh_0, cc_0)
+        eng.forward(frames, current_direct.reshape(B, 1), cls_hidden.contiguous().float(),
+                    lang_feature.contiguous().float(), p, seed, state=state)
+        ctx.mod, ctx.eng, ctx.feat_shape = mod, eng, feat.shape
+        ctx.save_for_backward(lease)
+        ctx.set_materialize_grads(False)
+        cat = eng.cat2[0]
+        return (cat[:, HID:HID + 192].clone(), eng.c_d[0].clone(), cat[:, HID + 192:].clone(), eng.c_v[0].clone(),
+                eng.output[0].clone(), eng.h_sali[0].clone())
+
+    @staticmethod
+    def backward(ctx, d_h, d_c, d_hh, d_cc, d_output, d_h_sali):
+        mod, eng = ctx.mod, ctx.eng
+        need = ctx.needs_input_grad      # (mod, eng, lease, p, seed, feat, direct, cls, lang, h_0, c_0, hh_0, cc_0, ...)
+        own = eng.G is not mod._grad_arena
+        if own:
+            for g in eng.G.values():
+                g.zero_()
+        f = lambda d: None if d is None else d.contiguous().float()
+        for buf, d in ((eng.d_output, d_output), (eng.d_h_sali, d_h_sali)):
+            buf.zero_() if d is None else buf[0].copy_(d)
+        d_state = tuple(f(d) for d in (d_h, d_c, d_hh, d_cc))
+        d_cls = torch.zeros((eng.B, NSP), dtype=torch.float32, device=eng.deg.device) if need[7] else None
+        d_lang = torch.zeros((eng.B, eng.L, HID), dtype=torch.float32, device=eng.deg.device) if need[8] else None
+        d_frames = eng.backward(d_lang, d_cls, d_state=None if all(d is None for d in d_state) else d_state)
+        d_s0 = eng.d_state0 if eng._state is not None else (None,) * 4
+        d_s0 = tuple(d if n else None for d, n in zip(d_s0, need[9:13]))
+        names = mod.used_parameters()
+        grads = [eng.G[n].clone() for n in names] if own else [None] * len(names)
+        return (None, None, None, None, None, d_frames.view(ctx.feat_shape).clone() if need[5] else None, None, d_cls,
+                d_lang, *d_s0, *grads)
